@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--config c2]      # the CUDA path (one rank per GPU)
     python bench.py --impl reference --gpus N --steps K ...           # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                            # + the last timed step's arrays as DIR/*.npy
 
 A step is one pass of the whole hot path (window search, site classification, read scan, read-site
 allele lookup, chaining, tally, final call) over one batch of DNMs.  Workloads (BASELINE.json configs):
@@ -76,7 +77,15 @@ def parse():
                     help="after the timed legs, phase EVERY DNM of the workload with the oracle port (all host cores) and compare "
                          "all record dicts of the timed end-to-end batch with it (N=1; adds about a minute)")
     ap.add_argument("--no-saturating", action="store_true", help="skip the 2^25-pair classifier measurement")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed resident step returned (BatchResult arrays) as DIR/<name>.npy, "
+                         "float64, so that two builds can be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the arrays of the CUDA path (--impl b200)")
+    return args
 
 
 def config_of(args):
@@ -308,7 +317,7 @@ def run_reference(args):
         pr.start()
         conns.append(a)
         procs.append(pr)
-    times, t_all0 = [], time.perf_counter()
+    times = []
     for step in range(args.warmup + args.steps):
         t0 = time.perf_counter()
         for c_ in conns:
@@ -318,8 +327,6 @@ def run_reference(args):
         dt = time.perf_counter() - t0
         if step >= args.warmup:
             times.append(dt)
-        if time.perf_counter() - t_all0 > 420 and len(times) >= 2:
-            break
     for c_ in conns:
         c_.send(None)
     for pr in procs:
@@ -443,6 +450,8 @@ def _run_b200_on_stream(args, eng, ds, t_gen, conf, runkw, cohort, rank, local_r
     barrier()
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(res, args.dump_outputs if rank == 0 else os.path.join(args.dump_outputs, "rank%d" % rank))
     launches_per_step = res.launches
     n_pairs, n_hits, n_reads = res.n_pairs, res.n_hits, ds.reads.n_reads
     phased = int((res.calls_strict["emitted"] == 1).sum())
@@ -657,6 +666,31 @@ def _run_b200_on_stream(args, eng, ds, t_gen, conf, runkw, cohort, rank, local_r
                                        "oracle_wall_s": round(time.perf_counter() - t_fp, 1)}
                 line["parity"] = line["parity"] and len(bad) == 0
         print(json.dumps(line))
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(res, path):
+    """The host arrays of a BatchResult (what Engine.run hands its caller) as float64 .npy files, exact for their
+    int32/int64 values; a structured array gives one file per field (``tally.n_dad_reads``).  Should they exceed
+    DUMP_LIMIT bytes in all, every array keeps the same seeded sample of its last axis."""
+    arrays = {name: getattr(res, name) for name in ("seg_row_lo", "seg_pair_off", "n_het", "n_cand", "cnv_dad", "cnv_mom",
+                                                     "win", "slot_off") if getattr(res, name) is not None}
+    for name in ("tally", "calls_strict", "calls_ambiguous"):
+        a = getattr(res, name)
+        for f in a.dtype.names:
+            arrays[name + "." + f] = a[f]
+    total = sum(8 * a.size for a in arrays.values())
+    budget = DUMP_LIMIT - 4096 * len(arrays)                 # room for the .npy headers
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if total > budget:
+            n = a.shape[-1]
+            keep = np.sort(np.random.default_rng(0).choice(n, max(1, n * budget // total), replace=False))
+            a = a[..., keep]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def _k(d):

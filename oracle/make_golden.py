@@ -1,11 +1,13 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.npz + *.json by running the UNMODIFIED
-reference (from /root/reference, over oracle/fakes.py) on small seeded synthetic trios and on
-hand-written unit vectors.  Run it in the build container (the reference is not on the GPU box):
+reference (the checkout named by $UNFAZED_REFERENCE, over oracle/fakes.py) on small seeded synthetic
+trios and on hand-written unit vectors.  It needs no GPU:
 
-    python -m oracle.make_golden
+    UNFAZED_REFERENCE=/path/to/unfazed python -m oracle.make_golden
 
 The fixtures pin oracle/port.py (tests/test_oracle_golden.py, CPU) and the CUDA path
-(tests/test_gpu_golden.py, GPU) to what the reference itself produced.
+(tests/test_gpu_golden.py, GPU) to what the reference itself produced; reference_answers.json.gz
+holds the reference's answers to the CPU tests that compare the drop-in modules and the port
+with it on generated inputs.
 """
 from __future__ import annotations
 
@@ -204,7 +206,23 @@ def unit_vectors():
     print("unit vectors:", {k: len(v) for k, v in out.items()})
 
 
+def reference_answers(driver=ref_driver):
+    """The answers of ``driver`` (the reference) to the tests that compare the project with it on generated inputs:
+    every ``ANSWERS`` entry of the modules in ``tests.golden_util.ANSWER_MODULES``, into one gzip'd JSON file."""
+    import gzip
+    import importlib
+    from tests import golden_util
+    out = {}
+    for name in golden_util.ANSWER_MODULES:
+        for test, answers in importlib.import_module("tests." + name).ANSWERS.items():
+            out[test] = golden_util.canon(answers(driver))
+    with open(golden_util.ANSWERS_FILE, "wb") as raw, gzip.GzipFile(fileobj=raw, mode="wb", mtime=0) as f:
+        f.write(json.dumps(out, sort_keys=True).encode())
+    print("reference answers:", {k: len(v) for k, v in out.items()})
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     dataset_cases()
     unit_vectors()
+    reference_answers()

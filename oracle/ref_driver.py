@@ -1,9 +1,9 @@
-"""TEST INFRASTRUCTURE ONLY -- runs the UNMODIFIED reference from ``/root/reference``.
+"""TEST INFRASTRUCTURE ONLY -- runs the UNMODIFIED reference (unfazed 1.0.3) from the checkout named by
+``$UNFAZED_REFERENCE``.
 
 The reference package is imported in place (never copied) after ``oracle.fakes`` has been
-installed as ``cyvcf2``/``pysam``.  This works only where ``/root/reference`` is mounted (the build
-container); it is used to validate ``oracle/port.py`` and to generate ``tests/golden`` fixtures
-(``oracle/make_golden.py``).  Nothing under ``-m gpu``, ``smoke()`` or ``bench.py`` imports it.
+installed as ``cyvcf2``/``pysam``.  It is used to generate the ``tests/golden`` fixtures
+(``oracle/make_golden.py``); the tests themselves compare with those fixtures and never import it.
 """
 from __future__ import annotations
 
@@ -13,7 +13,7 @@ import os
 import sys
 from typing import Dict, List, Optional
 
-REFERENCE_ROOT = os.environ.get("UNFAZED_REFERENCE", "/root/reference")
+REFERENCE_ROOT = os.environ.get("UNFAZED_REFERENCE", "")
 
 # CLI defaults, reference __main__.py:75-223
 DEFAULTS = dict(
@@ -37,7 +37,7 @@ def modules():
     if _mods is not None:
         return _mods
     if not available():
-        raise RuntimeError("reference not mounted at %s" % REFERENCE_ROOT)
+        raise RuntimeError("no reference checkout at $UNFAZED_REFERENCE (%r)" % REFERENCE_ROOT)
     from . import fakes
     fakes.install()
     if REFERENCE_ROOT not in sys.path:

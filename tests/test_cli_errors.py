@@ -10,8 +10,6 @@ import pytest
 from unfazed_b200 import __main__ as cli
 from unfazed_b200 import unfazed as orch
 
-DATA = "/root/reference/test/data"
-
 
 def _write(tmp_path, name, text):
     p = tmp_path / name

@@ -1,16 +1,16 @@
-"""CPU, build container only: `summarize_record` (the final call, `unfazed/unfazed.py:162-334`) of the
-drop-in module and of the oracle port against the reference's, over random evidence records that cover
-every branch of the decision table (read-backed / allele-balance / contradictory / ambiguous /
-autophased), for several `evidence_min_ratio` values and both flags."""
+"""CPU: `summarize_record` (the final call, `unfazed/unfazed.py:162-334`) of the drop-in module and of the
+oracle port against the reference's answers (tests/golden/reference_answers.json.gz), over random evidence
+records that cover every branch of the decision table (read-backed / allele-balance / contradictory /
+ambiguous / autophased), for several `evidence_min_ratio` values and both flags."""
 import copy
+import hashlib
+import json
 import random
 
-import pytest
+from oracle import port
+from tests.golden_util import PROJECT, assert_reference_answers, canon
 
-from oracle import port, ref_driver
-
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not ref_driver.available(), reason="reference checkout not mounted")]
+N_RECORDS, N_FULL, CALLS = 4000, 250, 12         # CALLS: 3 ratios x 2 include_ambiguous x 2 verbose per record
 
 
 def _record(rng):
@@ -33,30 +33,47 @@ def _record(rng):
     return rec
 
 
-def test_summarize_record_random():
-    ref = ref_driver.modules()["unfazed"]
-    from unfazed_b200 import unfazed as new
+def _calls():
     rng = random.Random(2024)
-    seen = set()
-    for _ in range(4000):
+    for _ in range(N_RECORDS):
         rec = _record(rng)
         for ratio in (1, 3, 10):
             for amb in (False, True):
                 for verbose in (False, True):
-                    try:
-                        want = ref.summarize_record(copy.deepcopy(rec), amb, verbose, ratio)
-                    except Exception as e:
-                        with pytest.raises(type(e)):
-                            new.summarize_record(copy.deepcopy(rec), amb, verbose, ratio)
-                        continue
-                    got = new.summarize_record(copy.deepcopy(rec), amb, verbose, ratio)
-                    assert got == want, (rec, ratio, amb, verbose)
-                    got_p = port.summarize_record(copy.deepcopy(rec), amb, verbose, ratio)
-                    assert got_p == want, (rec, ratio, amb, verbose)
-                    if want:
-                        seen.add(tuple(want["evidence_types"]))
+                    yield rec, amb, verbose, ratio
+
+
+def _summaries(summarize_record):
+    """summarize_record on every call of the sweep; an exception is answered by its type name."""
+    out = []
+    for rec, amb, verbose, ratio in _calls():
+        try:
+            out.append(summarize_record(copy.deepcopy(rec), amb, verbose, ratio))
+        except Exception as e:
+            out.append({"raises": type(e).__name__})
+    return out
+
+
+def _stored(answers):
+    """The answers to the first N_FULL records in full, and a 64-bit digest of the CALLS answers to every record."""
+    answers = canon(answers)
+    digest = [hashlib.sha256(json.dumps(answers[i: i + CALLS], sort_keys=True).encode()).hexdigest()[:16]
+              for i in range(0, len(answers), CALLS)]
+    return {"full": answers[: N_FULL * CALLS], "digest": digest}
+
+
+ANSWERS = {"test_summarize_record_random": lambda ref: _stored(_summaries(ref.modules()["unfazed"].summarize_record))}
+
+
+def test_summarize_record_random():
+    for impl in (PROJECT.modules()["unfazed"], port):
+        got = _summaries(impl.summarize_record)
+        stored = _stored(got)
+        for key in ("full", "digest"):
+            assert_reference_answers("test_summarize_record_random", stored[key], key)
     # the sweep reached every kind of call the reference can make (AMBIGUOUS_BOTH is unreachable there: the
     # origin is only ever a single parent when READBACKED was appended with it)
+    seen = {tuple(w["evidence_types"]) for w in got if w and "evidence_types" in w}
     for kind in (("READBACKED",), ("ALLELE-BALANCE",), ("READBACKED", "ALLELE-BALANCE"), ("AMBIGUOUS_READBACKED",),
                  ("AMBIGUOUS_ALLELE-BALANCE",), ("AMBIGUOUS_READBACKED", "AMBIGUOUS_ALLELE-BALANCE")):
         assert kind in seen, kind

@@ -1,19 +1,21 @@
-"""CPU, build container only: the output writers. `write_vcf_output` of the drop-in against the reference's own
-(`unfazed/unfazed.py:336-440`), both over one recording cyvcf2 stand-in: same header additions, same
-phased genotypes, same UOPS / UET arrays for every variant and sample."""
+"""CPU: the output writers. `write_vcf_output` and `write_bed_output` of the drop-in against the reference's
+own (`unfazed/unfazed.py:336-515`, answers stored in tests/golden/reference_answers.json.gz): the VCF writer over
+a recording cyvcf2 stand-in (same header additions, same phased genotypes, same UOPS / UET arrays for every variant
+and sample), the BED writer's rows."""
 import copy
+import os
 import sys
+import tempfile
 import types
+from unittest import mock
 
 import numpy as np
 import pytest
 
-from oracle import port, ref_driver
+from oracle import port
+from tests.golden_util import PROJECT, assert_reference_answers
 from tests.util import port_params
 from unfazed_b200.synth import SynthConfig, make_dataset
-
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not ref_driver.available(), reason="reference checkout not mounted")]
 
 
 class _Variant:
@@ -57,8 +59,8 @@ def _cyvcf2(variants, samples, log):
     return VCF, Writer
 
 
-@pytest.mark.parametrize("include_ambiguous", [False, True])
-def test_vcf_writer_matches_reference(include_ambiguous, monkeypatch):
+def _vcf_written(ref, include_ambiguous):
+    """Header lines (the version written as V), FORMAT definitions and records the writer hands to cyvcf2."""
     ds = make_dataset(SynthConfig(dnms_per_trio=14, seed=401, coverage=20.0, n_trios=2, sv_frac=0.3, sv_max_len=20000,
                                   sex_chrom_frac=0.2, male_frac=1.0))
     records = port.Phaser(ds.sites, ds.reads, ds.pedigrees, port_params()).phase(copy.deepcopy(ds.dnms))
@@ -70,44 +72,27 @@ def test_vcf_writer_matches_reference(include_ambiguous, monkeypatch):
     for d in ds.dnms:
         vt = d["vartype"] if d["vartype"] in ("DEL", "DUP", "INV", "CNV", "DUP:TANDEM", "DEL:ME", "CPX", "CTX") else None
         variants.append(_Variant(d["chrom"], int(d["start"]), int(d["end"]), vt, len(samples), samples.index(d["kid"])))
-
-    ref_mod = ref_driver.modules()["unfazed"]
-    ref_version = ref_mod.__version__
-    log_ref, log_new = _Log(), _Log()
-    VCF, Writer = _cyvcf2(variants, samples, log_ref)
-    monkeypatch.setattr(ref_mod, "VCF", VCF)
-    monkeypatch.setattr(ref_mod, "Writer", Writer)
-    ref_mod.write_vcf_output("dnms.vcf", copy.deepcopy(records), include_ambiguous, True, "out.vcf", 10)
-
-    from unfazed_b200 import unfazed as new_mod
-    VCF2, Writer2 = _cyvcf2(variants, samples, log_new)
+    log = _Log()
+    VCF, Writer = _cyvcf2(variants, samples, log)
+    # the reference binds VCF and Writer at import, the drop-in imports cyvcf2 when called: both see the stand-in
     fake = types.ModuleType("cyvcf2")
-    fake.VCF, fake.Writer, fake.__fake__ = VCF2, Writer2, True
-    monkeypatch.setitem(sys.modules, "cyvcf2", fake)
-    new_mod.write_vcf_output("dnms.vcf", copy.deepcopy(records), include_ambiguous, True, "out.vcf", 10)
-
-    assert log_new.formats == log_ref.formats
-    assert [h.replace(new_mod.__version__, "V") for h in log_new.header] == [h.replace(ref_version, "V") for h in log_ref.header]
-    assert len(log_ref.records) == len(variants)
-    assert log_new.records == log_ref.records
-    phased = sum(1 for r in log_ref.records for g in r[3] if g[2] is True)
-    assert phased >= 3
+    fake.VCF, fake.Writer, fake.__fake__ = VCF, Writer, True
+    mod = ref.modules()["unfazed"]
+    with mock.patch.object(mod, "VCF", VCF, create=True), mock.patch.object(mod, "Writer", Writer, create=True), \
+            mock.patch.dict(sys.modules, {"cyvcf2": fake}):
+        mod.write_vcf_output("dnms.vcf", copy.deepcopy(records), include_ambiguous, True, "out.vcf", 10)
+    return {"header": [h.replace(mod.__version__, "V") for h in log.header], "formats": log.formats, "records": log.records}
 
 
-@pytest.mark.parametrize("include_ambiguous,verbose", [(False, False), (True, True), (False, True)])
-def test_bed_writer_matches_reference(include_ambiguous, verbose, tmp_path):
-    """`write_bed_output` (`unfazed.py:443-515`) on the same records: same header, same rows (the read-name
-    columns are a joined Python set in the reference, Q23: compared as sets)."""
-    from unfazed_b200 import unfazed as new_mod
+def _bed_rows(ref, include_ambiguous, verbose):
+    """The rows ``write_bed_output`` writes (the read-name columns are a joined Python set in the reference, Q23:
+    sorted)."""
     ds = make_dataset(SynthConfig(dnms_per_trio=14, seed=402, coverage=20.0, n_trios=2, sv_frac=0.3, sv_max_len=20000,
                                   sex_chrom_frac=0.2, male_frac=1.0))
     records = port.Phaser(ds.sites, ds.reads, ds.pedigrees, port_params()).phase(copy.deepcopy(ds.dnms))
-    ref_mod = ref_driver.modules()["unfazed"]
-    a, b = str(tmp_path / "ref.bed"), str(tmp_path / "new.bed")
-    ref_mod.write_bed_output(copy.deepcopy(records), include_ambiguous, verbose, a, 10)
-    new_mod.write_bed_output(copy.deepcopy(records), include_ambiguous, verbose, b, 10)
-
-    def rows(path):
+    with tempfile.TemporaryDirectory() as tmp:
+        path = os.path.join(tmp, "out.bed")
+        ref.modules()["unfazed"].write_bed_output(copy.deepcopy(records), include_ambiguous, verbose, path, 10)
         out = []
         for line in open(path).read().strip().split("\n"):
             f = line.split("\t")
@@ -115,8 +100,28 @@ def test_bed_writer_matches_reference(include_ambiguous, verbose, tmp_path):
                 f[10] = ",".join(sorted(f[10].split(",")))
                 f[12] = ",".join(sorted(f[12].split(",")))
             out.append(f)
-        return out
+    return out
 
-    ra, rb = rows(a), rows(b)
-    assert ra[0] == rb[0] and ra[0][0].startswith("#")
-    assert ra == rb and len(ra) > 3
+
+VCF_CASES = [False, True]
+BED_CASES = [(False, False), (True, True), (False, True)]
+ANSWERS = {
+    "test_vcf_writer_matches_reference": lambda ref: {str(a): _vcf_written(ref, a) for a in VCF_CASES},
+    "test_bed_writer_matches_reference": lambda ref: {"%s-%s" % c: _bed_rows(ref, *c) for c in BED_CASES},
+}
+
+
+@pytest.mark.parametrize("include_ambiguous", VCF_CASES)
+def test_vcf_writer_matches_reference(include_ambiguous):
+    got = _vcf_written(PROJECT, include_ambiguous)
+    for key in ("header", "formats", "records"):
+        assert_reference_answers("test_vcf_writer_matches_reference", got[key], str(include_ambiguous), key)
+    assert len(got["records"]) == 2 * 14                  # every variant is written: 2 trios x 14 DNMs
+    assert sum(1 for r in got["records"] for g in r[3] if g[2] is True) >= 3
+
+
+@pytest.mark.parametrize("include_ambiguous,verbose", BED_CASES)
+def test_bed_writer_matches_reference(include_ambiguous, verbose):
+    got = _bed_rows(PROJECT, include_ambiguous, verbose)
+    assert_reference_answers("test_bed_writer_matches_reference", got, "%s-%s" % (include_ambiguous, verbose))
+    assert got[0][0].startswith("#") and len(got) > 3
