@@ -101,7 +101,7 @@ typedef struct {
     uint16_t n_cigar;
     uint8_t  mapq;
     uint8_t  aux;         /* bit0 next_ref==ref, bit1 has SA tag; device only: bit6 the CIGAR is one M/= operation of l_seq bases (set by
-                             unfz_read_starts), bit7 a base of the read is not ACGT (set by unfz_expand_nlist) */
+                             unfz_read_starts), bit7 a base of the read is not ACGT (set by unfz_expand_nlist or unfz_bam_emit_planes) */
     uint8_t  qoff_hi;
     uint8_t  pad;
 } UnfzRead;
@@ -404,6 +404,64 @@ typedef struct { void* ptr; int64_t bytes; } UnfzSpan;
 int unfz_run_batch_graph(UnfzCtx*, const UnfzBatch* h_batch, const UnfzSpan* h_zero, int32_t n_zero,
                          void* h_dst, const void* d_src, int64_t d2h_bytes, void* stream);
 int unfz_batch_struct_bytes(void);      /* sizeof(UnfzBatch), for bindings to check their mirror */
+
+/* ---- BAM record decoding (csrc/bam.cu) ------------------------------------------------------------
+ * Input: inflated BAM record bytes (BGZF blocks inflated on the host, records back to back, each starting with its
+ * int32 block_size) and the byte offset of every record in that buffer.
+ *
+ * The fixed part of one record, as the parse step reads it (host and device share the code, so the two agree bit for
+ * bit).  end is htslib's bam_endpos: pos + the reference length of the CIGAR, or pos + 1 for an unmapped read or one
+ * without a reference-consuming operation.  aux: bit0 next_refID == refID, bit1 an SA tag among the aux fields (full
+ * walk over all tag types), bit7 the record is malformed (its fields overrun block_size).  name_hash: 64-bit FNV-1a of
+ * the read name without its NUL.  48 bytes. */
+#define UNFZ_BAM_AUX_BAD 0x80
+typedef struct {
+    uint64_t name_hash;
+    int32_t  ref_id;
+    int32_t  pos;
+    int32_t  end;
+    int32_t  l_seq;
+    int32_t  tlen;
+    int32_t  next_ref_id;
+    int32_t  next_pos;
+    uint16_t flag;
+    uint16_t n_cigar;
+    uint8_t  mapq;
+    uint8_t  aux;
+    uint8_t  l_name;      /* read name length including the NUL */
+    uint8_t  _pad;
+    int32_t  ref_len;     /* sum of the reference-consuming CIGAR lengths, whatever the flag (may be 0) */
+} UnfzBamRec;
+
+/* Host only (no device call): the record boundaries of `buf` by walking block_size from byte 0.  Writes at most
+ * max_records offsets, stops at a record that does not end inside the buffer and stores where the walk stopped in
+ * *end_out.  Returns the number of offsets, or -1 for a block_size below the 32 bytes of the fixed fields. */
+int64_t unfz_bam_record_offsets(const uint8_t* buf, int64_t n_bytes, int64_t max_records, int64_t* offs, int64_t* end_out);
+/* Host only: the fixed fields of n records (the same function the device parse runs).  Returns the number of malformed
+ * records (aux bit7). */
+int64_t unfz_bam_parse_host(const uint8_t* buf, int64_t n_bytes, const int64_t* offs, int64_t n, UnfzBamRec* out);
+/* Host only: dst <- the byte ranges [src[i], src[i] + len[i]) of buf back to back. */
+int unfz_bam_gather_host(const uint8_t* buf, const int64_t* src, const int64_t* len, int64_t n, uint8_t* dst);
+
+/* Device: unfz_bam_parse_host on the GPU, one thread per record (buf, offs, out in device memory). */
+int unfz_bam_parse(UnfzCtx*, const uint8_t* buf, int64_t n_bytes, const int64_t* offs, int64_t n, UnfzBamRec* out,
+                   void* stream);
+/* Device: mate indices of n output reads as packers._mate_join defines them (same name, other segment bit, primary,
+ * first in block order; -1 for an unpaired read or one whose mate is unmapped).  order: a stable sort of the reads by
+ * (key_blk, key_hash) -- block and 64-bit name hash; flag: SAM flags; buf/src: the records, whose name bytes are compared
+ * for every joined pair.  mate[i] = -2 leaves read i to the host: its candidate's name differs (a hash collision) or it
+ * is its own candidate (both segment bits set). */
+int unfz_bam_mate_join(UnfzCtx*, const int64_t* order, const int64_t* key_hash, const int32_t* key_blk, const int32_t* flag,
+                       int64_t n, const uint8_t* buf, const int64_t* src, int32_t* mate, void* stream);
+/* Device: the CIGAR words of the output reads.  reads->hdr holds the headers (cigar_off, n_cigar); src[r] is the byte
+ * offset in buf of the record output read r is decoded from. */
+int unfz_bam_emit_cigar(UnfzCtx*, const UnfzReadCols* reads, const uint8_t* buf, const int64_t* src, void* stream);
+/* Device: the base planes of the output reads -- 2-bit bases (seq2), the low-quality plane of quality < min_bq (a
+ * quality string starting with 0xFF counts as all zeros), and the non-ACGT plane (nmask) with aux bit7 of the reads that
+ * own such a base: the device state unfz_expand_nlist leaves, so run it after unfz_read_starts (which clears aux bit7).
+ * One thread per 32 output bases; the planes must be zeroed up to the padding DeviceReads gives them. */
+int unfz_bam_emit_planes(UnfzCtx*, const UnfzReadCols* reads, const uint8_t* buf, const int64_t* src, int32_t min_bq,
+                         void* stream);
 
 #ifdef __cplusplus
 }

@@ -89,6 +89,12 @@ TALLY_DTYPE = np.dtype([
 CALL_DTYPE = np.dtype([("origin", "<i4"), ("evidence_count", "<i4"), ("evidence_types", "<i4"), ("emitted", "<i4")])
 RSUM_DTYPE = np.dtype([("end", "<i4"), ("fmark", "<i4"), ("flags", "<u2"), ("cnt", "<u2"), ("hoff", "<u4"),
                        ("start", "<i4"), ("mate", "<i4"), ("row_lb", "<i4"), ("pad", "<i4")])
+# UnfzBamRec: the fixed fields of one BAM record (csrc/bam.cu)
+BAM_REC_DTYPE = np.dtype([("name_hash", "<u8"), ("ref_id", "<i4"), ("pos", "<i4"), ("end", "<i4"), ("l_seq", "<i4"),
+                          ("tlen", "<i4"), ("next_ref_id", "<i4"), ("next_pos", "<i4"), ("flag", "<u2"), ("n_cigar", "<u2"),
+                          ("mapq", "u1"), ("aux", "u1"), ("l_name", "u1"), ("_pad", "u1"), ("ref_len", "<i4")])
+BAM_AUX_BAD = 0x80
+assert BAM_REC_DTYPE.itemsize == 48
 assert SEG_DTYPE.itemsize == 32 and DNM_DTYPE.itemsize == 48 and RSUM_DTYPE.itemsize == 32
 
 # constants of include/unfazed_sm100.h
@@ -137,6 +143,13 @@ SYMBOLS = {
     "unfz_insert_size_work_bytes": (c_int64, []),
     "unfz_insert_size_order_stats": (C.c_int, [_P, C.POINTER(ReadCols), _P, _P, c_int32, c_int32, _P, _P, _P, _P]),
     "unfz_summarize": (C.c_int, [_P, _P, c_int32, _P, _P, _P, _P, C.POINTER(Params), _P, _P, _P]),
+    "unfz_bam_record_offsets": (c_int64, [_P, c_int64, c_int64, _P, _P]),
+    "unfz_bam_parse_host": (c_int64, [_P, c_int64, _P, c_int64, _P]),
+    "unfz_bam_gather_host": (C.c_int, [_P, _P, _P, c_int64, _P]),
+    "unfz_bam_parse": (C.c_int, [_P, _P, c_int64, _P, c_int64, _P, _P]),
+    "unfz_bam_mate_join": (C.c_int, [_P, _P, _P, _P, _P, c_int64, _P, _P, _P, _P]),
+    "unfz_bam_emit_cigar": (C.c_int, [_P, C.POINTER(ReadCols), _P, _P, _P]),
+    "unfz_bam_emit_planes": (C.c_int, [_P, C.POINTER(ReadCols), _P, _P, c_int32, _P]),
 }
 
 _lib = None

@@ -1,8 +1,10 @@
 """Where the drop-in modules get their columnar tables from.
 
 * ``*.npz`` written by ``tableio.save_tables`` (our native cache of decoded inputs), or
-* the sites VCF/BCF through ``cyvcf2`` and the kids' BAM/CRAMs through ``pysam`` -- imported
-  lazily, so the package works without them as long as tables are supplied -- decoded only around
+* indexed BAM files (``*.bam`` with a ``.bai``) through ``bamio.py``, natively -- no pysam needed, and with an
+  engine the bulk of the records is decoded on the GPU, or
+* the sites VCF/BCF through ``cyvcf2`` and the kids' other alignment files (CRAM, unindexed BAM) through ``pysam``
+  -- imported lazily, so the package works without them as long as tables are supplied -- decoded only around
   the DNMs and packed by ``packers.py``.
 
 Tables are cached per (file, request) for the lifetime of the process, like the reference's
@@ -10,11 +12,12 @@ Tables are cached per (file, request) for the lifetime of the process, like the 
 """
 from __future__ import annotations
 
+import os
 from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 
-from . import packers
+from . import bamio, packers
 from .plan import strip_chr
 from .schema import ReadTable, SiteTable
 from .tableio import load_tables
@@ -66,8 +69,33 @@ def load_sites(vcf_name: str, dnms: List[dict], pedigrees: dict, search_dist: in
     return packers.pack_sites(VCF(vcf_name), trios, regions)
 
 
-def load_reads(dnms: List[dict], search_dist: int, readlen: int, insert_size_max_sample: int) -> Optional[ReadTable]:
-    """One ReadTable for all kids of the DNM list (their ``bam`` entries name the files)."""
+def is_indexed_bam(name: str) -> bool:
+    """An existing ``*.bam`` file with a ``.bai`` next to it: read natively by ``bamio``."""
+    return name.endswith(".bam") and os.path.isfile(name) and bamio.index_path(name) is not None
+
+
+def _regions(dnms, heads, has_contig, search_dist, readlen):
+    regions: Dict[str, Dict[str, List[Tuple[int, int]]]] = {}
+    for d in dnms:
+        kid = d["kid"]
+        h = heads[kid]
+        cul = int(np.percentile(np.abs(h - 2 * readlen), 99.5)) if h.shape[0] else 0
+        margin = max(search_dist, cul) + 2 * readlen + 2
+        chrom = d["chrom"]
+        if not has_contig(kid, chrom):
+            chrom = _toggle(chrom)
+        for p in {int(d["start"]), int(d["end"])}:
+            regions.setdefault(kid, {}).setdefault(chrom, []).append((p - margin, p + margin))
+    return regions
+
+
+def load_reads(dnms: List[dict], search_dist: int, readlen: int, insert_size_max_sample: int, engine=None,
+               min_gt_qual=20) -> Optional[ReadTable]:
+    """One ReadTable for all kids of the DNM list (their ``bam`` entries name the files).
+
+    When every file is an indexed BAM it is read by ``bamio`` (no pysam).  With ``engine`` the bases and qualities
+    are then decoded on that engine's GPU: the table has no ``qual`` / ``seq2`` and carries its ``DeviceReads`` for
+    the base-quality threshold of ``min_gt_qual`` (``table.device_reads``).  Every other input goes through pysam."""
     bam_of: Dict[str, str] = {}
     for d in dnms:
         bam_of.setdefault(d["kid"], d["bam"])
@@ -83,8 +111,15 @@ def load_reads(dnms: List[dict], search_dist: int, readlen: int, insert_size_max
     reg = [_registry[n][1] for n in names if n in _registry and _registry[n][1] is not None]
     if reg and all(r is reg[0] for r in reg) and len(reg) == len(names):
         return reg[0]
+    if all(is_indexed_bam(n) for n in names):
+        files = {kid: bamio.BamFile(name) for kid, name in bam_of.items()}
+        heads = {kid: f.head_tlen(insert_size_max_sample + 1) for kid, f in files.items()}
+        regions = _regions(dnms, heads, lambda kid, c: c in files[kid].tids, search_dist, readlen)
+        table = bamio.read_regions(files, regions, engine=engine, min_gt_qual=min_gt_qual)
+        table.head_tlen = heads
+        return table
     import pysam
-    bams, regions = {}, {}
+    bams = {}
     for kid, name in bam_of.items():
         cram_ref = next((d.get("cram_ref") for d in dnms if d["kid"] == kid), None)
         bam = pysam.AlignmentFile(name, "rc", reference_filename=cram_ref) if name[-4:] == "cram" else pysam.AlignmentFile(name, "rb")
@@ -99,18 +134,15 @@ def load_reads(dnms: List[dict], search_dist: int, readlen: int, insert_size_max
             if i >= insert_size_max_sample:
                 break
         heads[kid] = np.array(tl, dtype=np.int64)
-    for d in dnms:
-        kid = d["kid"]
-        h = heads[kid]
-        cul = int(np.percentile(np.abs(h - 2 * readlen), 99.5)) if h.shape[0] else 0
-        margin = max(search_dist, cul) + 2 * readlen + 2
-        chrom = d["chrom"]
+
+    def has_contig(kid, chrom):
         try:
             bams[kid].fetch(chrom, 0, 1)
         except ValueError:
-            chrom = _toggle(chrom)
-        for p in {int(d["start"]), int(d["end"])}:
-            regions.setdefault(kid, {}).setdefault(chrom, []).append((p - margin, p + margin))
+            return False
+        return True
+
+    regions = _regions(dnms, heads, has_contig, search_dist, readlen)
     table = packers.pack_reads(bams, regions)
     table.head_tlen = heads
     return table

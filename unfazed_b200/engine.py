@@ -98,6 +98,9 @@ class PackedReads:
     carry quality bytes (synthetic data, the oracle's fixtures) are reduced here."""
 
     def __init__(self, table: ReadTable, min_bq: int, pin: bool = False):
+        if table.qual is None:
+            raise ValueError("PackedReads needs the quality bytes and bases of the table; this ReadTable was decoded on "
+                             "the device (bamio.read_regions(engine=...)): use its device_reads")
         self.table, self.min_bq = table, int(min_bq)
         conv = (lambda a: torch.from_numpy(np.ascontiguousarray(a)).pin_memory().numpy()) if pin else np.ascontiguousarray
         self.hdr = conv(table.hdr.view(np.uint8).reshape(-1))
@@ -130,6 +133,47 @@ class DeviceReads:
         self.nidx = up(packed.nidx)
         self.nmask = torch.zeros(self.lowq.shape[0], dtype=torch.uint8, device=device)
         self.h2d_bytes = packed.nbytes
+        st = self._bind_cols(table, device, nq)
+        if engine is not None:
+            engine._check(engine.lib.unfz_read_starts(engine.ctx, C.byref(self.cols), self.start.data_ptr(), st), "read_starts")
+        else:
+            self.start.copy_(self.hdr.view(torch.int32).view(-1, 8)[:, 0]) if table.n_reads else None
+        if engine is not None and packed.nidx.shape[0]:
+            engine._check(engine.lib.unfz_expand_nlist(engine.ctx, C.byref(self.cols), self.hdr.data_ptr(), self.nmask.data_ptr(),
+                                                       self.nidx.data_ptr(), int(packed.nidx.shape[0]), st), "expand_nlist")
+
+    @classmethod
+    def from_bam(cls, table: ReadTable, device: torch.device, min_bq: int, engine: "Engine", dbuf: torch.Tensor,
+                 dsrc: torch.Tensor) -> "DeviceReads":
+        """The read columns decoded on the device from inflated BAM records (``dbuf``; ``dsrc[r]``: byte offset of the
+        record of read r): the headers of the host table go up, the CIGAR words and the three base planes are written
+        by unfz_bam_emit_cigar / unfz_bam_emit_planes, exactly as an upload of the host-decoded table leaves them.
+        One difference in the path, not in the result: there is no sparse index list of the non-ACGT bases
+        (``nidx`` stays empty, unfz_expand_nlist does not run) -- the planes kernel owns whole 32-base words, so it
+        writes the ``nmask`` words and sets aux bit7 of their reads itself; nothing downstream reads ``nidx``."""
+        self = cls.__new__(cls)
+        self.table, self.min_bq = table, int(min_bq)
+        self.n_reads = table.n_reads
+        self.max_l_seq = table.max_l_seq()
+        up = lambda a: _to_device(a, device, False)
+        self.blk_off = up(np.ascontiguousarray(table.blk_off.astype(np.int64)))
+        self.hdr = up(table.hdr.view(np.uint8).reshape(-1))
+        nq = table.n_qual
+        plane_bytes = (nq + 7) // 8
+        self.cigar = torch.empty((int(table.cigar.shape[0]),), dtype=torch.int32, device=device)
+        self.lowq = torch.zeros((plane_bytes + 48 + (-plane_bytes) % 4,), dtype=torch.uint8, device=device)
+        self.seq2 = torch.zeros(((nq + 3) // 4 + 16,), dtype=torch.uint8, device=device)
+        self.nidx = torch.zeros((0,), dtype=torch.int64, device=device)
+        self.nmask = torch.zeros(self.lowq.shape[0], dtype=torch.uint8, device=device)
+        self.h2d_bytes = int(table.hdr.nbytes + table.blk_off.nbytes)
+        st = self._bind_cols(table, device, nq)
+        lib, ctx, c = engine.lib, engine.ctx, C.byref(self.cols)
+        engine._check(lib.unfz_bam_emit_cigar(ctx, c, dbuf.data_ptr(), dsrc.data_ptr(), st), "bam_emit_cigar")
+        engine._check(lib.unfz_read_starts(ctx, c, self.start.data_ptr(), st), "read_starts")
+        engine._check(lib.unfz_bam_emit_planes(ctx, c, dbuf.data_ptr(), dsrc.data_ptr(), int(min_bq), st), "bam_emit_planes")
+        return self
+
+    def _bind_cols(self, table, device, nq):
         self.blk_sblk = torch.full((max(table.n_blocks, 1),), -1, dtype=torch.int32, device=device)
         self.blk_cul = torch.zeros((max(table.n_blocks, 1),), dtype=torch.float64, device=device)
         c = L.ReadCols()
@@ -141,19 +185,124 @@ class DeviceReads:
         c.lowq, c.nmask = self.lowq.data_ptr(), self.nmask.data_ptr()
         c.n_qual, c.n_cigar = nq, int(table.cigar.shape[0])
         self.cols = c
-        st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-        if engine is not None:
-            engine._check(engine.lib.unfz_read_starts(engine.ctx, C.byref(c), self.start.data_ptr(), st), "read_starts")
-        else:
-            self.start.copy_(self.hdr.view(torch.int32).view(-1, 8)[:, 0]) if table.n_reads else None
-        if engine is not None and packed.nidx.shape[0]:
-            engine._check(engine.lib.unfz_expand_nlist(engine.ctx, C.byref(c), self.hdr.data_ptr(), self.nmask.data_ptr(),
-                                                       self.nidx.data_ptr(), int(packed.nidx.shape[0]), st), "expand_nlist")
+        return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
     @property
     def nbytes(self) -> int:
         """Bytes that crossed PCIe for these columns."""
         return self.h2d_bytes
+
+
+class BamDecoder:
+    """Device side of ``bamio.read_regions(engine=...)``: the inflated record bytes go up once (pinned), the fixed
+    fields are parsed there (unfz_bam_parse) and come back for the host's selection, and the bulk columns are emitted
+    on the device.  The record bytes stay resident, so the planes of another base-quality threshold are decoded again
+    from them (``device_reads``) without touching the file.  Resident means every record of the fetched chunks, not
+    only the selected reads (1.5 GB with offsets for the 4.4 M reads of 2000 c2 DNMs, profiles/r3_bam_decode_c2_2000dnms.json);
+    with several files the parts are concatenated once on the device, which briefly holds both copies."""
+
+    def __init__(self, engine: "Engine"):
+        self.engine = engine
+        self.parts: List[torch.Tensor] = []
+        self.dbuf = self.dsrc = self.table = None
+        self._reads: Optional[DeviceReads] = None
+        self.h2d_bytes = 0
+        self.timings_ms: Dict[str, float] = {}
+
+    def _time(self, name, e0, e1):
+        self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
+
+    def parse(self, buf: np.ndarray, offs: np.ndarray, part: int) -> np.ndarray:
+        eng = self.engine
+        n = int(offs.shape[0])
+        with eng.on_stream():
+            st = torch.cuda.current_stream(eng.device)
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
+            e[0].record(st)
+            d = _to_device(np.ascontiguousarray(buf), eng.device, True, 16)
+            doffs = _to_device(np.ascontiguousarray(offs, dtype=np.int64), eng.device, True)
+            e[1].record(st)
+            out = torch.empty((max(n, 1) * L.BAM_REC_DTYPE.itemsize,), dtype=torch.uint8, device=eng.device)
+            eng._check(eng.lib.unfz_bam_parse(eng.ctx, d.data_ptr(), int(buf.shape[0]), doffs.data_ptr(), n, out.data_ptr(),
+                                              C.c_void_p(st.cuda_stream)), "bam_parse")
+            e[2].record(st)
+            rec = out[: n * L.BAM_REC_DTYPE.itemsize].cpu().numpy().view(L.BAM_REC_DTYPE)
+        self._time("h2d_records", e[0], e[1])
+        self._time("parse", e[1], e[2])
+        self.h2d_bytes += int(buf.nbytes + offs.nbytes)
+        bad = int(np.count_nonzero(rec["aux"] & L.BAM_AUX_BAD))
+        if bad:
+            raise ValueError("%d malformed BAM record(s): fields or aux tags overrun block_size" % bad)
+        self.parts.append(d[: int(buf.shape[0])])
+        return rec
+
+    def prepare(self, src: np.ndarray) -> None:
+        """The parts as one device buffer and the record offset of every output read (``src``: byte offsets in the parts
+        back to back)."""
+        eng = self.engine
+        with eng.on_stream():
+            st = torch.cuda.current_stream(eng.device)
+            e0 = torch.cuda.Event(enable_timing=True)
+            e0.record(st)
+            self.dbuf = torch.cat(self.parts) if len(self.parts) != 1 else self.parts[0]
+            if self.dbuf.numel() == 0:
+                self.dbuf = torch.zeros((16,), dtype=torch.uint8, device=eng.device)
+            self.parts = [self.dbuf]
+            self.dsrc = _to_device(np.ascontiguousarray(src, dtype=np.int64), eng.device, True)
+            self.h2d_bytes += int(src.nbytes)
+            e1 = torch.cuda.Event(enable_timing=True)
+            e1.record(st)
+        e1.synchronize()
+        self._time("concat_src", e0, e1)
+
+    def mate_join(self, name_hash: np.ndarray, blk: np.ndarray, flag: np.ndarray) -> np.ndarray:
+        """Mate index of every output read (after ``prepare``), as packers._mate_join defines it inside each block:
+        the reads are ordered by (block, name hash) with torch's stable sort, unfz_bam_mate_join picks the first primary
+        read of the other segment in each group and compares the name bytes of every joined pair; -2 marks the reads
+        left to the host (a hash collision, or a read that is its own candidate)."""
+        eng = self.engine
+        n = int(name_hash.shape[0])
+        if n == 0:
+            return np.zeros(0, dtype=np.int64)
+        with eng.on_stream():
+            st = torch.cuda.current_stream(eng.device)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(st)
+            dh = _to_device(np.ascontiguousarray(name_hash).view(np.int64), eng.device, True)
+            db = _to_device(np.ascontiguousarray(blk, dtype=np.int32), eng.device, True)
+            df = _to_device(np.ascontiguousarray(flag, dtype=np.int32), eng.device, True)
+            o1 = torch.sort(dh, stable=True).indices
+            order = o1[torch.sort(db[o1], stable=True).indices].contiguous()
+            mate = torch.empty((n,), dtype=torch.int32, device=eng.device)
+            eng._check(eng.lib.unfz_bam_mate_join(eng.ctx, order.data_ptr(), dh.data_ptr(), db.data_ptr(), df.data_ptr(), n,
+                                                  self.dbuf.data_ptr(), self.dsrc.data_ptr(), mate.data_ptr(),
+                                                  C.c_void_p(st.cuda_stream)), "bam_mate_join")
+            e1.record(st)
+            out = mate.cpu().numpy().astype(np.int64)
+        self._time("mate_join", e0, e1)
+        self.h2d_bytes += 16 * n
+        return out
+
+    def emit(self, table: ReadTable, min_gt_qual) -> DeviceReads:
+        """The DeviceReads of ``table`` (after ``prepare``)."""
+        self.table = table
+        return self.device_reads(min_gt_qual)
+
+    def device_reads(self, min_gt_qual=20) -> DeviceReads:
+        """DeviceReads with the low-quality plane of ``min_gt_qual`` (the last one is kept)."""
+        mb = min_base_qual(min_gt_qual)
+        if self._reads is None or self._reads.min_bq != mb:
+            self._reads = None
+            eng = self.engine
+            with eng.on_stream():
+                st = torch.cuda.current_stream(eng.device)
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record(st)
+                self._reads = DeviceReads.from_bam(self.table, eng.device, mb, eng, self.dbuf, self.dsrc)
+                e1.record(st)
+            e1.synchronize()
+            self._time("emit", e0, e1)
+        return self._reads
 
 
 def _to_device(a: np.ndarray, device, pin: bool, pad: int = 0) -> torch.Tensor:
@@ -370,6 +519,16 @@ class Engine:
         ``min_gt_qual`` first) or a PackedReads (copied as it is)."""
         with self.on_stream():
             return DeviceReads(table, self.device, pin, min_base_qual(min_gt_qual), self)
+
+    def bam_decoder(self) -> BamDecoder:
+        """A device decoder for one ``bamio.read_regions`` load."""
+        return BamDecoder(self)
+
+    def decode_bam(self, paths, regions, head_reads: int = 0, min_gt_qual=20) -> DeviceReads:
+        """Indexed BAM files -> DeviceReads, the bulk of the records decoded on this GPU (``bamio.read_regions``).
+        ``.table`` is the host half: headers, CIGAR, names, block layout, head template lengths; no bases."""
+        from . import bamio
+        return bamio.read_regions(paths, regions, head_reads=head_reads, engine=self, min_gt_qual=min_gt_qual).device_reads
 
     def pack_reads(self, table: ReadTable, min_gt_qual=20, pin: bool = True) -> PackedReads:
         return PackedReads(table, min_base_qual(min_gt_qual), pin)

@@ -104,6 +104,10 @@ class BatchPhaser:
         mb = min_base_qual(min_gt_qual)
         if self._dreads is None or self._dreads.min_bq != mb:
             self._dreads = None                      # release the old planes first
+            if self.reads.qual is None:
+                # decoded on the device: the planes of this threshold are emitted again from the resident records
+                self._dreads = self.reads.device_source.device_reads(min_gt_qual)
+                return self._dreads
             src = self.packed if (self.packed is not None and self.packed.min_bq == mb) else self.reads
             self._dreads = self.engine.upload_reads(src, min_gt_qual=min_gt_qual)
         return self._dreads

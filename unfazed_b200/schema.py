@@ -156,10 +156,23 @@ class ReadTable:
     qual: np.ndarray                            # u8[Q]
     seq2: np.ndarray                            # u8[ceil(Q/4)], base i at bits 2*(i&3) of byte i>>2
     names: Optional[List[str]] = None           # per read; None -> synthesized from pair id
+    # a table whose bases and qualities were decoded on the device only (bamio.read_regions(engine=...)) has
+    # qual = seq2 = None and records its number of query bases here
+    n_bases: Optional[int] = None
 
     @property
     def n_reads(self) -> int:
         return int(self.hdr.shape[0])
+
+    @property
+    def n_qual(self) -> int:
+        """Number of query bases (the length of the quality / base columns)."""
+        return int(self.n_bases) if self.qual is None else int(self.qual.shape[0])
+
+    def _need_bases(self, what: str) -> None:
+        if self.qual is None:
+            raise ValueError("%s needs the quality bytes: this ReadTable was decoded on the device and carries no "
+                             "qual / seq2 columns (use its device_reads, or read the file with engine=None)" % what)
 
     def max_l_seq(self) -> int:
         """Longest read (cached: a pass over the strided header field costs tens of ms at 20 M reads)."""
@@ -216,6 +229,7 @@ class ReadTable:
         """One bit per query base, bit i&7 of byte i>>3: ``(qual & 0x7f) < min_bq``.  This is what the
         device gets instead of the quality bytes -- every base-quality test of the path is this one
         comparison (reference read_collector.py:44-46, :123, :281-284)."""
+        self._need_bases("lowq_plane")
         Q = int(self.qual.shape[0])
         out = np.zeros((Q + 7) // 8, dtype=np.uint8)
         for a in range(0, Q, chunk):
@@ -225,6 +239,7 @@ class ReadTable:
 
     def n_index(self, chunk: int = 1 << 26) -> np.ndarray:
         """Sorted base indices of the non-ACGT bases (quality bit7)."""
+        self._need_bases("n_index")
         Q = int(self.qual.shape[0])
         parts = [np.flatnonzero(self.qual[a: a + chunk] & QUAL_ESCAPE) + a for a in range(0, Q, chunk)]
         return np.concatenate(parts).astype(np.int64) if parts else np.zeros(0, dtype=np.int64)
@@ -245,9 +260,13 @@ class ReadTable:
 
     def validate(self) -> None:
         assert self.hdr.dtype == READ_HDR
-        assert self.cigar.dtype == np.uint32 and self.qual.dtype == np.uint8
-        assert self.seq2.dtype == np.uint8
-        assert self.seq2.shape[0] * 4 >= self.qual.shape[0]
+        assert self.cigar.dtype == np.uint32
+        if self.qual is None:
+            assert self.seq2 is None and self.n_bases is not None
+            assert self.n_bases == int(self.hdr["l_seq"].astype(np.int64).sum())
+        else:
+            assert self.qual.dtype == np.uint8 and self.seq2.dtype == np.uint8
+            assert self.seq2.shape[0] * 4 >= self.qual.shape[0]
         assert self.blk_off[0] == 0 and self.blk_off[-1] == self.n_reads
         for b in range(self.n_blocks):
             s = self.hdr["start"][self.blk_off[b]: self.blk_off[b + 1]]

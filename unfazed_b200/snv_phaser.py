@@ -79,8 +79,10 @@ def run_batch(snvs, svs, pedigrees, sites, threads, build, no_extended, multirea
     from .phaser import BatchPhaser
     dnms = list(svs) + list(snvs)
     site_table = datasource.load_sites(sites, dnms, pedigrees, search_dist)
-    read_table = datasource.load_reads(dnms, search_dist, readlen, insert_size_max_sample)
-    bp = BatchPhaser(get_engine(), site_table, read_table, pedigrees)
+    # indexed BAM inputs are decoded on the engine's GPU; the table then comes with its device columns
+    read_table = datasource.load_reads(dnms, search_dist, readlen, insert_size_max_sample, engine=get_engine(),
+                                       min_gt_qual=min_gt_qual)
+    bp = BatchPhaser(get_engine(), site_table, read_table, pedigrees, dreads=getattr(read_table, "device_reads", None))
     try:
         res, layout = bp.run(snvs, svs, threads=threads, build=build, no_extended=no_extended,
                              multiread_proc_min=multiread_proc_min, ab_homref=ab_homref, ab_homalt=ab_homalt,
