@@ -463,6 +463,67 @@ int unfz_bam_emit_cigar(UnfzCtx*, const UnfzReadCols* reads, const uint8_t* buf,
 int unfz_bam_emit_planes(UnfzCtx*, const UnfzReadCols* reads, const uint8_t* buf, const int64_t* src, int32_t min_bq,
                          void* stream);
 
+/* ---- VCF text decoding (csrc/vcf.cu) ---------------------------------------------------------------
+ * Input: the inflated text of the BGZF chunks of a tabix region query (whole lines, each ending in '\n').
+ *
+ * The fixed fields of one line, as the parse step reads it.  Offsets and lengths are relative to the line start;
+ * line_len excludes the '\n' (and a '\r' before it).  rend is the end tabix indexes the record by: INFO END when it is
+ * a number above pos0, else pos0 + ref_len.  n_alt: the ALT count (0 for ALT '.').  slot: the FORMAT index of GT, GQ,
+ * AD, RO and AO, or -1.  fmt_off = -1: no FORMAT column.  flags: UNFZ_VCF_SIMPLE (one ALT of one base, REF of one base,
+ * ALT not '*'), UNFZ_VCF_BAD (fewer than 8 columns, POS not a positive int32, END overflow).  chrom_hash: 32-bit FNV-1a
+ * of CHROM.  64 bytes. */
+#define UNFZ_VCF_SIMPLE 0x01
+#define UNFZ_VCF_BAD 0x80
+/* per-cell status bits of the sample decode */
+#define UNFZ_VCF_CELL_HOST 0x01   /* GQ is a float off the exact fast path: gq holds the int32 line offset of its text */
+#define UNFZ_VCF_CELL_BAD 0x02    /* a GT / GQ / AD / RO / AO value is malformed or overflows int32 */
+typedef struct {
+    int64_t  line_off;    /* byte offset of the line in the text */
+    int32_t  line_len;
+    int32_t  pos0;        /* POS - 1 */
+    int32_t  rend;
+    int32_t  chrom_len;
+    uint32_t chrom_hash;
+    int32_t  ref_off, ref_len;
+    int32_t  alt_off, alt_len;
+    int32_t  fmt_off, fmt_len;
+    int32_t  n_alt;
+    int8_t   slot[5];     /* GT GQ AD RO AO */
+    uint8_t  ref0;        /* first byte of REF (0 when empty) */
+    uint8_t  flags;
+    uint8_t  _pad;
+} UnfzVcfRec;
+
+/* Host only: the positions of the '\n' bytes of buf (at most cap of them).  Returns their number, or -1 when cap is too
+ * small.  The same per-16-byte-chunk code as the device pass. */
+int64_t unfz_vcf_line_ends_host(const uint8_t* buf, int64_t n_bytes, int64_t cap, int64_t* ends);
+/* Host only: the fixed fields of n_lines lines (line i spans ends[i-1] + 1 .. ends[i]).  Returns the number of lines
+ * with UNFZ_VCF_BAD. */
+int64_t unfz_vcf_parse_host(const uint8_t* buf, const int64_t* ends, int64_t n_lines, UnfzVcfRec* out);
+/* Host only: the genotype fields of the selected lines sel[0..n_sel) (indices into recs).  slot_of[s]: the member column
+ * of sample s, or -1 (n_samples entries).  Outputs are [n_sel][n_members]: gt (cyvcf2 gt_types), gq (GQ as float32,
+ * -1 missing), rd (AD[0], or RO), ad (the sum of AD[1:], or of AO; -1 missing) and status (UNFZ_VCF_CELL_*); cells of
+ * members without a column stay missing.  gq_float: the header declares GQ as Float (else Integer).  max_digits (<= 15):
+ * significant digits a float may have on the fast path (0 sends every float to the host).  line_bad[i] = 1: line i has
+ * more sample columns than n_samples. */
+int unfz_vcf_samples_host(const uint8_t* buf, const UnfzVcfRec* recs, const int64_t* sel, int64_t n_sel,
+                          const int32_t* slot_of, int32_t n_samples, int32_t n_members, int32_t gq_float, int32_t max_digits,
+                          uint8_t* gt, float* gq, int32_t* rd, int32_t* ad, uint8_t* status, uint8_t* line_bad);
+/* Number of 16-byte chunks of n_bytes: the length of the newline-count array (and of its scan, plus one). */
+int64_t unfz_vcf_chunks(int64_t n_bytes);
+
+/* Device: newline count of every 16-byte chunk of buf (cnt: unfz_vcf_chunks(n_bytes) entries). */
+int unfz_vcf_line_count(UnfzCtx*, const uint8_t* buf, int64_t n_bytes, uint32_t* cnt, void* stream);
+/* Device: the newline positions; at: the exclusive scan of the counts (unfz_exclusive_scan_u32, chunks + 1 entries). */
+int unfz_vcf_line_write(UnfzCtx*, const uint8_t* buf, int64_t n_bytes, const uint32_t* at, int64_t* ends, void* stream);
+/* Device: unfz_vcf_parse_host, one thread per line. */
+int unfz_vcf_parse(UnfzCtx*, const uint8_t* buf, const int64_t* ends, int64_t n_lines, UnfzVcfRec* out, void* stream);
+/* Device: unfz_vcf_samples_host, one warp per selected line.  buf must be 16-byte aligned and readable 16 bytes past
+ * its end. */
+int unfz_vcf_samples(UnfzCtx*, const uint8_t* buf, const UnfzVcfRec* recs, const int64_t* sel, int64_t n_sel,
+                     const int32_t* slot_of, int32_t n_samples, int32_t n_members, int32_t gq_float, int32_t max_digits,
+                     uint8_t* gt, float* gq, int32_t* rd, int32_t* ad, uint8_t* status, uint8_t* line_bad, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -95,6 +95,13 @@ BAM_REC_DTYPE = np.dtype([("name_hash", "<u8"), ("ref_id", "<i4"), ("pos", "<i4"
                           ("mapq", "u1"), ("aux", "u1"), ("l_name", "u1"), ("_pad", "u1"), ("ref_len", "<i4")])
 BAM_AUX_BAD = 0x80
 assert BAM_REC_DTYPE.itemsize == 48
+# UnfzVcfRec: the fixed fields of one VCF line (csrc/vcf.cu)
+VCF_REC_DTYPE = np.dtype([("line_off", "<i8"), ("line_len", "<i4"), ("pos0", "<i4"), ("rend", "<i4"), ("chrom_len", "<i4"),
+                          ("chrom_hash", "<u4"), ("ref_off", "<i4"), ("ref_len", "<i4"), ("alt_off", "<i4"),
+                          ("alt_len", "<i4"), ("fmt_off", "<i4"), ("fmt_len", "<i4"), ("n_alt", "<i4"), ("slot", "i1", (5,)),
+                          ("ref0", "u1"), ("flags", "u1"), ("_pad", "u1")])
+VCF_SIMPLE, VCF_BAD, VCF_CELL_HOST, VCF_CELL_BAD = 0x01, 0x80, 0x01, 0x02
+assert VCF_REC_DTYPE.itemsize == 64
 assert SEG_DTYPE.itemsize == 32 and DNM_DTYPE.itemsize == 48 and RSUM_DTYPE.itemsize == 32
 
 # constants of include/unfazed_sm100.h
@@ -150,6 +157,15 @@ SYMBOLS = {
     "unfz_bam_mate_join": (C.c_int, [_P, _P, _P, _P, _P, c_int64, _P, _P, _P, _P]),
     "unfz_bam_emit_cigar": (C.c_int, [_P, C.POINTER(ReadCols), _P, _P, _P]),
     "unfz_bam_emit_planes": (C.c_int, [_P, C.POINTER(ReadCols), _P, _P, c_int32, _P]),
+    "unfz_vcf_line_ends_host": (c_int64, [_P, c_int64, c_int64, _P]),
+    "unfz_vcf_parse_host": (c_int64, [_P, _P, c_int64, _P]),
+    "unfz_vcf_samples_host": (C.c_int, [_P, _P, _P, c_int64, _P, c_int32, c_int32, c_int32, c_int32, _P, _P, _P, _P, _P, _P]),
+    "unfz_vcf_chunks": (c_int64, [c_int64]),
+    "unfz_vcf_line_count": (C.c_int, [_P, _P, c_int64, _P, _P]),
+    "unfz_vcf_line_write": (C.c_int, [_P, _P, c_int64, _P, _P, _P]),
+    "unfz_vcf_parse": (C.c_int, [_P, _P, _P, c_int64, _P, _P]),
+    "unfz_vcf_samples": (C.c_int, [_P, _P, _P, _P, c_int64, _P, c_int32, c_int32, c_int32, c_int32, _P, _P, _P, _P, _P, _P,
+                                   _P]),
 }
 
 _lib = None

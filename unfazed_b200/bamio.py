@@ -225,6 +225,30 @@ def reg2bin(beg: int, end: int) -> int:
     return 0
 
 
+def parse_bins(d: bytes, p: int, n_ref: int) -> Tuple[List[Dict[int, np.ndarray]], List[np.ndarray], int]:
+    """The per-reference part BAI and TBI share, from byte p of the index: bins (bin -> chunk array [n, 2] of virtual
+    offsets, the pseudo-bin 37450 of counts dropped) and the linear index of every reference, and where it ended."""
+    bins_all: List[Dict[int, np.ndarray]] = []
+    linear: List[np.ndarray] = []
+    for _ in range(n_ref):
+        n_bin = struct.unpack_from("<i", d, p)[0]
+        p += 4
+        bins = {}
+        for _ in range(n_bin):
+            b, n_chunk = struct.unpack_from("<Ii", d, p)
+            p += 8
+            ch = np.frombuffer(d, dtype="<u8", count=2 * n_chunk, offset=p).reshape(n_chunk, 2)
+            p += 16 * n_chunk
+            if b != 37450:                    # pseudo-bin of mapped / unmapped counts
+                bins[b] = ch
+        n_intv = struct.unpack_from("<i", d, p)[0]
+        p += 4
+        linear.append(np.frombuffer(d, dtype="<u8", count=n_intv, offset=p).copy())
+        p += 8 * n_intv
+        bins_all.append(bins)
+    return bins_all, linear, p
+
+
 class BaiIndex:
     """Bins (bin -> chunk array [n, 2] of virtual offsets) and linear index of every reference."""
 
@@ -233,25 +257,7 @@ class BaiIndex:
         if d[:4] != b"BAI\x01":
             raise ValueError("%s: not a BAI index" % path)
         n_ref = struct.unpack_from("<i", d, 4)[0]
-        p = 8
-        self.bins: List[Dict[int, np.ndarray]] = []
-        self.linear: List[np.ndarray] = []
-        for _ in range(n_ref):
-            n_bin = struct.unpack_from("<i", d, p)[0]
-            p += 4
-            bins = {}
-            for _ in range(n_bin):
-                b, n_chunk = struct.unpack_from("<Ii", d, p)
-                p += 8
-                ch = np.frombuffer(d, dtype="<u8", count=2 * n_chunk, offset=p).reshape(n_chunk, 2)
-                p += 16 * n_chunk
-                if b != 37450:                    # pseudo-bin of mapped / unmapped counts
-                    bins[b] = ch
-            n_intv = struct.unpack_from("<i", d, p)[0]
-            p += 4
-            self.linear.append(np.frombuffer(d, dtype="<u8", count=n_intv, offset=p).copy())
-            p += 8 * n_intv
-            self.bins.append(bins)
+        self.bins, self.linear, _ = parse_bins(d, 8, n_ref)
 
     def chunks(self, tid: int, beg: int, end: int) -> List[Tuple[int, int]]:
         """Merged chunk list of [beg, end) on reference tid: the chunks of reg2bins' bins that end after the linear
@@ -770,7 +776,6 @@ def write_bam(table: ReadTable, kid: int, path: str, extra_tags: Optional[Dict[i
     nib_of_code = np.array([1, 2, 4, 8], dtype=np.uint8)
     iupac = np.frombuffer(bytes([_NIB_CHARS.index(ch) for ch in b"=MRSVWYHKDB"]), dtype=np.uint8)
     out_blocks: List[bytes] = []
-    pool = ThreadPoolExecutor(_THREADS)
     # records: serialised in chunks of reads; every record's start is remembered as an uncompressed stream offset
     rec_start = np.zeros(rows.shape[0] + 1, dtype=np.int64)
     stream: List[bytes] = []
@@ -838,11 +843,18 @@ def write_bam(table: ReadTable, kid: int, path: str, extra_tags: Optional[Dict[i
         rec_start[a + 1: a + m + 1] = pos_u + np.cumsum(size)
         pos_u += int(size.sum())
         stream.append(data.tobytes())
-    body = b"".join(stream)
-    head_blocks = [bytes(head[i: i + _BLOCK_IN]) for i in range(0, len(head), _BLOCK_IN)] or [b""]
+    voff = write_bgzf(path, bytes(head), b"".join(stream), level)
+    _write_bai(path + ".bai", n_ref, tid_of_row, t.hdr["start"][rows].astype(np.int64), ends[rows],
+               voff(rec_start[:-1]), voff(rec_start[1:]))
+
+
+def write_bgzf(path: str, head: bytes, body: bytes, level: int = 6):
+    """``head`` and ``body`` BGZF-compressed into ``path`` (the header in blocks of its own, as htslib writes it), plus the
+    EOF block.  Returns the map of uncompressed body offsets (an array) to virtual file offsets."""
+    head_blocks = [head[i: i + _BLOCK_IN] for i in range(0, len(head), _BLOCK_IN)] or [b""]
     body_blocks = [body[i: i + _BLOCK_IN] for i in range(0, len(body), _BLOCK_IN)]
-    comp = list(pool.map(lambda raw: _bgzf_block(raw, level), head_blocks + body_blocks))
-    pool.shutdown()
+    with ThreadPoolExecutor(_THREADS) as pool:
+        comp = list(pool.map(lambda raw: _bgzf_block(raw, level), head_blocks + body_blocks))
     coff = np.cumsum([0] + [len(c) for c in comp])
     body_coff = coff[len(head_blocks):]                     # file offset of each body block (and of the EOF block)
     with open(path, "wb") as f:
@@ -853,9 +865,7 @@ def write_bam(table: ReadTable, kid: int, path: str, extra_tags: Optional[Dict[i
     def voff(u: np.ndarray) -> np.ndarray:
         blk = u // _BLOCK_IN
         return (body_coff[blk].astype(np.uint64) << np.uint64(16)) | (u % _BLOCK_IN).astype(np.uint64)
-
-    _write_bai(path + ".bai", n_ref, tid_of_row, t.hdr["start"][rows].astype(np.int64), ends[rows],
-               voff(rec_start[:-1]), voff(rec_start[1:]))
+    return voff
 
 
 def _ranges(start: np.ndarray, length: np.ndarray) -> np.ndarray:
@@ -866,10 +876,18 @@ def _ranges(start: np.ndarray, length: np.ndarray) -> np.ndarray:
 
 def _write_bai(path: str, n_ref: int, tid: np.ndarray, pos: np.ndarray, end_raw: np.ndarray, vbeg: np.ndarray,
                vend: np.ndarray) -> None:
-    """BAI of records sorted by (tid, pos): per reference the bins (chunks of consecutive records of the same bin
-    merged), the pseudo-bin of counts and the 16 kb linear index."""
+    """BAI of records sorted by (tid, pos)."""
+    with open(path, "wb") as f:
+        f.write(b"BAI\x01" + struct.pack("<i", n_ref) + index_refs(n_ref, tid, pos, end_raw, vbeg, vend))
+
+
+def index_refs(n_ref: int, tid: np.ndarray, pos: np.ndarray, end_raw: np.ndarray, vbeg: np.ndarray,
+               vend: np.ndarray) -> bytes:
+    """The per-reference part of a BAI or TBI for records sorted by (tid, pos) spanning [pos, end_raw) at virtual offsets
+    [vbeg, vend): per reference the bins (chunks of consecutive records of the same bin merged), the pseudo-bin of counts
+    and the 16 kb linear index; then the count of records without a coordinate (0)."""
     end = np.maximum(end_raw, pos + 1)
-    out = bytearray(b"BAI\x01" + struct.pack("<i", n_ref))
+    out = bytearray()
     for t in range(n_ref):
         sel = np.flatnonzero(tid == t)
         bins: Dict[int, List[List[int]]] = {}
@@ -901,5 +919,4 @@ def _write_bai(path: str, n_ref: int, tid: np.ndarray, pos: np.ndarray, end_raw:
             vals.append(last)
         out += struct.pack("<i", n_intv) + struct.pack("<%dQ" % n_intv, *vals)
     out += struct.pack("<Q", 0)
-    with open(path, "wb") as f:
-        f.write(bytes(out))
+    return bytes(out)

@@ -3,7 +3,9 @@
 * ``*.npz`` written by ``tableio.save_tables`` (our native cache of decoded inputs), or
 * indexed BAM files (``*.bam`` with a ``.bai``) through ``bamio.py``, natively -- no pysam needed, and with an
   engine the bulk of the records is decoded on the GPU, or
-* the sites VCF/BCF through ``cyvcf2`` and the kids' other alignment files (CRAM, unindexed BAM) through ``pysam``
+* a bgzipped, tabix-indexed sites VCF (``*.vcf.gz`` / ``*.vcf.bgz`` with a ``.tbi``) through ``vcfio.py``, natively --
+  no cyvcf2 needed, and with an engine the genotype fields are decoded on the GPU, or
+* other sites VCF/BCF files through ``cyvcf2`` and the kids' other alignment files (CRAM, unindexed BAM) through ``pysam``
   -- imported lazily, so the package works without them as long as tables are supplied -- decoded only around
   the DNMs and packed by ``packers.py``.
 
@@ -17,7 +19,7 @@ from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 
-from . import bamio, packers
+from . import bamio, packers, vcfio
 from .plan import strip_chr
 from .schema import ReadTable, SiteTable
 from .tableio import load_tables
@@ -47,14 +49,27 @@ def _toggle(chrom: str) -> str:
     return strip_chr(chrom) if "chr" in chrom else "chr" + chrom
 
 
-def load_sites(vcf_name: str, dnms: List[dict], pedigrees: dict, search_dist: int) -> SiteTable:
+def is_indexed_vcf(name: str) -> bool:
+    """An existing ``*.vcf.gz`` / ``*.vcf.bgz`` file with a ``.tbi`` next to it: read natively by ``vcfio``."""
+    return name.endswith((".vcf.gz", ".vcf.bgz")) and os.path.isfile(name) and vcfio.index_path(name) is not None
+
+
+def load_sites(vcf_name: str, dnms: List[dict], pedigrees: dict, search_dist: int, engine=None) -> SiteTable:
+    """The SiteTable of the trios of the DNM list around their DNMs.  A tabix-indexed ``.vcf.gz`` is read by ``vcfio``
+    (with ``engine``, its genotype fields are decoded on that engine's GPU); BCF, CSI-indexed or unindexed files go
+    through cyvcf2."""
     if vcf_name in _registry and _registry[vcf_name][0] is not None:
         return _registry[vcf_name][0]
     if vcf_name.endswith(".npz"):
         return _npz(vcf_name)[0]
-    from cyvcf2 import VCF
-    from .utils import get_prefix
-    prefix = get_prefix(VCF(vcf_name))
+    native = is_indexed_vcf(vcf_name)
+    if native:
+        vf = vcfio.VcfFile(vcf_name)
+        prefix = vf.prefix
+    else:
+        from cyvcf2 import VCF
+        from .utils import get_prefix
+        prefix = get_prefix(VCF(vcf_name))
     trios, seen = [], set()
     for d in dnms:
         ped = pedigrees.get(d["kid"])
@@ -66,6 +81,8 @@ def load_sites(vcf_name: str, dnms: List[dict], pedigrees: dict, search_dist: in
         contig = prefix + strip_chr(d["chrom"])
         s, e = int(d["start"]), int(d["end"])
         regions.setdefault(contig, []).append((s - search_dist - 2, e + search_dist + 2))
+    if native:
+        return vcfio.read_sites(vf, trios, regions, engine=engine)
     return packers.pack_sites(VCF(vcf_name), trios, regions)
 
 

@@ -305,6 +305,103 @@ class BamDecoder:
         return self._reads
 
 
+class VcfDecoder:
+    """Device side of ``vcfio.read_sites(engine=...)``, with the calls of ``vcfio.HostDecoder``: the inflated text goes
+    up once (pinned staging), the newline pass (unfz_vcf_line_count, a scan, unfz_vcf_line_write) and the fixed-field
+    parse (unfz_vcf_parse) run on the engine's stream and the 64-byte records come back for the host's selection; then
+    unfz_vcf_samples decodes the member columns of the selected lines, which come back as the table's genotype arrays.
+    The floats it leaves to the host are decoded by ``vcfio.finish_cells``."""
+
+    def __init__(self, engine: "Engine"):
+        self.engine = engine
+        self.h2d_bytes = self.d2h_bytes = 0
+        self.timings_ms: Dict[str, float] = {}
+
+    def _time(self, name, e0, e1):
+        self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
+
+    def lines(self, buf: np.ndarray) -> np.ndarray:
+        eng = self.engine
+        lib, ctx, dev = eng.lib, eng.ctx, eng.device
+        n = int(buf.shape[0])
+        chunks = int(lib.unfz_vcf_chunks(n))
+        with eng.on_stream():
+            st = torch.cuda.current_stream(dev)
+            sp = C.c_void_p(st.cuda_stream)
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
+            e[0].record(st)
+            # 16 bytes of padding: the sample pass reads whole 16-byte words
+            self.dbuf = _to_device(np.ascontiguousarray(buf), dev, True, 16) if n else torch.zeros(16, dtype=torch.uint8,
+                                                                                                 device=dev)
+            e[1].record(st)
+            cnt = torch.empty((max(chunks, 1),), dtype=torch.int32, device=dev)
+            at = torch.empty((chunks + 1,), dtype=torch.int32, device=dev)
+            total = torch.zeros((1,), dtype=torch.int64, device=dev)
+            work = torch.empty((int(lib.unfz_scan_work_bytes(chunks)),), dtype=torch.uint8, device=dev)
+            eng._check(lib.unfz_vcf_line_count(ctx, self.dbuf.data_ptr(), n, cnt.data_ptr(), sp), "vcf_line_count")
+            eng._check(lib.unfz_exclusive_scan_u32(ctx, cnt.data_ptr(), at.data_ptr(), chunks, total.data_ptr(),
+                                                   work.data_ptr(), sp), "exclusive_scan_u32")
+            n_lines = int(total.item())
+            self.ends = torch.empty((max(n_lines, 1),), dtype=torch.int64, device=dev)
+            eng._check(lib.unfz_vcf_line_write(ctx, self.dbuf.data_ptr(), n, at.data_ptr(), self.ends.data_ptr(), sp),
+                       "vcf_line_write")
+            e[2].record(st)
+            rsz = L.VCF_REC_DTYPE.itemsize
+            self.drecs = torch.empty((max(n_lines, 1) * rsz,), dtype=torch.uint8, device=dev)
+            eng._check(lib.unfz_vcf_parse(ctx, self.dbuf.data_ptr(), self.ends.data_ptr(), n_lines, self.drecs.data_ptr(),
+                                          sp), "vcf_parse")
+            e[3].record(st)
+            recs = self.drecs[: n_lines * rsz].cpu().numpy().view(L.VCF_REC_DTYPE)
+            e[4].record(st)
+        e[4].synchronize()
+        self._time("h2d_text", e[0], e[1])
+        self._time("line_bounds", e[1], e[2])
+        self._time("parse", e[2], e[3])
+        self._time("d2h_records", e[3], e[4])
+        self.h2d_bytes += n
+        self.d2h_bytes += int(recs.nbytes) + 8
+        return recs
+
+    def samples(self, sel: np.ndarray, slot_of: np.ndarray, n_members: int, gq_float: bool,
+                max_digits: int = 15) -> Dict[str, np.ndarray]:
+        eng = self.engine
+        lib, ctx, dev = eng.lib, eng.ctx, eng.device
+        ns = int(sel.shape[0])
+        m = int(n_members)
+        cells = ns * m
+        with eng.on_stream():
+            st = torch.cuda.current_stream(dev)
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+            e[0].record(st)
+            dsel = _to_device(np.ascontiguousarray(sel, dtype=np.int64), dev, True) if ns else \
+                torch.zeros(1, dtype=torch.int64, device=dev)
+            dslot = _to_device(np.ascontiguousarray(slot_of, dtype=np.int32), dev, True) if slot_of.shape[0] else \
+                torch.full((1,), -1, dtype=torch.int32, device=dev)
+            e[1].record(st)
+            out = {"gt": torch.empty((max(cells, 1),), dtype=torch.uint8, device=dev),
+                   "gq": torch.empty((max(cells, 1),), dtype=torch.float32, device=dev),
+                   "rd": torch.empty((max(cells, 1),), dtype=torch.int32, device=dev),
+                   "ad": torch.empty((max(cells, 1),), dtype=torch.int32, device=dev),
+                   "status": torch.empty((max(cells, 1),), dtype=torch.uint8, device=dev),
+                   "line_bad": torch.empty((max(ns, 1),), dtype=torch.uint8, device=dev)}
+            eng._check(lib.unfz_vcf_samples(ctx, self.dbuf.data_ptr(), self.drecs.data_ptr(), dsel.data_ptr(), ns,
+                                            dslot.data_ptr(), int(slot_of.shape[0]), m, int(bool(gq_float)), int(max_digits),
+                                            *(out[k].data_ptr() for k in ("gt", "gq", "rd", "ad", "status", "line_bad")),
+                                            C.c_void_p(st.cuda_stream)), "vcf_samples")
+            e[2].record(st)
+            host = {k: v.cpu().numpy() for k, v in out.items()}
+            e[3].record(st)
+        e[3].synchronize()
+        self._time("h2d_select", e[0], e[1])
+        self._time("samples", e[1], e[2])
+        self._time("d2h_cells", e[2], e[3])
+        self.h2d_bytes += int(sel.nbytes + slot_of.nbytes)
+        self.d2h_bytes += cells * 14 + ns
+        res = {k: host[k][:cells].reshape(ns, m) for k in ("gt", "gq", "rd", "ad", "status")}
+        res["line_bad"] = host["line_bad"][:ns]
+        return res
+
+
 def _to_device(a: np.ndarray, device, pin: bool, pad: int = 0) -> torch.Tensor:
     """Host array -> device tensor (+ ``pad`` zero elements).  Arrays that already live in pinned
     memory are copied asynchronously; ``pin`` stages pageable arrays through a pinned copy."""
@@ -523,6 +620,10 @@ class Engine:
     def bam_decoder(self) -> BamDecoder:
         """A device decoder for one ``bamio.read_regions`` load."""
         return BamDecoder(self)
+
+    def vcf_decoder(self) -> VcfDecoder:
+        """A device decoder for one ``vcfio.read_sites`` load."""
+        return VcfDecoder(self)
 
     def decode_bam(self, paths, regions, head_reads: int = 0, min_gt_qual=20) -> DeviceReads:
         """Indexed BAM files -> DeviceReads, the bulk of the records decoded on this GPU (``bamio.read_regions``).

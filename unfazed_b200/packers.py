@@ -71,11 +71,8 @@ def pack_sites(vcf, trios: Sequence[Tuple[str, str, str]], regions: Optional[Dic
         rds.append(v.gt_ref_depths)
         ads.append(v.gt_alt_depths)
     n = len(pos)
-    contigs: List[str] = []
     cindex: Dict[str, int] = {}
     cid = np.fromiter((cindex.setdefault(c, len(cindex)) for c in chrom), dtype=np.int64, count=n)
-    contigs = list(cindex)
-    pos_a = np.array(pos, dtype=np.int64)
     simple = np.fromiter((len(al) == 1 and len(r) == 1 and len(al[0]) == 1 and al[0] != "*" for r, al in zip(refs, alts_l)),
                          dtype=bool, count=n)
     ref_b = np.fromiter((ord(r[0]) if r else 0 for r in refs), dtype=np.uint8, count=n)
@@ -83,6 +80,19 @@ def pack_sites(vcf, trios: Sequence[Tuple[str, str, str]], regions: Optional[Dic
     ns = len(samples)
     stack = lambda lst, dt: (np.stack([np.asarray(x) for x in lst]).astype(dt, copy=False) if n else np.zeros((0, ns), dtype=dt))
     GT, GQ, RD, AD = stack(gts, np.uint8), stack(gqs, np.float32), stack(rds, np.int32), stack(ads, np.int32)
+    refalt = {r: (refs[r], alts_l[r]) for r in np.flatnonzero(~simple).tolist()}
+    return build_site_table(trios, cols, list(cindex), cid, np.array(pos, dtype=np.int64), simple, ref_b, alt_b,
+                            GT, GQ, RD, AD, refalt)
+
+
+def build_site_table(trios, cols, contigs: List[str], cid: np.ndarray, pos_a: np.ndarray, simple: np.ndarray,
+                     ref_b: np.ndarray, alt_b: np.ndarray, GT: np.ndarray, GQ: np.ndarray, RD: np.ndarray, AD: np.ndarray,
+                     refalt: Dict[int, Tuple[str, List[str]]]) -> SiteTable:
+    """The trio-major SiteTable of n records in decoder order (``rec_id`` = that order): ``cid`` contig index into
+    ``contigs``, ``pos_a`` 0-based start, ``simple`` / ``ref_b`` / ``alt_b`` per record; ``GT`` / ``GQ`` / ``RD`` / ``AD``
+    [n, columns] per-sample arrays, ``cols`` [(trio index, [column of kid, dad, mom])] the trios that get blocks;
+    ``refalt``: record -> (REF, ALT list) of every record that is not simple."""
+    n = int(pos_a.shape[0])
     # block order: (trio, contig id); rows of a block sorted by position, file order among equal positions
     order_in_contig = np.lexsort((np.arange(n), pos_a, cid)) if n else np.zeros(0, dtype=np.int64)
     c_sorted = cid[order_in_contig]
@@ -108,7 +118,7 @@ def pack_sites(vcf, trios: Sequence[Tuple[str, str, str]], regions: Optional[Dic
             parts["rid"].append(rows)
             for local in np.flatnonzero(~simple[rows]).tolist():
                 r = int(rows[local])
-                extras[offs[-1] + local] = (refs[r], alts_l[r])
+                extras[offs[-1] + local] = refalt[r]
             offs.append(offs[-1] + rows.shape[0])
     cat = lambda name, dt: (np.concatenate(parts[name]).astype(dt) if parts[name] else np.zeros(0, dtype=dt))
     V = offs[-1]

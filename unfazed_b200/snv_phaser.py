@@ -78,7 +78,8 @@ def run_batch(snvs, svs, pedigrees, sites, threads, build, no_extended, multirea
               split_error_margin, compact=False):
     from .phaser import BatchPhaser
     dnms = list(svs) + list(snvs)
-    site_table = datasource.load_sites(sites, dnms, pedigrees, search_dist)
+    # an indexed sites VCF has its genotype fields decoded on the engine's GPU
+    site_table = datasource.load_sites(sites, dnms, pedigrees, search_dist, engine=get_engine())
     # indexed BAM inputs are decoded on the engine's GPU; the table then comes with its device columns
     read_table = datasource.load_reads(dnms, search_dist, readlen, insert_size_max_sample, engine=get_engine(),
                                        min_gt_qual=min_gt_qual)

@@ -43,6 +43,11 @@ def read_vars_bedzip(bedzipname):
 
 
 def read_vars_vcf(vcfname):
+    if not vcfname.endswith(".bcf") and os.path.isfile(vcfname):
+        # an existing .vcf / .vcf.gz: read natively (vcfio), no cyvcf2 needed
+        from .vcfio import read_dnms
+        yield from read_dnms(vcfname)
+        return
     from cyvcf2 import VCF
     vcf = VCF(vcfname)
     for v in vcf:

@@ -1,0 +1,494 @@
+"""Tabix-indexed sites VCFs without cyvcf2: BGZF inflate and TBI region queries on the host, field decoding in native
+code (csrc/vcf.cu), on the GPU with an engine.
+
+* ``VcfFile`` -- one bgzipped VCF and its ``.tbi``: the header (sample names, the declared Type of the GQ / AD / RO /
+  AO FORMAT fields, the first record's CHROM for ``get_prefix``) and region queries (``TbiIndex``: the BAI bins, chunks
+  and linear index behind a tabix header, read by ``bamio``'s code; overlap by tabix's end, INFO END or POS + len(REF)).
+* ``read_sites`` -- the ``SiteTable`` ``packers.pack_sites`` builds from a cyvcf2 handle over the same regions, array
+  for array.  The text of the union of every interval's chunks is inflated once; line boundaries, fixed fields and the
+  genotype fields of the trio members are decoded natively -- on the host, or with ``engine=`` on the GPU
+  (``engine.VcfDecoder``), where only the text goes up and only the fixed fields and member columns come back.
+* ``read_dnms`` -- the DNM dicts ``unfazed.read_vars_vcf`` yields, from a plain or gzipped VCF read whole.
+* ``write_vcf`` -- a sorted ``.vcf.gz`` + ``.tbi`` from a ``SiteTable`` (tests and tools generate their inputs with it).
+
+Field decoding follows cyvcf2 0.31.0's defaults (gts012=False, strict_gt=False); DESIGN §5 lists the assumptions.  BCF,
+CSI indexes and unindexed files are not read here: ``datasource.load_sites`` sends them to cyvcf2.
+"""
+from __future__ import annotations
+
+import gzip
+import os
+import re
+import struct
+from typing import Dict, List, Optional, Sequence, Tuple
+
+import numpy as np
+
+from . import _lib as L
+from .bamio import BaiIndex, BgzfReader, index_refs, parse_bins, write_bgzf
+from .packers import _merge, build_site_table
+from .schema import GT_UNKNOWN, HET, HOM_ALT, HOM_REF, SiteTable
+
+FAST_DIGITS = 15                 # significant digits of a float GQ decoded in native code (the exact fast path)
+
+
+def _ptr(a: np.ndarray) -> int:
+    return a.ctypes.data
+
+
+# ------------------------------------------------------------------------------------------------
+# native decode on the host (the device decoder, engine.VcfDecoder, has the same two calls)
+# ------------------------------------------------------------------------------------------------
+
+class HostDecoder:
+    """``lines`` and ``samples`` with the host entry points of csrc/vcf.cu."""
+
+    def lines(self, buf: np.ndarray) -> np.ndarray:
+        """Fixed fields (``_lib.VCF_REC_DTYPE``) of every '\\n'-terminated line of ``buf``."""
+        self.buf = buf
+        lib = L.load()
+        cap = int(np.count_nonzero(buf == 10))
+        ends = np.empty(max(cap, 1), dtype=np.int64)
+        n = lib.unfz_vcf_line_ends_host(_ptr(buf), int(buf.shape[0]), cap, _ptr(ends))
+        self.recs = np.empty(n, dtype=L.VCF_REC_DTYPE)
+        if n:
+            lib.unfz_vcf_parse_host(_ptr(buf), _ptr(ends), n, _ptr(self.recs))
+        return self.recs
+
+    def samples(self, sel: np.ndarray, slot_of: np.ndarray, n_members: int, gq_float: bool,
+                max_digits: int = FAST_DIGITS) -> Dict[str, np.ndarray]:
+        """Genotype fields of the selected lines for the member columns (``slot_of``: sample -> column or -1)."""
+        sel = np.ascontiguousarray(sel, dtype=np.int64)
+        slot_of = np.ascontiguousarray(slot_of, dtype=np.int32)
+        out = _empty_cells(sel.shape[0], n_members)
+        L.load().unfz_vcf_samples_host(_ptr(self.buf), _ptr(self.recs), _ptr(sel), int(sel.shape[0]), _ptr(slot_of),
+                                       int(slot_of.shape[0]), int(n_members), int(bool(gq_float)), int(max_digits),
+                                       *(_ptr(out[k]) for k in ("gt", "gq", "rd", "ad", "status", "line_bad")))
+        return out
+
+
+def _empty_cells(n: int, m: int) -> Dict[str, np.ndarray]:
+    return {"gt": np.empty((n, m), np.uint8), "gq": np.empty((n, m), np.float32), "rd": np.empty((n, m), np.int32),
+            "ad": np.empty((n, m), np.int32), "status": np.empty((n, m), np.uint8), "line_bad": np.empty(n, np.uint8)}
+
+
+def _field_end(text: np.ndarray, a: int) -> int:
+    e = a
+    while e < text.shape[0] and text[e] not in (9, 10, 13, 58):      # tab, newline, CR, ':'
+        e += 1
+    return e
+
+
+def finish_cells(cells: Dict[str, np.ndarray], buf: np.ndarray, recs: np.ndarray, sel: np.ndarray, where) -> None:
+    """Raises ``ValueError`` for malformed fields; decodes on the host the float GQs the native code left to it (their
+    cell holds the int32 offset of the text from the line start) with Python's correctly rounded ``float``, then cast
+    to float32 -- what htslib's strtod-to-float gives."""
+    bad = np.flatnonzero(cells["line_bad"])
+    if bad.shape[0]:
+        raise ValueError("%s: more sample columns than header samples" % where(int(recs["line_off"][sel[bad[0]]])))
+    st = cells["status"]
+    badc = np.argwhere(st & L.VCF_CELL_BAD)
+    if badc.shape[0]:
+        raise ValueError("%s: malformed or overflowing genotype field" % where(int(recs["line_off"][sel[badc[0, 0]]])))
+    host = np.argwhere(st & L.VCF_CELL_HOST)
+    if host.shape[0]:
+        gq = cells["gq"]
+        offs = gq.view(np.int32)
+        for i, m in host.tolist():
+            a = int(recs["line_off"][sel[i]]) + int(offs[i, m])
+            txt = buf[a:_field_end(buf, a)].tobytes().decode("ascii", "replace")
+            try:
+                gq[i, m] = np.float32(float(txt))
+            except ValueError:
+                raise ValueError("%s: GQ %r is not a number" % (where(a), txt))
+
+
+# ------------------------------------------------------------------------------------------------
+# TBI
+# ------------------------------------------------------------------------------------------------
+
+class TbiIndex(BaiIndex):
+    """A tabix index: the reference names of its header, then bins, chunks and linear index laid out as BAI's (the
+    region queries are ``BaiIndex.chunks``)."""
+
+    def __init__(self, path: str):
+        raw, _ = BgzfReader(path).stream_from(0, 1 << 62)
+        d = raw.tobytes()
+        if d[:4] != b"TBI\x01":
+            raise ValueError("%s: not a TBI index" % path)
+        n_ref, _fmt, _cs, _cb, _ce, _meta, _skip, l_nm = struct.unpack_from("<8i", d, 4)
+        self.names = [x.decode() for x in d[36:36 + l_nm].split(b"\0")[:n_ref]]
+        self.bins, self.linear, _ = parse_bins(d, 36 + l_nm, n_ref)
+
+
+def index_path(path: str) -> Optional[str]:
+    """``<file>.tbi`` if it exists."""
+    p = path + ".tbi"
+    return p if os.path.exists(p) else None
+
+
+# ------------------------------------------------------------------------------------------------
+# VCF file
+# ------------------------------------------------------------------------------------------------
+
+_FORMAT_RE = re.compile(rb"^##FORMAT=<ID=([^,>]+),.*?Type=([A-Za-z]+)")
+
+
+def _prefix_of(chrom: Optional[str]) -> str:
+    """``utils.get_prefix`` on a first record of this CHROM (None: no record)."""
+    if chrom is None or "chr" not in chrom.lower():
+        return ""
+    return chrom[:3]
+
+
+def _parse_header(text: bytes, path: str):
+    """(samples, FORMAT types, first CHROM or None, offset of the first data line) of a VCF whose text starts with
+    ``text``; None when ``text`` ends before the #CHROM line and the line after it are complete."""
+    i = 0 if text.startswith(b"#CHROM") else text.find(b"\n#CHROM") + 1
+    if i <= 0 and not text.startswith(b"#CHROM"):
+        return None
+    j = text.find(b"\n", i)
+    if j < 0:
+        return None
+    k = text.find(b"\n", j + 1)
+    cols = text[i:j].rstrip(b"\r").decode().split("\t")
+    if len(cols) < 8:
+        raise ValueError("%s: malformed #CHROM header line" % path)
+    types = {}
+    for line in text[:i].split(b"\n"):
+        m = _FORMAT_RE.match(line)
+        if m:
+            types[m.group(1).decode()] = m.group(2).decode()
+    first = text[j + 1:k if k >= 0 else len(text)]
+    chrom = first.split(b"\t", 1)[0].decode() if first.strip() else None
+    return cols[9:], types, chrom, j + 1, k >= 0
+
+
+class VcfFile:
+    """One bgzipped, tabix-indexed VCF: header and region queries."""
+
+    def __init__(self, path: str, index: Optional[str] = None):
+        self.path = path
+        self.bgzf = BgzfReader(path)
+        ip = index or index_path(path)
+        if ip is None:
+            raise ValueError("%s: no .tbi index" % path)
+        self.tbi = TbiIndex(ip)
+        self.tids = {n: i for i, n in enumerate(self.tbi.names)}
+        want = 1 << 16
+        while True:
+            head, eof = self.bgzf.stream_from(0, want)
+            hb = head.tobytes()
+            got = _parse_header(hb, path)
+            if got is not None and (got[4] or eof):
+                break
+            if eof:
+                raise ValueError("%s: no #CHROM header line" % path)
+            want = 4 * len(hb)
+        self.samples, self.format_types, chrom, _, _ = got
+        self.prefix = _prefix_of(chrom)
+
+    def gq_float(self) -> bool:
+        """GQ is decoded as a float unless the header declares it Integer."""
+        return self.format_types.get("GQ", "Float") != "Integer"
+
+    def fetch_union(self, queries: Sequence[Tuple[int, int, int]]):
+        """Inflated text of the union of the chunk lists of many (tid, beg, end) queries, and a function that names a
+        byte of it (the file and the virtual offset of its chunk plus the bytes after it) for error messages."""
+        ch = sorted(c for tid, beg, end in queries for c in self.tbi.chunks(tid, beg, end))
+        merged: List[List[int]] = []
+        for b, e in ch:
+            if merged and b <= merged[-1][1]:
+                merged[-1][1] = max(merged[-1][1], e)
+            else:
+                merged.append([b, e])
+        parts = self.bgzf.read_ranges([(b, e) for b, e in merged])
+        for (vb, _), p in zip(merged, parts):
+            if p.shape[0] and p[-1] != 10:
+                raise ValueError("%s: the TBI chunk at virtual offset %d does not end on a line boundary" % (self.path, vb))
+        starts = np.cumsum([0] + [p.shape[0] for p in parts])
+        buf = np.concatenate(parts) if parts else np.zeros(0, dtype=np.uint8)
+
+        def where(off: int):
+            k = int(np.searchsorted(starts, off, side="right")) - 1
+            return "%s, line at virtual offset %d + %d bytes" % (self.path, merged[k][0], off - int(starts[k]))
+        return buf, where
+
+    def query(self, contig: str, beg: int, end: int) -> np.ndarray:
+        """Fixed fields of the records overlapping [beg, end) of contig, in file order (host decode)."""
+        tid = self.tids.get(contig)
+        if tid is None:
+            return np.zeros(0, dtype=L.VCF_REC_DTYPE)
+        buf, where = self.fetch_union([(tid, beg, end)])
+        recs = _lines(HostDecoder(), buf, where)
+        keep = (_chrom_ids(buf, recs, self.tids, where) == tid) & (recs["pos0"] < end) & (recs["rend"] > beg)
+        return recs[keep]
+
+
+def _lines(dec, buf: np.ndarray, where) -> np.ndarray:
+    recs = dec.lines(buf)
+    bad = np.flatnonzero(recs["flags"] & L.VCF_BAD)
+    if bad.shape[0]:
+        off = int(recs["line_off"][bad[0]])
+        line = buf[off: off + 60].tobytes().split(b"\n")[0]
+        raise ValueError("%s: malformed VCF record %r (fewer than 8 columns, or POS / END not a valid position)"
+                         % (where(off), line))
+    return recs
+
+
+def _chrom_ids(buf: np.ndarray, recs: np.ndarray, tids: Dict[str, int], where) -> np.ndarray:
+    """Reference id of every line's CHROM (-1: not in the index), from the CHROM hashes; every line of a hash is
+    checked byte for byte against the first."""
+    out = np.full(recs.shape[0], -1, dtype=np.int64)
+    if not recs.shape[0]:
+        return out
+    uh, inv = np.unique(recs["chrom_hash"], return_inverse=True)
+    for g in range(uh.shape[0]):
+        ix = np.flatnonzero(inv == g)
+        ln = recs["chrom_len"][ix]
+        off = recs["line_off"][ix]
+        l0 = int(ln[0])
+        name = buf[int(off[0]): int(off[0]) + l0].tobytes()
+        same = ln == l0
+        if l0 and same.all():
+            same = (buf[off[:, None] + np.arange(l0)] == np.frombuffer(name, np.uint8)).all(axis=1)
+        if not same.all():                       # a hash shared by two names: resolve this group one line at a time
+            for i in ix.tolist():
+                o, n = int(recs["line_off"][i]), int(recs["chrom_len"][i])
+                out[i] = tids.get(buf[o:o + n].tobytes().decode("ascii", "replace"), -1)
+            continue
+        out[ix] = tids.get(name.decode("ascii", "replace"), -1)
+    return out
+
+
+# ------------------------------------------------------------------------------------------------
+# site reader
+# ------------------------------------------------------------------------------------------------
+
+def read_sites(path, trios: Sequence[Tuple[str, str, str]], regions: Dict[str, List[Tuple[int, int]]], engine=None,
+               max_digits: int = FAST_DIGITS) -> SiteTable:
+    """``packers.pack_sites(VCF(path), trios, regions)`` from the file directly.  ``path``: a file name or a
+    ``VcfFile``.  With ``engine`` the text is decoded on that engine's GPU (``Engine.vcf_decoder``).  ``max_digits``:
+    significant digits a float GQ may have to be decoded natively (0 sends every float GQ to the host decode)."""
+    vf = path if isinstance(path, VcfFile) else VcfFile(path)
+    sidx = {s: i for i, s in enumerate(vf.samples)}
+    cols_s = [(t, [sidx[m] for m in trio]) for t, trio in enumerate(trios) if all(m in sidx for m in trio)]
+    slot_of = np.full(len(vf.samples), -1, dtype=np.int32)
+    n_members = 0
+    for _t, ix in cols_s:
+        for s in ix:
+            if slot_of[s] < 0:
+                slot_of[s] = n_members
+                n_members += 1
+    cols = [(t, [int(slot_of[s]) for s in ix]) for t, ix in cols_s]
+    # every merged interval, queried as pack_sites queries it: [max(a, 0), max(b, 1)) by overlap
+    plan = []
+    for contig, ivs in regions.items():
+        plan.append((contig, vf.tids.get(contig), [(max(a, 0), max(b, 1)) for a, b in _merge(ivs)]))
+    queries = [(tid, beg, end) for _c, tid, iv in plan if tid is not None for beg, end in iv]
+    buf, where = vf.fetch_union(queries)
+    dec = engine.vcf_decoder() if engine is not None else HostDecoder()
+    recs = _lines(dec, buf, where)
+    tid_of = _chrom_ids(buf, recs, vf.tids, where)
+    pos0 = recs["pos0"].astype(np.int64)
+    rend = recs["rend"].astype(np.int64)
+    parts, cid_parts, contigs = [], [], []
+    for contig, tid, iv in plan:
+        if tid is None:
+            continue
+        ix_t = np.flatnonzero(tid_of == tid)                   # file order = sorted by position
+        if not ix_t.shape[0]:
+            continue
+        pos_t = pos0[ix_t]
+        span = int((rend[ix_t] - pos_t).max())
+        prev_end = None
+        got = []
+        for beg, end in iv:
+            lo = int(np.searchsorted(pos_t, beg - span, side="left"))
+            hi = int(np.searchsorted(pos_t, end, side="left"))
+            ix = ix_t[lo:hi]
+            keep = rend[ix] > beg
+            if prev_end is not None:
+                # a record that starts before the end of the previous (disjoint) interval came back there already
+                keep &= pos0[ix] >= prev_end
+            got.append(ix[keep])
+            prev_end = end
+        sel_c = np.concatenate(got)
+        if sel_c.shape[0]:
+            parts.append(sel_c)
+            cid_parts.append(np.full(sel_c.shape[0], len(contigs), dtype=np.int64))
+            contigs.append(contig)
+    sel = np.concatenate(parts) if parts else np.zeros(0, dtype=np.int64)
+    cid = np.concatenate(cid_parts) if cid_parts else np.zeros(0, dtype=np.int64)
+    r = recs[sel]
+    simple = (r["flags"] & L.VCF_SIMPLE) != 0
+    alt_b = np.zeros(sel.shape[0], dtype=np.uint8)
+    has_alt = (r["n_alt"] > 0) & (r["alt_len"] > 0)
+    alt_b[has_alt] = buf[(r["line_off"] + r["alt_off"])[has_alt]]
+    refalt = {}
+    for i in np.flatnonzero(~simple).tolist():
+        o = int(r["line_off"][i])
+        ref = buf[o + int(r["ref_off"][i]): o + int(r["ref_off"][i]) + int(r["ref_len"][i])].tobytes().decode()
+        alt = buf[o + int(r["alt_off"][i]): o + int(r["alt_off"][i]) + int(r["alt_len"][i])].tobytes().decode()
+        refalt[i] = (ref, [] if alt == "." else alt.split(","))
+    cells = dec.samples(sel, slot_of, n_members, vf.gq_float(), max_digits)
+    finish_cells(cells, buf, recs, sel, where)
+    return build_site_table(trios, cols, contigs, cid, pos0[sel], simple, r["ref0"].astype(np.uint8), alt_b,
+                            cells["gt"], cells["gq"], cells["rd"], cells["ad"], refalt)
+
+
+# ------------------------------------------------------------------------------------------------
+# DNM reader
+# ------------------------------------------------------------------------------------------------
+
+def read_dnms(path: str):
+    """The DNMs of a plain or gzip / bgzip-compressed VCF, read whole without an index: for every record and every
+    sample whose genotype is HET or HOM_ALT, in header order, {chrom, start, end, kid, vartype, bam: ""} with start the
+    0-based POS, end tabix's end (INFO END, else start + len(REF)) and vartype INFO SVTYPE or "POINT" -- what
+    ``unfazed.read_vars_vcf`` yields from cyvcf2."""
+    from .utils import SNV_TYPES
+    opener = gzip.open if path.endswith((".gz", ".bgz")) else open
+    with opener(path, "rb") as f:
+        data = f.read()
+    if data and not data.endswith(b"\n"):
+        data += b"\n"
+    got = _parse_header(data, path)
+    if got is None:
+        raise ValueError("%s: no #CHROM header line" % path)
+    samples, types, _chrom, body, _ = got
+    buf = np.frombuffer(data, dtype=np.uint8)[body:]
+    where = lambda off: "%s, line at byte %d" % (path, body + off)
+    dec = HostDecoder()
+    recs = _lines(dec, buf, where)
+    sel = np.arange(recs.shape[0], dtype=np.int64)
+    cells = dec.samples(sel, np.arange(len(samples), dtype=np.int32), len(samples),
+                        types.get("GQ", "Float") != "Integer")
+    finish_cells(cells, buf, recs, sel, where)
+    gt = cells["gt"]
+    for i in range(recs.shape[0]):
+        o = int(recs["line_off"][i])
+        cols = buf[o: o + int(recs["line_len"][i])].tobytes().decode().split("\t", 8)
+        info = {}
+        for kv in cols[7].split(";"):
+            k, _, v = kv.partition("=")
+            info.setdefault(k, v)
+        vartype = info.get("SVTYPE") or SNV_TYPES[0]
+        for s in np.flatnonzero((gt[i] == HET) | (gt[i] == HOM_ALT)).tolist():
+            yield {"chrom": cols[0], "start": int(recs["pos0"][i]), "end": int(recs["rend"][i]), "kid": samples[s],
+                   "vartype": vartype, "bam": ""}
+
+
+# ------------------------------------------------------------------------------------------------
+# writer
+# ------------------------------------------------------------------------------------------------
+
+_GT_TEXT = {HOM_REF: "0/0", HET: "0/1", HOM_ALT: "1/1", GT_UNKNOWN: "./."}
+
+
+def _float_text(x: np.float32) -> str:
+    return np.format_float_positional(x, unique=True, trim="-")
+
+
+def write_vcf(table: SiteTable, path: str, end: Optional[Dict[int, int]] = None,
+              format_order: Optional[Sequence[Sequence[str]]] = None, level: int = 6) -> None:
+    """Sorted ``path`` (.vcf.gz) + ``path.tbi`` of ``table``: one line per record (rows grouped by ``rec_id`` and contig,
+    as ``oracle.fakes`` groups them into records), every sample of every trio, ``./.`` for a trio without a row in the
+    record.  FORMAT GT:AD:GQ; GQ is declared Float when a value is not integral (written in the shortest text that
+    parses back to the same float32) and Integer otherwise; AD is ``rd,ad`` (``.`` for -1).  ``end``: record index ->
+    INFO END (1-based inclusive); ``format_order``: record index -> the order of GT / AD / GQ on that line."""
+    t = table
+    view_rows, g_lo, g_contig = _records(t)
+    n_rec = g_lo.shape[0] - 1
+    samples: List[str] = []
+    for trio in t.trios:
+        for s in trio:
+            if s not in samples:
+                samples.append(s)
+    sidx = {s: i for i, s in enumerate(samples)}
+    blk = np.repeat(np.arange(t.n_blocks), np.diff(t.blk_off))
+    gq = t.gq
+    is_float = bool(np.any((gq != np.round(gq)) & (gq != -1)))
+    text_gq = np.empty(gq.shape, dtype=object)
+    for m in range(3):
+        if is_float:
+            text_gq[m] = [_float_text(x) for x in gq[m]]
+        else:
+            text_gq[m] = [str(int(x)) for x in gq[m]]
+        text_gq[m][gq[m] == -1] = "."
+    if is_float:
+        back = np.array([np.float32(float(x)) if x != "." else np.float32(-1) for x in text_gq.reshape(-1)],
+                        dtype=np.float32).reshape(gq.shape)
+        assert np.array_equal(back, gq), "GQ text does not parse back to the same float32"
+    head = ["##fileformat=VCFv4.2"]
+    for c in t.contigs:
+        head.append("##contig=<ID=%s>" % c)
+    head += ['##INFO=<ID=END,Number=1,Type=Integer,Description="End position">',
+             '##FORMAT=<ID=GT,Number=1,Type=String,Description="Genotype">',
+             '##FORMAT=<ID=AD,Number=R,Type=Integer,Description="Allelic depths">',
+             '##FORMAT=<ID=GQ,Number=1,Type=%s,Description="Genotype quality">' % ("Float" if is_float else "Integer"),
+             "\t".join(["#CHROM", "POS", "ID", "REF", "ALT", "QUAL", "FILTER", "INFO", "FORMAT"] + samples)]
+    head_b = ("\n".join(head) + "\n").encode()
+    dep = lambda v: "." if v == -1 else str(int(v))
+    lines: List[bytes] = []
+    pos0 = np.zeros(n_rec, dtype=np.int64)
+    rend = np.zeros(n_rec, dtype=np.int64)
+    fill: Dict[Tuple[str, ...], str] = {}
+    for g in range(n_rec):
+        rows = view_rows[g_lo[g]: g_lo[g + 1]]
+        lead = int(rows[0])
+        ref, alts = t.ref_alts(lead)
+        p0 = int(t.pos[lead])
+        order = tuple(format_order[g]) if format_order is not None else ("GT", "AD", "GQ")
+        miss = "./." if order[0] == "GT" else ":".join("./." if k == "GT" else "." for k in order)
+        cells = {}
+        for row in rows.tolist():
+            b = 3 * int(t.blk_trio[blk[row]])
+            for m in range(3):
+                v = {"GT": _GT_TEXT[int(t.gt[m, row])], "AD": "%s,%s" % (dep(t.rd[m, row]), dep(t.ad[m, row]))
+                     if not (t.rd[m, row] == -1 and t.ad[m, row] == -1) else ".", "GQ": text_gq[m, row]}
+                cells[sidx[t.trios[int(t.blk_trio[blk[row]])][m]]] = ":".join(v[k] for k in order)
+        out, at = [], 0
+        for s in sorted(cells):
+            if s > at:
+                out.append(_fill(fill, miss, s - at))
+            out.append(cells[s])
+            at = s + 1
+        if at < len(samples):
+            out.append(_fill(fill, miss, len(samples) - at))
+        e = (end or {}).get(g)
+        info = "END=%d" % e if e is not None else "."
+        lines.append(("%s\t%d\t.\t%s\t%s\t.\tPASS\t%s\t%s\t%s\n" % (
+            t.contigs[int(g_contig[g])], p0 + 1, ref, ",".join(alts) if alts else ".", info, ":".join(order),
+            "\t".join(out))).encode())
+        pos0[g] = p0
+        rend[g] = e if (e is not None and e > p0) else p0 + len(ref)
+    body = b"".join(lines)
+    starts = np.cumsum([0] + [len(x) for x in lines]).astype(np.int64)
+    voff = write_bgzf(path, head_b, body, level)
+    names = b"".join(c.encode() + b"\0" for c in t.contigs)
+    tbi = (b"TBI\x01" + struct.pack("<8i", len(t.contigs), 2, 1, 2, 0, ord("#"), 0, len(names)) + names
+           + index_refs(len(t.contigs), g_contig.astype(np.int64), pos0, rend, voff(starts[:-1]), voff(starts[1:])))
+    write_bgzf(path + ".tbi", tbi, b"", level)
+
+
+def _fill(cache: Dict, miss: str, k: int) -> str:
+    key = (miss, k)
+    s = cache.get(key)
+    if s is None:
+        s = cache[key] = "\t".join([miss] * k)
+    return s
+
+
+def _records(t: SiteTable):
+    """Rows grouped into records as ``oracle.fakes._VcfView`` groups them: (rows in record order, group bounds,
+    contig of each group)."""
+    V = t.n_rows
+    blk = np.repeat(np.arange(t.n_blocks), np.diff(t.blk_off))
+    contig = t.blk_contig[blk].astype(np.int64)
+    rid = t.record_ids().astype(np.int64)
+    order = np.lexsort((blk, rid, t.pos.astype(np.int64), contig))
+    srid = rid[order]
+    first = np.ones(V, dtype=bool)
+    first[1:] = (srid[1:] != srid[:-1]) | (contig[order][1:] != contig[order][:-1])
+    g_first = np.flatnonzero(first)
+    return order, np.concatenate([g_first, [V]]).astype(np.int64), contig[order][g_first]
