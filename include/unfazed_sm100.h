@@ -524,6 +524,63 @@ int unfz_vcf_samples(UnfzCtx*, const uint8_t* buf, const UnfzVcfRec* recs, const
                      const int32_t* slot_of, int32_t n_samples, int32_t n_members, int32_t gq_float, int32_t max_digits,
                      uint8_t* gt, float* gq, int32_t* rd, int32_t* ad, uint8_t* status, uint8_t* line_bad, void* stream);
 
+/* ---- BCF decoding (csrc/bcf.cu) ----------------------------------------------------------------------
+ * Input: the inflated bytes of the BGZF chunks of a CSI region query (whole BCF 2.2 records back to back).
+ *
+ * The fixed fields of one record, as the parse step reads it.  Offsets are relative to rec_off (the record's l_shared).
+ * rend = pos0 + rlen as stored.  ref / alt: the first two allele strings (alt_len 0 when n_allele < 2), NUL padding
+ * dropped.  fmt_off: the first value of GT, GQ, AD, RO and AO (FORMAT keys given by the host as string-dictionary
+ * indices), -1 when the record has no such field; fmt_ct: values per sample << 4 | BCF type.  Sample s's values of field
+ * k start at rec_off + fmt_off[k] + s * count * width.  flags: UNFZ_BCF_SIMPLE (two alleles, REF and ALT of one base,
+ * ALT not '*'), UNFZ_BCF_BAD with the reason bits.  80 bytes. */
+#define UNFZ_BCF_SIMPLE 0x01
+#define UNFZ_BCF_BAD_OVERRUN 0x02   /* a typed value runs past l_shared or l_indiv */
+#define UNFZ_BCF_BAD_SAMPLES 0x04   /* n_sample differs from the header's sample count */
+#define UNFZ_BCF_BAD_TYPE 0x08      /* a type BCF 2.2 does not define, or a key / count / allele of the wrong type */
+#define UNFZ_BCF_BAD_POS 0x10       /* POS or rlen negative, or pos0 + rlen above INT32_MAX */
+#define UNFZ_BCF_BAD 0x80
+/* per-cell status bit of the sample decode: a reserved integer value, a GT / AD / RO / AO that is not an integer, a GQ
+ * that is neither integer nor float, a negative GT value, or an AD / AO sum that overflows int32 */
+#define UNFZ_BCF_CELL_BAD 0x02
+typedef struct {
+    int64_t  rec_off;     /* byte offset of the record in the buffer */
+    int32_t  contig;      /* CHROM: index into the contig dictionary */
+    int32_t  pos0;
+    int32_t  rend;
+    int32_t  ref_off, ref_len;
+    int32_t  alt_off, alt_len;
+    int32_t  fmt_off[5];  /* GT GQ AD RO AO */
+    uint32_t fmt_ct[5];
+    uint16_t n_allele;
+    uint8_t  ref0;        /* first byte of REF (0 when empty) */
+    uint8_t  flags;
+} UnfzBcfRec;
+
+/* Host only (no device call): the record boundaries of `buf` by walking l_shared + l_indiv from byte 0.  Writes at most
+ * max_records offsets, stops at a record that does not end inside the buffer and stores where the walk stopped in
+ * *end_out.  Returns the number of offsets, or -1 for an l_shared below the 24 bytes of the fixed fields. */
+int64_t unfz_bcf_record_offsets(const uint8_t* buf, int64_t n_bytes, int64_t max_records, int64_t* offs, int64_t* end_out);
+/* Host only: the fixed fields of the n records at offs (the same function the device parse runs).  keys: 5 host int32,
+ * the string-dictionary indices of GT GQ AD RO AO (-1: not in the header); n_samples: the header's sample count.
+ * Returns the number of records with UNFZ_BCF_BAD. */
+int64_t unfz_bcf_parse_host(const uint8_t* buf, const int64_t* offs, int64_t n, const int32_t* keys, int32_t n_samples,
+                            UnfzBcfRec* out);
+/* Host only: the genotype fields of the selected records sel[0..n_sel) (indices into recs) for the member columns;
+ * member_sample[m] is the sample of column m.  Outputs are [n_sel][n_members] with the contract of
+ * unfz_vcf_samples_host: gt (cyvcf2 gt_types), gq (float32, -1 missing), rd (AD[0], or RO), ad (the sum of AD[1:], or
+ * of AO; -1 missing) and status (UNFZ_BCF_CELL_BAD). */
+int unfz_bcf_samples_host(const uint8_t* buf, const UnfzBcfRec* recs, const int64_t* sel, int64_t n_sel,
+                          const int32_t* member_sample, int32_t n_members, uint8_t* gt, float* gq, int32_t* rd, int32_t* ad,
+                          uint8_t* status);
+
+/* Device: unfz_bcf_parse_host, one thread per record (buf, offs, out in device memory; keys in host memory). */
+int unfz_bcf_parse(UnfzCtx*, const uint8_t* buf, const int64_t* offs, int64_t n, const int32_t* keys, int32_t n_samples,
+                   UnfzBcfRec* out, void* stream);
+/* Device: unfz_bcf_samples_host, one thread per (selected record x member) cell. */
+int unfz_bcf_samples(UnfzCtx*, const uint8_t* buf, const UnfzBcfRec* recs, const int64_t* sel, int64_t n_sel,
+                     const int32_t* member_sample, int32_t n_members, uint8_t* gt, float* gq, int32_t* rd, int32_t* ad,
+                     uint8_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -102,6 +102,13 @@ VCF_REC_DTYPE = np.dtype([("line_off", "<i8"), ("line_len", "<i4"), ("pos0", "<i
                           ("ref0", "u1"), ("flags", "u1"), ("_pad", "u1")])
 VCF_SIMPLE, VCF_BAD, VCF_CELL_HOST, VCF_CELL_BAD = 0x01, 0x80, 0x01, 0x02
 assert VCF_REC_DTYPE.itemsize == 64
+# UnfzBcfRec: the fixed fields of one BCF record (csrc/bcf.cu)
+BCF_REC_DTYPE = np.dtype([("rec_off", "<i8"), ("contig", "<i4"), ("pos0", "<i4"), ("rend", "<i4"), ("ref_off", "<i4"),
+                          ("ref_len", "<i4"), ("alt_off", "<i4"), ("alt_len", "<i4"), ("fmt_off", "<i4", (5,)),
+                          ("fmt_ct", "<u4", (5,)), ("n_allele", "<u2"), ("ref0", "u1"), ("flags", "u1")])
+BCF_SIMPLE, BCF_BAD_OVERRUN, BCF_BAD_SAMPLES, BCF_BAD_TYPE, BCF_BAD_POS, BCF_BAD = 0x01, 0x02, 0x04, 0x08, 0x10, 0x80
+BCF_CELL_BAD = 0x02
+assert BCF_REC_DTYPE.itemsize == 80
 assert SEG_DTYPE.itemsize == 32 and DNM_DTYPE.itemsize == 48 and RSUM_DTYPE.itemsize == 32
 
 # constants of include/unfazed_sm100.h
@@ -166,6 +173,11 @@ SYMBOLS = {
     "unfz_vcf_parse": (C.c_int, [_P, _P, _P, c_int64, _P, _P]),
     "unfz_vcf_samples": (C.c_int, [_P, _P, _P, _P, c_int64, _P, c_int32, c_int32, c_int32, c_int32, _P, _P, _P, _P, _P, _P,
                                    _P]),
+    "unfz_bcf_record_offsets": (c_int64, [_P, c_int64, c_int64, _P, _P]),
+    "unfz_bcf_parse_host": (c_int64, [_P, _P, c_int64, _P, c_int32, _P]),
+    "unfz_bcf_samples_host": (C.c_int, [_P, _P, _P, c_int64, _P, c_int32, _P, _P, _P, _P, _P]),
+    "unfz_bcf_parse": (C.c_int, [_P, _P, _P, c_int64, _P, c_int32, _P, _P]),
+    "unfz_bcf_samples": (C.c_int, [_P, _P, _P, _P, c_int64, _P, c_int32, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None

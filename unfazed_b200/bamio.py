@@ -1,6 +1,6 @@
 """Indexed BAM files without pysam: BGZF inflate and BAI region queries on the host, record decoding in native code.
 
-* ``BamFile`` -- one coordinate-sorted BAM and its ``.bai``: the header (reference names and lengths), the BAI bins,
+* ``BamFile`` -- one coordinate-sorted BAM and its ``.bai`` (or ``.csi``): the header (reference names and lengths), the BAI bins,
   chunks and linear index, and region queries that return the records overlapping an interval (htslib's ``reg2bins``
   and linear-index minimum offset, ``bam_endpos`` overlap).  BGZF blocks are inflated with zlib in a thread pool
   (zlib releases the GIL), CRC32 and ISIZE checked, and cached by file offset for the length of one load.
@@ -9,9 +9,12 @@
   else is numpy over the inflated buffer -- no Python work per record except splitting the read names into a list.
   With ``engine=`` the bulk columns (CIGAR, bases, qualities) are decoded on the GPU instead and the table comes back
   as the host half of a device-decoded ``DeviceReads`` (``Engine.decode_bam``).
-* ``write_bam`` -- a coordinate-sorted BAM + BAI from a ``ReadTable`` (tests and tools generate their inputs with it).
+* ``write_bam`` -- a coordinate-sorted BAM + BAI or CSI from a ``ReadTable`` (tests and tools generate their inputs
+  with it).
+* ``CsiIndex`` / ``write_csi`` -- the CSI index (any ``min_shift`` / ``depth``) with the ``chunks`` queries of
+  ``BaiIndex``; a BAM may come with a ``.csi`` instead of a ``.bai``, and ``vcfio`` and ``bcfio`` use it too.
 
-CRAM and CSI indexes are not read here; ``datasource.load_reads`` sends those inputs to pysam.
+CRAM is not read here; ``datasource.load_reads`` sends it to pysam.
 """
 from __future__ import annotations
 
@@ -205,24 +208,41 @@ def _bgzf_block(raw: bytes, level: int) -> bytes:
 # BAI
 # ------------------------------------------------------------------------------------------------
 
-def reg2bins(beg: int, end: int) -> List[int]:
-    """htslib's reg2bins: the bins that may hold records overlapping [beg, end) (0-based, half-open)."""
+def reg2bins(beg: int, end: int, min_shift: int = 14, depth: int = 5) -> List[int]:
+    """htslib's reg2bins: the bins that may hold records overlapping [beg, end) (0-based, half-open) in a binning of
+    ``depth`` levels below the root whose leaves span 2^min_shift bases ((14, 5): BAI and TBI)."""
     if beg >= end:
         return []
     end -= 1
-    bins = [0]
-    for shift, off in ((26, 1), (23, 9), (20, 73), (17, 585), (14, 4681)):
-        bins += range(off + (beg >> shift), off + (end >> shift) + 1)
+    bins: List[int] = []
+    s, t = min_shift + 3 * depth, 0
+    for lvl in range(depth + 1):
+        bins += range(t + (beg >> s), t + (end >> s) + 1)
+        s -= 3
+        t += 1 << (3 * lvl)
     return bins
 
 
-def reg2bin(beg: int, end: int) -> int:
+def reg2bin(beg: int, end: int, min_shift: int = 14, depth: int = 5) -> int:
     """htslib's reg2bin: the smallest bin containing [beg, end)."""
     end -= 1
-    for shift, off in ((14, 4681), (17, 585), (20, 73), (23, 9), (26, 1)):
-        if beg >> shift == end >> shift:
-            return off + (beg >> shift)
+    s, t = min_shift, ((1 << (3 * depth)) - 1) // 7
+    for lvl in range(depth, 0, -1):
+        if beg >> s == end >> s:
+            return t + (beg >> s)
+        s += 3
+        t -= 1 << (3 * (lvl - 1))
     return 0
+
+
+def bin_first(lvl: int) -> int:
+    """The first bin of level ``lvl`` (the root is level 0)."""
+    return ((1 << (3 * lvl)) - 1) // 7
+
+
+def pseudo_bin(depth: int) -> int:
+    """The bin number that holds the mapped / unmapped counts of a reference (37450 at depth 5)."""
+    return bin_first(depth + 1) + 1
 
 
 def parse_bins(d: bytes, p: int, n_ref: int) -> Tuple[List[Dict[int, np.ndarray]], List[np.ndarray], int]:
@@ -251,6 +271,7 @@ def parse_bins(d: bytes, p: int, n_ref: int) -> Tuple[List[Dict[int, np.ndarray]
 
 class BaiIndex:
     """Bins (bin -> chunk array [n, 2] of virtual offsets) and linear index of every reference."""
+    min_shift, depth = 14, 5
 
     def __init__(self, path: str):
         d = open(path, "rb").read()
@@ -259,18 +280,21 @@ class BaiIndex:
         n_ref = struct.unpack_from("<i", d, 4)[0]
         self.bins, self.linear, _ = parse_bins(d, 8, n_ref)
 
+    def min_offset(self, tid: int, beg: int) -> int:
+        """The virtual offset before which no record overlapping beg starts: the linear index at beg's 16 kb window."""
+        lin = self.linear[tid]
+        return int(lin[min(beg >> 14, lin.shape[0] - 1)]) if lin.shape[0] else 0
+
     def chunks(self, tid: int, beg: int, end: int) -> List[Tuple[int, int]]:
-        """Merged chunk list of [beg, end) on reference tid: the chunks of reg2bins' bins that end after the linear
-        index's minimum offset, sorted and merged.  A zero-length interval asks for the records covering beg (the
+        """Merged chunk list of [beg, end) on reference tid: the chunks of reg2bins' bins that end after the minimum
+        offset (``min_offset``), sorted and merged.  A zero-length interval asks for the records covering beg (the
         overlap test pos < end and bam_endpos > beg is the caller's)."""
         end = max(end, beg + 1)
-        if tid >= len(self.bins):
+        if tid < 0 or tid >= len(self.bins):
             return []
-        bins, lin = self.bins[tid], self.linear[tid]
-        min_off = 0
-        if lin.shape[0]:
-            min_off = int(lin[min(beg >> 14, lin.shape[0] - 1)])
-        ch = [bins[b] for b in reg2bins(beg, end) if b in bins]
+        bins = self.bins[tid]
+        min_off = self.min_offset(tid, beg)
+        ch = [bins[b] for b in reg2bins(beg, end, self.min_shift, self.depth) if b in bins]
         if not ch:
             return []
         c = np.concatenate(ch)
@@ -287,28 +311,89 @@ class BaiIndex:
         return [(max(b, min_off), e) for b, e in out]
 
 
+class CsiIndex(BaiIndex):
+    """A CSI index (BGZF-compressed): ``min_shift`` and ``depth`` of its binning, the ``aux`` bytes (a tabix header for a
+    .vcf.gz, empty for BCF and BAM; ``names`` holds the reference names of a tabix header, else None), and per
+    reference the bins with their chunks and ``loffset``.  There is no linear index: the minimum offset of a query is the
+    ``loffset`` of the nearest existing bin at or left of beg's leaf bin, walking towards the root (htslib's
+    ``hts_itr_query``).  Region queries are ``BaiIndex.chunks``."""
+
+    def __init__(self, path: str):
+        raw, _ = BgzfReader(path).stream_from(0, 1 << 62)
+        d = raw.tobytes()
+        if d[:4] != b"CSI\x01" or len(d) < 16:
+            raise ValueError("%s: not a CSI index" % path)
+        self.min_shift, self.depth, l_aux = struct.unpack_from("<3i", d, 4)
+        if not (0 < self.min_shift and 0 < self.depth and self.min_shift + 3 * self.depth < 64) or l_aux < 0:
+            raise ValueError("%s: CSI min_shift %d / depth %d out of range" % (path, self.min_shift, self.depth))
+        self.aux = d[16:16 + l_aux]
+        self.names = None
+        if l_aux >= 28:                                        # tabix header: format, columns, meta, skip, names
+            l_nm = struct.unpack_from("<i", self.aux, 24)[0]
+            self.names = [x.decode() for x in self.aux[28:28 + l_nm].split(b"\0") if x]
+        p = 16 + l_aux
+        try:
+            n_ref = struct.unpack_from("<i", d, p)[0]
+            p += 4
+            pseudo = pseudo_bin(self.depth)
+            self.bins, self.loff = [], []
+            for _ in range(n_ref):
+                n_bin = struct.unpack_from("<i", d, p)[0]
+                p += 4
+                bins, loff = {}, {}
+                for _ in range(n_bin):
+                    b, lo, n_chunk = struct.unpack_from("<IQi", d, p)
+                    p += 16
+                    ch = np.frombuffer(d, dtype="<u8", count=2 * n_chunk, offset=p).reshape(n_chunk, 2)
+                    p += 16 * n_chunk
+                    if b != pseudo:
+                        bins[b], loff[b] = ch, lo
+                self.bins.append(bins)
+                self.loff.append(loff)
+        except (struct.error, ValueError):
+            raise ValueError("%s: truncated CSI index" % path)
+
+    def min_offset(self, tid: int, beg: int) -> int:
+        loff = self.loff[tid]
+        b = bin_first(self.depth) + (beg >> self.min_shift)
+        while b and b not in loff:
+            first = (((b - 1) >> 3) << 3) + 1                  # the first child of b's parent
+            b = b - 1 if b > first else (b - 1) >> 3
+        return loff.get(b, 0)
+
+
+def open_index(path: str):
+    """The BAI (uncompressed, ``BAI\\1``) or CSI (BGZF) index of a BAM at ``path``, by its first bytes."""
+    with open(path, "rb") as f:
+        head = f.read(4)
+    return BaiIndex(path) if head == b"BAI\x01" else CsiIndex(path)
+
+
 # ------------------------------------------------------------------------------------------------
 # BAM file
 # ------------------------------------------------------------------------------------------------
 
 def index_path(path: str) -> Optional[str]:
-    """``<file>.bam.bai`` or ``<file>.bai`` if one exists."""
-    for p in (path + ".bai", os.path.splitext(path)[0] + ".bai"):
+    """The index of a BAM: ``<file>.bam.bai`` or ``<file>.bai`` if one exists, else ``<file>.bam.csi`` or
+    ``<file>.csi``."""
+    stem = os.path.splitext(path)[0]
+    for p in (path + ".bai", stem + ".bai", path + ".csi", stem + ".csi"):
         if os.path.exists(p):
             return p
     return None
 
 
 class BamFile:
-    """One indexed BAM: header, BAI and region queries.  Records come back as (buffer, offsets, parsed fields)."""
+    """One indexed BAM: header, BAI or CSI index and region queries.  Records come back as (buffer, offsets, parsed
+    fields)."""
 
     def __init__(self, path: str, index: Optional[str] = None):
         self.path = path
         self.bgzf = BgzfReader(path)
         ip = index or index_path(path)
         if ip is None:
-            raise ValueError("%s: no .bai index" % path)
-        self.bai = BaiIndex(ip)
+            raise ValueError("%s: no .bai or .csi index" % path)
+        self.bai = open_index(ip)
         head, _ = self.bgzf.stream_from(0, 1 << 16)
         hb = head.tobytes()
         need = 12
@@ -739,8 +824,9 @@ def encode_tag(tag: str, typ: str, value) -> bytes:
 def write_bam(table: ReadTable, kid: int, path: str, extra_tags: Optional[Dict[int, bytes]] = None,
               missing_qual: Optional[np.ndarray] = None, other_ref: Optional[np.ndarray] = None,
               ref_lens: Optional[Dict[str, int]] = None, level: int = 6, chunk_reads: int = 1 << 18,
-              common_tags: bytes = b"") -> None:
-    """Coordinate-sorted BAM + BAI (``path + ".bai"``) of kid ``kid``'s reads of ``table``.
+              common_tags: bytes = b"", index: str = "bai") -> None:
+    """Coordinate-sorted BAM + index of kid ``kid``'s reads of ``table``: ``path + ".bai"``, or with ``index="csi"``
+    ``path + ".csi"`` (min_shift 14, depth 5, as ``samtools index -c`` writes it).
 
     References: ``table.contigs`` in table order (a contig without reads of this kid is an empty reference).  Names:
     ``table.names`` or the synthesized pair names.  Bases: A C G T as they are; an escaped code 0 is N and an escaped
@@ -844,8 +930,14 @@ def write_bam(table: ReadTable, kid: int, path: str, extra_tags: Optional[Dict[i
         pos_u += int(size.sum())
         stream.append(data.tobytes())
     voff = write_bgzf(path, bytes(head), b"".join(stream), level)
-    _write_bai(path + ".bai", n_ref, tid_of_row, t.hdr["start"][rows].astype(np.int64), ends[rows],
-               voff(rec_start[:-1]), voff(rec_start[1:]))
+    cols = (n_ref, tid_of_row, t.hdr["start"][rows].astype(np.int64), ends[rows], voff(rec_start[:-1]),
+            voff(rec_start[1:]))
+    if index == "csi":
+        write_csi(path + ".csi", *cols)
+    elif index == "bai":
+        _write_bai(path + ".bai", *cols)
+    else:
+        raise ValueError("index must be 'bai' or 'csi', not %r" % index)
 
 
 def write_bgzf(path: str, head: bytes, body: bytes, level: int = 6):
@@ -918,5 +1010,63 @@ def index_refs(n_ref: int, tid: np.ndarray, pos: np.ndarray, end_raw: np.ndarray
             last = lin.get(w, last)
             vals.append(last)
         out += struct.pack("<i", n_intv) + struct.pack("<%dQ" % n_intv, *vals)
+    out += struct.pack("<Q", 0)
+    return bytes(out)
+
+
+def csi_depth(max_end: int, min_shift: int = 14) -> int:
+    """The smallest depth (at least 5) whose binning spans [0, max_end), as htslib sizes a CSI."""
+    depth = 5
+    while (1 << (min_shift + 3 * depth)) < max_end:
+        depth += 1
+    return depth
+
+
+def write_csi(path: str, n_ref: int, tid: np.ndarray, pos: np.ndarray, end_raw: np.ndarray, vbeg: np.ndarray,
+              vend: np.ndarray, min_shift: int = 14, depth: Optional[int] = None, aux: bytes = b"",
+              level: int = 6) -> None:
+    """CSI (BGZF-compressed) of records sorted by (tid, pos) spanning [pos, end_raw) at virtual offsets [vbeg, vend).
+    ``depth`` None: the smallest that spans the records.  ``aux``: the tabix header of a .vcf.gz index, empty for BCF and
+    BAM."""
+    if depth is None:
+        depth = csi_depth(int(np.max(np.maximum(end_raw, pos + 1))) if len(pos) else 1, min_shift)
+    body = (b"CSI\x01" + struct.pack("<3i", min_shift, depth, len(aux)) + aux + struct.pack("<i", n_ref)
+            + csi_refs(n_ref, tid, pos, end_raw, vbeg, vend, min_shift, depth))
+    write_bgzf(path, body, b"", level)
+
+
+def csi_refs(n_ref: int, tid: np.ndarray, pos: np.ndarray, end_raw: np.ndarray, vbeg: np.ndarray, vend: np.ndarray,
+             min_shift: int, depth: int) -> bytes:
+    """The per-reference part of a CSI: per reference the bins (chunks of consecutive records of the same bin merged)
+    with their ``loffset`` -- the virtual offset of the first record that ends after the bin's start, so no record before
+    it overlaps the bin -- and the pseudo-bin of counts; then the count of records without a coordinate (0)."""
+    tid = np.asarray(tid, dtype=np.int64)
+    pos = np.asarray(pos, dtype=np.int64)
+    end = np.maximum(np.asarray(end_raw, dtype=np.int64), pos + 1)
+    out = bytearray()
+    for t in range(n_ref):
+        sel = np.flatnonzero(tid == t)
+        bins: Dict[int, List[List[int]]] = {}
+        for i in sel.tolist():
+            b = reg2bin(int(pos[i]), int(end[i]), min_shift, depth)
+            ch = bins.setdefault(b, [])
+            vb, ve = int(vbeg[i]), int(vend[i])
+            if ch and ch[-1][1] == vb:
+                ch[-1][1] = ve
+            else:
+                ch.append([vb, ve])
+        run_end = np.maximum.accumulate(end[sel]) if sel.shape[0] else end[sel]
+        out += struct.pack("<i", len(bins) + (1 if sel.shape[0] else 0))
+        for b in sorted(bins):
+            lvl = next(l for l in range(depth, -1, -1) if b >= bin_first(l))
+            start = (b - bin_first(lvl)) << (min_shift + 3 * (depth - lvl))
+            first = int(np.searchsorted(run_end, start, side="right"))
+            loff = int(vbeg[sel[first]]) if first < sel.shape[0] else 0
+            out += struct.pack("<IQi", b, loff, len(bins[b]))
+            for vb, ve in bins[b]:
+                out += struct.pack("<QQ", vb, ve)
+        if sel.shape[0]:
+            out += struct.pack("<IQi", pseudo_bin(depth), 0, 2) + struct.pack("<QQ", int(vbeg[sel[0]]), int(vend[sel[-1]]))
+            out += struct.pack("<QQ", sel.shape[0], 0)
     out += struct.pack("<Q", 0)
     return bytes(out)

@@ -3,9 +3,11 @@
 * ``*.npz`` written by ``tableio.save_tables`` (our native cache of decoded inputs), or
 * indexed BAM files (``*.bam`` with a ``.bai``) through ``bamio.py``, natively -- no pysam needed, and with an
   engine the bulk of the records is decoded on the GPU, or
-* a bgzipped, tabix-indexed sites VCF (``*.vcf.gz`` / ``*.vcf.bgz`` with a ``.tbi``) through ``vcfio.py``, natively --
-  no cyvcf2 needed, and with an engine the genotype fields are decoded on the GPU, or
-* other sites VCF/BCF files through ``cyvcf2`` and the kids' other alignment files (CRAM, unindexed BAM) through ``pysam``
+* indexed BAM files (``*.bam`` with a ``.bai`` or ``.csi``) through ``bamio.py`` as above, or
+* a bgzipped, indexed sites VCF (``*.vcf.gz`` / ``*.vcf.bgz`` with a ``.tbi`` or ``.csi``) through ``vcfio.py``, natively
+  -- no cyvcf2 needed, and with an engine the genotype fields are decoded on the GPU, or
+* a CSI-indexed BCF 2.2 sites file (``*.bcf`` with a ``.csi``) through ``bcfio.py``, natively, likewise, or
+* other sites VCF/BCF files (unindexed, uncompressed BCF, other BCF versions) through ``cyvcf2`` and the kids' other alignment files (CRAM, unindexed BAM) through ``pysam``
   -- imported lazily, so the package works without them as long as tables are supplied -- decoded only around
   the DNMs and packed by ``packers.py``.
 
@@ -19,7 +21,7 @@ from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 
-from . import bamio, packers, vcfio
+from . import bamio, bcfio, packers, vcfio
 from .plan import strip_chr
 from .schema import ReadTable, SiteTable
 from .tableio import load_tables
@@ -50,21 +52,39 @@ def _toggle(chrom: str) -> str:
 
 
 def is_indexed_vcf(name: str) -> bool:
-    """An existing ``*.vcf.gz`` / ``*.vcf.bgz`` file with a ``.tbi`` next to it: read natively by ``vcfio``."""
+    """An existing ``*.vcf.gz`` / ``*.vcf.bgz`` file with a ``.tbi`` or ``.csi`` next to it: read natively by
+    ``vcfio``."""
     return name.endswith((".vcf.gz", ".vcf.bgz")) and os.path.isfile(name) and vcfio.index_path(name) is not None
 
 
+def is_indexed_bcf(name: str) -> bool:
+    """An existing BGZF-compressed ``*.bcf`` file with a ``.csi`` next to it that is not a BCF of another version than
+    2.2: read natively by ``bcfio`` (whose reader rejects a file that is not BCF at all)."""
+    if not (name.endswith(".bcf") and os.path.isfile(name) and bcfio.index_path(name) is not None):
+        return False
+    with open(name, "rb") as f:
+        if f.read(4) != b"\x1f\x8b\x08\x04":
+            return False                               # uncompressed BCF
+    head, _ = bamio.BgzfReader(name).stream_from(0, 5)
+    magic = head[:5].tobytes()
+    return not (magic[:3] == b"BCF" and magic != bcfio.MAGIC)
+
+
 def load_sites(vcf_name: str, dnms: List[dict], pedigrees: dict, search_dist: int, engine=None) -> SiteTable:
-    """The SiteTable of the trios of the DNM list around their DNMs.  A tabix-indexed ``.vcf.gz`` is read by ``vcfio``
-    (with ``engine``, its genotype fields are decoded on that engine's GPU); BCF, CSI-indexed or unindexed files go
-    through cyvcf2."""
+    """The SiteTable of the trios of the DNM list around their DNMs.  An indexed ``.vcf.gz`` is read by ``vcfio`` and a
+    CSI-indexed BCF 2.2 by ``bcfio`` (with ``engine``, their genotype fields are decoded on that engine's GPU); other
+    BCF and unindexed files go through cyvcf2."""
     if vcf_name in _registry and _registry[vcf_name][0] is not None:
         return _registry[vcf_name][0]
     if vcf_name.endswith(".npz"):
         return _npz(vcf_name)[0]
     native = is_indexed_vcf(vcf_name)
+    bcf = not native and is_indexed_bcf(vcf_name)
     if native:
         vf = vcfio.VcfFile(vcf_name)
+        prefix = vf.prefix
+    elif bcf:
+        vf = bcfio.BcfFile(vcf_name)
         prefix = vf.prefix
     else:
         from cyvcf2 import VCF
@@ -83,11 +103,13 @@ def load_sites(vcf_name: str, dnms: List[dict], pedigrees: dict, search_dist: in
         regions.setdefault(contig, []).append((s - search_dist - 2, e + search_dist + 2))
     if native:
         return vcfio.read_sites(vf, trios, regions, engine=engine)
+    if bcf:
+        return bcfio.read_sites(vf, trios, regions, engine=engine)
     return packers.pack_sites(VCF(vcf_name), trios, regions)
 
 
 def is_indexed_bam(name: str) -> bool:
-    """An existing ``*.bam`` file with a ``.bai`` next to it: read natively by ``bamio``."""
+    """An existing ``*.bam`` file with a ``.bai`` or ``.csi`` next to it: read natively by ``bamio``."""
     return name.endswith(".bam") and os.path.isfile(name) and bamio.index_path(name) is not None
 
 

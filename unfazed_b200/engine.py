@@ -402,6 +402,84 @@ class VcfDecoder:
         return res
 
 
+class BcfDecoder:
+    """Device side of ``bcfio.read_sites(engine=...)``, with the calls of ``bcfio.HostDecoder``: the inflated record
+    bytes go up once (pinned staging) with the record offsets the host walked, unfz_bcf_parse runs on the engine's stream
+    and the 80-byte records come back for the host's selection; then unfz_bcf_samples decodes the member cells of the
+    selected records -- one thread per cell, a direct load at the field's sample stride -- which come back as the
+    table's genotype arrays."""
+
+    def __init__(self, engine: "Engine"):
+        self.engine = engine
+        self.h2d_bytes = self.d2h_bytes = 0
+        self.timings_ms: Dict[str, float] = {}
+
+    def _time(self, name, e0, e1):
+        self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
+
+    def records(self, buf: np.ndarray, offs: np.ndarray, keys: np.ndarray, n_samples: int) -> np.ndarray:
+        eng = self.engine
+        lib, ctx, dev = eng.lib, eng.ctx, eng.device
+        n = int(offs.shape[0])
+        keys = np.ascontiguousarray(keys, dtype=np.int32)
+        with eng.on_stream():
+            st = torch.cuda.current_stream(dev)
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+            e[0].record(st)
+            self.dbuf = _to_device(np.ascontiguousarray(buf), dev, True) if buf.shape[0] else \
+                torch.zeros(16, dtype=torch.uint8, device=dev)
+            doffs = _to_device(np.ascontiguousarray(offs, dtype=np.int64), dev, True) if n else \
+                torch.zeros(1, dtype=torch.int64, device=dev)
+            e[1].record(st)
+            rsz = L.BCF_REC_DTYPE.itemsize
+            self.drecs = torch.empty((max(n, 1) * rsz,), dtype=torch.uint8, device=dev)
+            eng._check(lib.unfz_bcf_parse(ctx, self.dbuf.data_ptr(), doffs.data_ptr(), n, keys.ctypes.data, int(n_samples),
+                                          self.drecs.data_ptr(), C.c_void_p(st.cuda_stream)), "bcf_parse")
+            e[2].record(st)
+            recs = self.drecs[: n * rsz].cpu().numpy().view(L.BCF_REC_DTYPE)
+            e[3].record(st)
+        e[3].synchronize()
+        self._time("h2d_records", e[0], e[1])
+        self._time("parse", e[1], e[2])
+        self._time("d2h_records", e[2], e[3])
+        self.h2d_bytes += int(buf.nbytes + offs.nbytes)
+        self.d2h_bytes += int(recs.nbytes)
+        return recs
+
+    def samples(self, sel: np.ndarray, member_sample: np.ndarray) -> Dict[str, np.ndarray]:
+        eng = self.engine
+        lib, ctx, dev = eng.lib, eng.ctx, eng.device
+        ns, m = int(sel.shape[0]), int(member_sample.shape[0])
+        cells = ns * m
+        with eng.on_stream():
+            st = torch.cuda.current_stream(dev)
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+            e[0].record(st)
+            dsel = _to_device(np.ascontiguousarray(sel, dtype=np.int64), dev, True) if ns else \
+                torch.zeros(1, dtype=torch.int64, device=dev)
+            dms = _to_device(np.ascontiguousarray(member_sample, dtype=np.int32), dev, True) if m else \
+                torch.zeros(1, dtype=torch.int32, device=dev)
+            e[1].record(st)
+            out = {"gt": torch.empty((max(cells, 1),), dtype=torch.uint8, device=dev),
+                   "gq": torch.empty((max(cells, 1),), dtype=torch.float32, device=dev),
+                   "rd": torch.empty((max(cells, 1),), dtype=torch.int32, device=dev),
+                   "ad": torch.empty((max(cells, 1),), dtype=torch.int32, device=dev),
+                   "status": torch.empty((max(cells, 1),), dtype=torch.uint8, device=dev)}
+            eng._check(lib.unfz_bcf_samples(ctx, self.dbuf.data_ptr(), self.drecs.data_ptr(), dsel.data_ptr(), ns,
+                                            dms.data_ptr(), m, *(out[k].data_ptr() for k in ("gt", "gq", "rd", "ad", "status")),
+                                            C.c_void_p(st.cuda_stream)), "bcf_samples")
+            e[2].record(st)
+            host = {k: v.cpu().numpy() for k, v in out.items()}
+            e[3].record(st)
+        e[3].synchronize()
+        self._time("h2d_select", e[0], e[1])
+        self._time("samples", e[1], e[2])
+        self._time("d2h_cells", e[2], e[3])
+        self.h2d_bytes += int(sel.nbytes + member_sample.nbytes)
+        self.d2h_bytes += cells * 14
+        return {k: host[k][:cells].reshape(ns, m) for k in ("gt", "gq", "rd", "ad", "status")}
+
+
 def _to_device(a: np.ndarray, device, pin: bool, pad: int = 0) -> torch.Tensor:
     """Host array -> device tensor (+ ``pad`` zero elements).  Arrays that already live in pinned
     memory are copied asynchronously; ``pin`` stages pageable arrays through a pinned copy."""
@@ -624,6 +702,10 @@ class Engine:
     def vcf_decoder(self) -> VcfDecoder:
         """A device decoder for one ``vcfio.read_sites`` load."""
         return VcfDecoder(self)
+
+    def bcf_decoder(self) -> BcfDecoder:
+        """A device decoder for one ``bcfio.read_sites`` load."""
+        return BcfDecoder(self)
 
     def decode_bam(self, paths, regions, head_reads: int = 0, min_gt_qual=20) -> DeviceReads:
         """Indexed BAM files -> DeviceReads, the bulk of the records decoded on this GPU (``bamio.read_regions``).

@@ -43,9 +43,12 @@ def read_vars_bedzip(bedzipname):
 
 
 def read_vars_vcf(vcfname):
-    if not vcfname.endswith(".bcf") and os.path.isfile(vcfname):
-        # an existing .vcf / .vcf.gz: read natively (vcfio), no cyvcf2 needed
-        from .vcfio import read_dnms
+    if os.path.isfile(vcfname):
+        # an existing .vcf / .vcf.gz / .bcf: read natively (vcfio, bcfio), no cyvcf2 needed
+        if vcfname.endswith(".bcf"):
+            from .bcfio import read_dnms
+        else:
+            from .vcfio import read_dnms
         yield from read_dnms(vcfname)
         return
     from cyvcf2 import VCF

@@ -1,7 +1,7 @@
 """Tabix-indexed sites VCFs without cyvcf2: BGZF inflate and TBI region queries on the host, field decoding in native
 code (csrc/vcf.cu), on the GPU with an engine.
 
-* ``VcfFile`` -- one bgzipped VCF and its ``.tbi``: the header (sample names, the declared Type of the GQ / AD / RO /
+* ``VcfFile`` -- one bgzipped VCF and its ``.tbi`` or ``.csi``: the header (sample names, the declared Type of the GQ / AD / RO /
   AO FORMAT fields, the first record's CHROM for ``get_prefix``) and region queries (``TbiIndex``: the BAI bins, chunks
   and linear index behind a tabix header, read by ``bamio``'s code; overlap by tabix's end, INFO END or POS + len(REF)).
 * ``read_sites`` -- the ``SiteTable`` ``packers.pack_sites`` builds from a cyvcf2 handle over the same regions, array
@@ -11,8 +11,9 @@ code (csrc/vcf.cu), on the GPU with an engine.
 * ``read_dnms`` -- the DNM dicts ``unfazed.read_vars_vcf`` yields, from a plain or gzipped VCF read whole.
 * ``write_vcf`` -- a sorted ``.vcf.gz`` + ``.tbi`` from a ``SiteTable`` (tests and tools generate their inputs with it).
 
-Field decoding follows cyvcf2 0.31.0's defaults (gts012=False, strict_gt=False); DESIGN §5 lists the assumptions.  BCF,
-CSI indexes and unindexed files are not read here: ``datasource.load_sites`` sends them to cyvcf2.
+Field decoding follows cyvcf2 0.31.0's defaults (gts012=False, strict_gt=False); DESIGN §5 lists the assumptions.  A
+``.csi`` index (``bamio.CsiIndex``, with the tabix header in its aux bytes) serves where no ``.tbi`` exists.  BCF is read
+by ``bcfio``, which shares the interval selection (``select_records``); unindexed files go to cyvcf2.
 """
 from __future__ import annotations
 
@@ -25,7 +26,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib as L
-from .bamio import BaiIndex, BgzfReader, index_refs, parse_bins, write_bgzf
+from .bamio import BaiIndex, BgzfReader, CsiIndex, index_refs, parse_bins, write_bgzf, write_csi
 from .packers import _merge, build_site_table
 from .schema import GT_UNKNOWN, HET, HOM_ALT, HOM_REF, SiteTable
 
@@ -122,9 +123,21 @@ class TbiIndex(BaiIndex):
 
 
 def index_path(path: str) -> Optional[str]:
-    """``<file>.tbi`` if it exists."""
-    p = path + ".tbi"
-    return p if os.path.exists(p) else None
+    """``<file>.tbi`` if it exists, else ``<file>.csi`` if it exists."""
+    for p in (path + ".tbi", path + ".csi"):
+        if os.path.exists(p):
+            return p
+    return None
+
+
+def open_tabix_index(path: str):
+    """The TBI or CSI index of a bgzipped VCF; both carry the tabix header with the reference names."""
+    if path.endswith(".csi"):
+        idx = CsiIndex(path)
+        if idx.names is None:
+            raise ValueError("%s: a CSI index without a tabix header cannot index a VCF" % path)
+        return idx
+    return TbiIndex(path)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -165,15 +178,15 @@ def _parse_header(text: bytes, path: str):
 
 
 class VcfFile:
-    """One bgzipped, tabix-indexed VCF: header and region queries."""
+    """One bgzipped VCF indexed by a TBI or a CSI: header and region queries."""
 
     def __init__(self, path: str, index: Optional[str] = None):
         self.path = path
         self.bgzf = BgzfReader(path)
         ip = index or index_path(path)
         if ip is None:
-            raise ValueError("%s: no .tbi index" % path)
-        self.tbi = TbiIndex(ip)
+            raise ValueError("%s: no .tbi or .csi index" % path)
+        self.tbi = open_tabix_index(ip)
         self.tids = {n: i for i, n in enumerate(self.tbi.names)}
         want = 1 << 16
         while True:
@@ -205,7 +218,7 @@ class VcfFile:
         parts = self.bgzf.read_ranges([(b, e) for b, e in merged])
         for (vb, _), p in zip(merged, parts):
             if p.shape[0] and p[-1] != 10:
-                raise ValueError("%s: the TBI chunk at virtual offset %d does not end on a line boundary" % (self.path, vb))
+                raise ValueError("%s: the index chunk at virtual offset %d does not end on a line boundary" % (self.path, vb))
         starts = np.cumsum([0] + [p.shape[0] for p in parts])
         buf = np.concatenate(parts) if parts else np.zeros(0, dtype=np.uint8)
 
@@ -265,33 +278,18 @@ def _chrom_ids(buf: np.ndarray, recs: np.ndarray, tids: Dict[str, int], where) -
 # site reader
 # ------------------------------------------------------------------------------------------------
 
-def read_sites(path, trios: Sequence[Tuple[str, str, str]], regions: Dict[str, List[Tuple[int, int]]], engine=None,
-               max_digits: int = FAST_DIGITS) -> SiteTable:
-    """``packers.pack_sites(VCF(path), trios, regions)`` from the file directly.  ``path``: a file name or a
-    ``VcfFile``.  With ``engine`` the text is decoded on that engine's GPU (``Engine.vcf_decoder``).  ``max_digits``:
-    significant digits a float GQ may have to be decoded natively (0 sends every float GQ to the host decode)."""
-    vf = path if isinstance(path, VcfFile) else VcfFile(path)
-    sidx = {s: i for i, s in enumerate(vf.samples)}
-    cols_s = [(t, [sidx[m] for m in trio]) for t, trio in enumerate(trios) if all(m in sidx for m in trio)]
-    slot_of = np.full(len(vf.samples), -1, dtype=np.int32)
-    n_members = 0
-    for _t, ix in cols_s:
-        for s in ix:
-            if slot_of[s] < 0:
-                slot_of[s] = n_members
-                n_members += 1
-    cols = [(t, [int(slot_of[s]) for s in ix]) for t, ix in cols_s]
-    # every merged interval, queried as pack_sites queries it: [max(a, 0), max(b, 1)) by overlap
-    plan = []
-    for contig, ivs in regions.items():
-        plan.append((contig, vf.tids.get(contig), [(max(a, 0), max(b, 1)) for a, b in _merge(ivs)]))
-    queries = [(tid, beg, end) for _c, tid, iv in plan if tid is not None for beg, end in iv]
-    buf, where = vf.fetch_union(queries)
-    dec = engine.vcf_decoder() if engine is not None else HostDecoder()
-    recs = _lines(dec, buf, where)
-    tid_of = _chrom_ids(buf, recs, vf.tids, where)
-    pos0 = recs["pos0"].astype(np.int64)
-    rend = recs["rend"].astype(np.int64)
+def query_plan(regions: Dict[str, List[Tuple[int, int]]], tids: Dict[str, int]):
+    """Every merged interval of every contig, as ``pack_sites`` queries it -- [max(a, 0), max(b, 1)) by overlap: a list
+    of (contig, reference id or None, intervals), and the (tid, beg, end) queries of the contigs the file has."""
+    plan = [(contig, tids.get(contig), [(max(a, 0), max(b, 1)) for a, b in _merge(ivs)]) for contig, ivs in regions.items()]
+    return plan, [(tid, beg, end) for _c, tid, iv in plan if tid is not None for beg, end in iv]
+
+
+def select_records(plan, tid_of: np.ndarray, pos0: np.ndarray, rend: np.ndarray):
+    """The records a region query per merged interval returns, in the order ``pack_sites`` visits them: (record indices,
+    contig index of each into ``contigs``, ``contigs``).  ``tid_of`` / ``pos0`` / ``rend``: reference id, 0-based start
+    and end of every decoded record (file order, so sorted by position within a reference).  A record that an earlier
+    disjoint interval of its contig already returned is not returned again."""
     parts, cid_parts, contigs = [], [], []
     for contig, tid, iv in plan:
         if tid is None:
@@ -320,6 +318,39 @@ def read_sites(path, trios: Sequence[Tuple[str, str, str]], regions: Dict[str, L
             contigs.append(contig)
     sel = np.concatenate(parts) if parts else np.zeros(0, dtype=np.int64)
     cid = np.concatenate(cid_parts) if cid_parts else np.zeros(0, dtype=np.int64)
+    return sel, cid, contigs
+
+
+def member_columns(samples: Sequence[str], trios: Sequence[Tuple[str, str, str]]):
+    """The member columns of the trios whose three samples are all in the file: (slot_of: sample -> column or -1, the
+    number of columns, [(trio index, [column of kid, dad, mom])])."""
+    sidx = {s: i for i, s in enumerate(samples)}
+    cols_s = [(t, [sidx[m] for m in trio]) for t, trio in enumerate(trios) if all(m in sidx for m in trio)]
+    slot_of = np.full(len(samples), -1, dtype=np.int32)
+    n_members = 0
+    for _t, ix in cols_s:
+        for s in ix:
+            if slot_of[s] < 0:
+                slot_of[s] = n_members
+                n_members += 1
+    return slot_of, n_members, [(t, [int(slot_of[s]) for s in ix]) for t, ix in cols_s]
+
+
+def read_sites(path, trios: Sequence[Tuple[str, str, str]], regions: Dict[str, List[Tuple[int, int]]], engine=None,
+               max_digits: int = FAST_DIGITS) -> SiteTable:
+    """``packers.pack_sites(VCF(path), trios, regions)`` from the file directly.  ``path``: a file name or a
+    ``VcfFile``.  With ``engine`` the text is decoded on that engine's GPU (``Engine.vcf_decoder``).  ``max_digits``:
+    significant digits a float GQ may have to be decoded natively (0 sends every float GQ to the host decode)."""
+    vf = path if isinstance(path, VcfFile) else VcfFile(path)
+    slot_of, n_members, cols = member_columns(vf.samples, trios)
+    plan, queries = query_plan(regions, vf.tids)
+    buf, where = vf.fetch_union(queries)
+    dec = engine.vcf_decoder() if engine is not None else HostDecoder()
+    recs = _lines(dec, buf, where)
+    tid_of = _chrom_ids(buf, recs, vf.tids, where)
+    pos0 = recs["pos0"].astype(np.int64)
+    rend = recs["rend"].astype(np.int64)
+    sel, cid, contigs = select_records(plan, tid_of, pos0, rend)
     r = recs[sel]
     simple = (r["flags"] & L.VCF_SIMPLE) != 0
     alt_b = np.zeros(sel.shape[0], dtype=np.uint8)
@@ -390,8 +421,10 @@ def _float_text(x: np.float32) -> str:
 
 
 def write_vcf(table: SiteTable, path: str, end: Optional[Dict[int, int]] = None,
-              format_order: Optional[Sequence[Sequence[str]]] = None, level: int = 6) -> None:
-    """Sorted ``path`` (.vcf.gz) + ``path.tbi`` of ``table``: one line per record (rows grouped by ``rec_id`` and contig,
+              format_order: Optional[Sequence[Sequence[str]]] = None, level: int = 6, index: str = "tbi",
+              min_shift: int = 14, depth: Optional[int] = None) -> None:
+    """Sorted ``path`` (.vcf.gz) + ``path.tbi`` (or with ``index="csi"`` ``path.csi`` of ``min_shift`` / ``depth``, depth
+    None: the smallest that spans the records) of ``table``: one line per record (rows grouped by ``rec_id`` and contig,
     as ``oracle.fakes`` groups them into records), every sample of every trio, ``./.`` for a trio without a row in the
     record.  FORMAT GT:AD:GQ; GQ is declared Float when a value is not integral (written in the shortest text that
     parses back to the same float32) and Integer otherwise; AD is ``rd,ad`` (``.`` for -1).  ``end``: record index ->
@@ -466,9 +499,15 @@ def write_vcf(table: SiteTable, path: str, end: Optional[Dict[int, int]] = None,
     starts = np.cumsum([0] + [len(x) for x in lines]).astype(np.int64)
     voff = write_bgzf(path, head_b, body, level)
     names = b"".join(c.encode() + b"\0" for c in t.contigs)
-    tbi = (b"TBI\x01" + struct.pack("<8i", len(t.contigs), 2, 1, 2, 0, ord("#"), 0, len(names)) + names
-           + index_refs(len(t.contigs), g_contig.astype(np.int64), pos0, rend, voff(starts[:-1]), voff(starts[1:])))
-    write_bgzf(path + ".tbi", tbi, b"", level)
+    cols = (len(t.contigs), g_contig.astype(np.int64), pos0, rend, voff(starts[:-1]), voff(starts[1:]))
+    if index == "csi":
+        aux = struct.pack("<7i", 2, 1, 2, 0, ord("#"), 0, len(names)) + names
+        write_csi(path + ".csi", *cols, min_shift=min_shift, depth=depth, aux=aux, level=level)
+    elif index == "tbi":
+        tbi = b"TBI\x01" + struct.pack("<8i", len(t.contigs), 2, 1, 2, 0, ord("#"), 0, len(names)) + names + index_refs(*cols)
+        write_bgzf(path + ".tbi", tbi, b"", level)
+    else:
+        raise ValueError("index must be 'tbi' or 'csi', not %r" % index)
 
 
 def _fill(cache: Dict, miss: str, k: int) -> str:
