@@ -524,6 +524,39 @@ int unfz_vcf_samples(UnfzCtx*, const uint8_t* buf, const UnfzVcfRec* recs, const
                      const int32_t* slot_of, int32_t n_samples, int32_t n_members, int32_t gq_float, int32_t max_digits,
                      uint8_t* gt, float* gq, int32_t* rd, int32_t* ad, uint8_t* status, uint8_t* line_bad, void* stream);
 
+/* ---- phased VCF output (csrc/vcfout.cu) --------------------------------------------------------------
+ * Input: the body text and the UnfzVcfRec lines of unfz_vcf_line_ends_host / unfz_vcf_parse (or their device calls),
+ * and the sparse edit list of the phased cells: edit_off[n_lines + 1] (CSR by line), edits sorted by (line, sample).
+ *
+ * Output per line: the text up to FORMAT verbatim; FORMAT with ":UOPS" / ":UET" appended unless present; then for every
+ * header sample s, '\t' + the cell: every subfield of the output FORMAT, the cell's own text where it has one, '.'
+ * where it dropped it, UOPS / UET = the edit's values (-1 without an edit); an absent trailing column is that of a
+ * cell "."; a phase edit writes GT "1|0" (dad) or "0|1" (mom) followed by every allele past the second behind '|'.
+ * A line without FORMAT passes through.  Every line ends in '\n' (a '\r' before it is dropped). */
+#define UNFZ_VCFOUT_COLUMNS 0x01  /* line status: more sample columns than header samples */
+#define UNFZ_VCFOUT_HAPLOID 0x02  /* line status: a phase edit on a GT without a separator */
+#define UNFZ_VCFOUT_FIELDS 0x04   /* line status: a cell with more subfields than FORMAT keys */
+typedef struct {
+    int32_t sample;       /* sample column */
+    int32_t phase;        /* 0 keep GT, 1 dad (1|0), 2 mom (0|1) */
+    int32_t uops;         /* UOPS value */
+    int32_t uet;          /* UET value */
+} UnfzVcfEdit;
+
+/* Host only: the output length of every line (int64, '\n' included) and its status (UNFZ_VCFOUT_*).  Returns the sum. */
+int64_t unfz_vcf_rewrite_size_host(const uint8_t* buf, const UnfzVcfRec* recs, int64_t n_lines, const int64_t* edit_off,
+                                   const UnfzVcfEdit* edits, int32_t n_samples, int64_t* out_len, uint8_t* line_bad);
+/* Host only: the output of every line at out_off[i] (the exclusive scan of out_len). */
+int unfz_vcf_rewrite_write_host(const uint8_t* buf, const UnfzVcfRec* recs, int64_t n_lines, const int64_t* edit_off,
+                                const UnfzVcfEdit* edits, int32_t n_samples, const int64_t* out_off, uint8_t* out);
+/* Device: unfz_vcf_rewrite_size_host, one warp per line.  buf must be 16-byte aligned and readable 16 bytes past its
+ * end. */
+int unfz_vcf_rewrite_size(UnfzCtx*, const uint8_t* buf, const UnfzVcfRec* recs, int64_t n_lines, const int64_t* edit_off,
+                          const UnfzVcfEdit* edits, int32_t n_samples, int64_t* out_len, uint8_t* line_bad, void* stream);
+/* Device: unfz_vcf_rewrite_write_host, one warp per line (out_off from unfz_exclusive_scan_i64 of out_len). */
+int unfz_vcf_rewrite_write(UnfzCtx*, const uint8_t* buf, const UnfzVcfRec* recs, int64_t n_lines, const int64_t* edit_off,
+                           const UnfzVcfEdit* edits, int32_t n_samples, const int64_t* out_off, uint8_t* out, void* stream);
+
 /* ---- BCF decoding (csrc/bcf.cu) ----------------------------------------------------------------------
  * Input: the inflated bytes of the BGZF chunks of a CSI region query (whole BCF 2.2 records back to back).
  *

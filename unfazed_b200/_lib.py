@@ -109,6 +109,10 @@ BCF_REC_DTYPE = np.dtype([("rec_off", "<i8"), ("contig", "<i4"), ("pos0", "<i4")
 BCF_SIMPLE, BCF_BAD_OVERRUN, BCF_BAD_SAMPLES, BCF_BAD_TYPE, BCF_BAD_POS, BCF_BAD = 0x01, 0x02, 0x04, 0x08, 0x10, 0x80
 BCF_CELL_BAD = 0x02
 assert BCF_REC_DTYPE.itemsize == 80
+# UnfzVcfEdit: one phased cell of the VCF writer (csrc/vcfout.cu)
+VCF_EDIT_DTYPE = np.dtype([("sample", "<i4"), ("phase", "<i4"), ("uops", "<i4"), ("uet", "<i4")])
+VCFOUT_COLUMNS, VCFOUT_HAPLOID, VCFOUT_FIELDS = 0x01, 0x02, 0x04
+assert VCF_EDIT_DTYPE.itemsize == 16
 assert SEG_DTYPE.itemsize == 32 and DNM_DTYPE.itemsize == 48 and RSUM_DTYPE.itemsize == 32
 
 # constants of include/unfazed_sm100.h
@@ -173,6 +177,10 @@ SYMBOLS = {
     "unfz_vcf_parse": (C.c_int, [_P, _P, _P, c_int64, _P, _P]),
     "unfz_vcf_samples": (C.c_int, [_P, _P, _P, _P, c_int64, _P, c_int32, c_int32, c_int32, c_int32, _P, _P, _P, _P, _P, _P,
                                    _P]),
+    "unfz_vcf_rewrite_size_host": (c_int64, [_P, _P, c_int64, _P, _P, c_int32, _P, _P]),
+    "unfz_vcf_rewrite_write_host": (C.c_int, [_P, _P, c_int64, _P, _P, c_int32, _P, _P]),
+    "unfz_vcf_rewrite_size": (C.c_int, [_P, _P, _P, c_int64, _P, _P, c_int32, _P, _P, _P]),
+    "unfz_vcf_rewrite_write": (C.c_int, [_P, _P, _P, c_int64, _P, _P, c_int32, _P, _P, _P]),
     "unfz_bcf_record_offsets": (c_int64, [_P, c_int64, c_int64, _P, _P]),
     "unfz_bcf_parse_host": (c_int64, [_P, _P, c_int64, _P, c_int32, _P]),
     "unfz_bcf_samples_host": (C.c_int, [_P, _P, _P, c_int64, _P, c_int32, _P, _P, _P, _P, _P]),

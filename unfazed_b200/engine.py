@@ -310,7 +310,8 @@ class VcfDecoder:
     up once (pinned staging), the newline pass (unfz_vcf_line_count, a scan, unfz_vcf_line_write) and the fixed-field
     parse (unfz_vcf_parse) run on the engine's stream and the 64-byte records come back for the host's selection; then
     unfz_vcf_samples decodes the member columns of the selected lines, which come back as the table's genotype arrays.
-    The floats it leaves to the host are decoded by ``vcfio.finish_cells``."""
+    The floats it leaves to the host are decoded by ``vcfio.finish_cells``.  ``rewrite`` writes the phased VCF body from
+    the same resident text and records (``vcfio.write_phased_vcf``)."""
 
     def __init__(self, engine: "Engine"):
         self.engine = engine
@@ -341,7 +342,7 @@ class VcfDecoder:
             eng._check(lib.unfz_vcf_line_count(ctx, self.dbuf.data_ptr(), n, cnt.data_ptr(), sp), "vcf_line_count")
             eng._check(lib.unfz_exclusive_scan_u32(ctx, cnt.data_ptr(), at.data_ptr(), chunks, total.data_ptr(),
                                                    work.data_ptr(), sp), "exclusive_scan_u32")
-            n_lines = int(total.item())
+            n_lines = self.n_lines = int(total.item())
             self.ends = torch.empty((max(n_lines, 1),), dtype=torch.int64, device=dev)
             eng._check(lib.unfz_vcf_line_write(ctx, self.dbuf.data_ptr(), n, at.data_ptr(), self.ends.data_ptr(), sp),
                        "vcf_line_write")
@@ -400,6 +401,67 @@ class VcfDecoder:
         res = {k: host[k][:cells].reshape(ns, m) for k in ("gt", "gq", "rd", "ad", "status")}
         res["line_bad"] = host["line_bad"][:ns]
         return res
+
+    def rewrite(self, edit_off: np.ndarray, edits: np.ndarray, n_samples: int):
+        """Every line of the text ``lines()`` left on the device, rewritten with the edit list (csrc/vcfout.cu):
+        (the output bytes, the status of every line, UNFZ_VCFOUT_*).  Only the edits go up; the line lengths are sized
+        (unfz_vcf_rewrite_size), scanned (unfz_exclusive_scan_i64) and written (unfz_vcf_rewrite_write) on the engine's
+        stream, and the output comes down in one copy.  With a bad line nothing is written: the output
+        is empty and the status says why."""
+        eng = self.engine
+        lib, ctx, dev = eng.lib, eng.ctx, eng.device
+        n = self.n_lines
+        ne = int(edits.shape[0])
+        with eng.on_stream():
+            st = torch.cuda.current_stream(dev)
+            sp = C.c_void_p(st.cuda_stream)
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
+            e[0].record(st)
+            doff = _to_device(np.ascontiguousarray(edit_off, dtype=np.int64), dev, True)
+            ded = _to_device(np.ascontiguousarray(edits, dtype=L.VCF_EDIT_DTYPE), dev, True) if ne else \
+                torch.zeros(16, dtype=torch.uint8, device=dev)
+            e[1].record(st)
+            out_len = torch.empty((max(n, 1),), dtype=torch.int64, device=dev)
+            # the status of every line, then the total output length, in one download
+            nb = (n + 7) // 8 * 8
+            stat = torch.zeros((nb + 8,), dtype=torch.uint8, device=dev)
+            out_off = torch.empty((n + 1,), dtype=torch.int64, device=dev)
+            work = torch.empty((int(lib.unfz_scan_work_bytes(max(n, 1))),), dtype=torch.uint8, device=dev)
+            eng._check(lib.unfz_vcf_rewrite_size(ctx, self.dbuf.data_ptr(), self.drecs.data_ptr(), n, doff.data_ptr(),
+                                                 ded.data_ptr(), int(n_samples), out_len.data_ptr(), stat.data_ptr(), sp),
+                       "vcf_rewrite_size")
+            if n:
+                eng._check(lib.unfz_exclusive_scan_i64(ctx, out_len.data_ptr(), out_off.data_ptr(), n, work.data_ptr(), sp),
+                           "exclusive_scan_i64")
+            else:
+                out_off.zero_()
+            stat[nb:].view(torch.int64).copy_(out_off[n:])
+            host_stat = stat.cpu().numpy()
+            e[2].record(st)
+        line_bad = host_stat[:n].copy()
+        total = int(host_stat[nb:].view(np.int64)[0])
+        self.h2d_bytes += int(edit_off.nbytes) + ne * L.VCF_EDIT_DTYPE.itemsize
+        self.d2h_bytes += nb + 8
+        if line_bad.any():
+            self._time("h2d_edits", e[0], e[1])
+            return np.zeros(0, dtype=np.uint8), line_bad
+        with eng.on_stream():
+            out = torch.empty((max(total, 1),), dtype=torch.uint8, device=dev)
+            eng._check(lib.unfz_vcf_rewrite_write(ctx, self.dbuf.data_ptr(), self.drecs.data_ptr(), n, doff.data_ptr(),
+                                                  ded.data_ptr(), int(n_samples), out_off.data_ptr(), out.data_ptr(), sp),
+                       "vcf_rewrite_write")
+            e[3].record(st)
+            # one copy into pageable memory (the driver stages it): page-locking a fresh block of the output's size costs
+            # more than the copy itself
+            host = out[:total].cpu()
+            e[4].record(st)
+        e[4].synchronize()
+        self._time("h2d_edits", e[0], e[1])
+        self._time("rewrite_size", e[1], e[2])
+        self._time("rewrite_write", e[2], e[3])
+        self._time("d2h_output", e[3], e[4])
+        self.d2h_bytes += total
+        return host.numpy(), line_bad
 
 
 class BcfDecoder:

@@ -213,7 +213,12 @@ def uet_code(evidence_types):
     return 2 if (rb and ab) else 0 if rb else 1 if ab else -1
 
 
-def write_vcf_output(in_vcf_name, read_records, include_ambiguous, verbose, outfile, evidence_min_ratio):
+def write_vcf_output(in_vcf_name, read_records, include_ambiguous, verbose, outfile, evidence_min_ratio, engine=None):
+    if os.path.isfile(in_vcf_name) and in_vcf_name.endswith((".vcf", ".vcf.gz")) and not outfile.endswith(".bcf"):
+        # an existing text VCF written as text or BGZF: natively (vcfio), no cyvcf2 needed
+        from .vcfio import write_phased_vcf
+        write_phased_vcf(in_vcf_name, read_records, include_ambiguous, verbose, outfile, evidence_min_ratio, engine)
+        return
     import numpy as np
     from cyvcf2 import VCF, Writer
     vcf = VCF(in_vcf_name)
@@ -342,6 +347,8 @@ def unfazed(args):
         phased = phase_snvs(snvs, *common) if snvs else {}
         phased.update(phased_svs)
     if output_type == "vcf":
-        write_vcf_output(args.dnms, phased, args.include_ambiguous, args.verbose, args.outfile, args.evidence_min_ratio)
+        from . import informative_site_finder
+        write_vcf_output(args.dnms, phased, args.include_ambiguous, args.verbose, args.outfile, args.evidence_min_ratio,
+                         informative_site_finder._engine)
     else:
         write_bed_output(phased, args.include_ambiguous, args.verbose, args.outfile, args.evidence_min_ratio)

@@ -10,6 +10,8 @@ code (csrc/vcf.cu), on the GPU with an engine.
   (``engine.VcfDecoder``), where only the text goes up and only the fixed fields and member columns come back.
 * ``read_dnms`` -- the DNM dicts ``unfazed.read_vars_vcf`` yields, from a plain or gzipped VCF read whole.
 * ``write_vcf`` -- a sorted ``.vcf.gz`` + ``.tbi`` from a ``SiteTable`` (tests and tools generate their inputs with it).
+* ``write_phased_vcf`` -- the phased VCF ``unfazed.write_vcf_output`` writes, from a plain or gzipped DNM VCF: the
+  edit list of the phased cells on the host, the sample columns rewritten natively (csrc/vcfout.cu).
 
 Field decoding follows cyvcf2 0.31.0's defaults (gts012=False, strict_gt=False); DESIGN §5 lists the assumptions.  A
 ``.csi`` index (``bamio.CsiIndex``, with the tabix header in its aux bytes) serves where no ``.tbi`` exists.  BCF is read
@@ -38,11 +40,11 @@ def _ptr(a: np.ndarray) -> int:
 
 
 # ------------------------------------------------------------------------------------------------
-# native decode on the host (the device decoder, engine.VcfDecoder, has the same two calls)
+# native decode on the host (the device decoder, engine.VcfDecoder, has the same calls)
 # ------------------------------------------------------------------------------------------------
 
 class HostDecoder:
-    """``lines`` and ``samples`` with the host entry points of csrc/vcf.cu."""
+    """``lines`` and ``samples`` with the host entry points of csrc/vcf.cu, ``rewrite`` with those of csrc/vcfout.cu."""
 
     def lines(self, buf: np.ndarray) -> np.ndarray:
         """Fixed fields (``_lib.VCF_REC_DTYPE``) of every '\\n'-terminated line of ``buf``."""
@@ -66,6 +68,25 @@ class HostDecoder:
                                        int(slot_of.shape[0]), int(n_members), int(bool(gq_float)), int(max_digits),
                                        *(_ptr(out[k]) for k in ("gt", "gq", "rd", "ad", "status", "line_bad")))
         return out
+
+    def rewrite(self, edit_off: np.ndarray, edits: np.ndarray, n_samples: int):
+        """Every line of ``lines()`` rewritten with the edit list (``_lib.VCF_EDIT_DTYPE``, CSR by line): (the output
+        bytes, the status of every line, ``_lib.VCFOUT_*``).  With a bad line the output is empty."""
+        lib = L.load()
+        n = int(self.recs.shape[0])
+        edit_off = np.ascontiguousarray(edit_off, dtype=np.int64)
+        edits = np.ascontiguousarray(edits, dtype=L.VCF_EDIT_DTYPE)
+        out_len = np.empty(max(n, 1), dtype=np.int64)
+        line_bad = np.zeros(max(n, 1), dtype=np.uint8)
+        args = (_ptr(self.buf), _ptr(self.recs), n, _ptr(edit_off), _ptr(edits), int(n_samples))
+        total = int(lib.unfz_vcf_rewrite_size_host(*args, _ptr(out_len), _ptr(line_bad)))
+        if line_bad[:n].any():
+            return np.zeros(0, dtype=np.uint8), line_bad[:n]
+        out_off = np.zeros(n + 1, dtype=np.int64)
+        np.cumsum(out_len[:n], out=out_off[1:])
+        out = np.empty(total, dtype=np.uint8)
+        lib.unfz_vcf_rewrite_write_host(*args, _ptr(out_off), _ptr(out))
+        return out, line_bad[:n]
 
 
 def _empty_cells(n: int, m: int) -> Dict[str, np.ndarray]:
@@ -407,6 +428,167 @@ def read_dnms(path: str):
         for s in np.flatnonzero((gt[i] == HET) | (gt[i] == HOM_ALT)).tolist():
             yield {"chrom": cols[0], "start": int(recs["pos0"][i]), "end": int(recs["rend"][i]), "kid": samples[s],
                    "vartype": vartype, "bam": ""}
+
+
+# ------------------------------------------------------------------------------------------------
+# phased VCF writer
+# ------------------------------------------------------------------------------------------------
+
+UNFAZED_LINE = ("##unfazed=%s. Phase info in pipe-separated GT field order -> 1|0 is paternal, 0|1 is maternal")
+UOPS_LINE = ('##FORMAT=<ID=UOPS,Number=1,Type=Float,Description="Count of pieces of evidence supporting the '
+             'unfazed-identified origin parent or `-1` if missing">')
+UET_LINE = ('##FORMAT=<ID=UET,Number=1,Type=Float,Description="Unfazed evidence type: `0` (readbacked), `1` '
+            '(allele-balance, for CNVs only), `2` (both), `3` (ambiguous readbacked), `4` (ambiguous allele-balance), '
+            '`5` (ambiguous both), `6` (auto-phased sex-chromosome variant in male), or `-1` (missing)">')
+PASS_LINE = '##FILTER=<ID=PASS,Description="All filters passed">'
+_ID_RE = re.compile(rb"^##(FORMAT|FILTER)=<ID=([^,>]+)[,>]")
+
+
+def phased_header(head: bytes, version: str) -> bytes:
+    """The header of the phased VCF: the input's lines verbatim (a trailing '\\r' dropped), the PASS filter after
+    ``##fileformat`` when the input declares none (htslib's header parser adds it), and before ``#CHROM`` the
+    ``##unfazed=`` line and the UOPS / UET FORMAT lines not already declared."""
+    lines = [x[:-1] if x.endswith(b"\r") else x for x in head.split(b"\n")]
+    if lines and lines[-1] == b"":
+        lines.pop()
+    ids = {(m.group(1), m.group(2)) for m in map(_ID_RE.match, lines) if m}
+    out = []
+    for x in lines:
+        if x.startswith(b"#CHROM"):
+            out.append((UNFAZED_LINE % version).encode())
+            for key, line in ((b"UOPS", UOPS_LINE), (b"UET", UET_LINE)):
+                if (b"FORMAT", key) not in ids:
+                    out.append(line.encode())
+        out.append(x)
+    if (b"FILTER", b"PASS") not in ids:
+        at = 1 if out and out[0].startswith(b"##fileformat") else 0
+        out.insert(at, PASS_LINE.encode())
+    return b"\n".join(out) + b"\n"
+
+
+def _svtype(buf: np.ndarray, rec) -> str:
+    """INFO SVTYPE of a line as ``read_dnms`` takes it (the first SVTYPE key; "POINT" when absent or empty)."""
+    from .utils import SNV_TYPES
+    o = int(rec["line_off"])
+    cols = buf[o: o + int(rec["line_len"])].tobytes().decode().split("\t", 8)
+    for kv in cols[7].split(";"):
+        k, _, v = kv.partition("=")
+        if k == "SVTYPE":
+            return v or SNV_TYPES[0]
+    return SNV_TYPES[0]
+
+
+def phase_edits(buf: np.ndarray, recs: np.ndarray, samples: Sequence[str], read_records, include_ambiguous, verbose,
+                evidence_min_ratio, dec=None):
+    """The edit list of the phased cells (``_lib.VCF_EDIT_DTYPE`` sorted by (line, sample), and its CSR offsets by
+    line), in O(#records): the candidate lines are those whose (CHROM, pos0, end) is some record's region; their
+    genotypes are decoded for the records' kids only, and every HET / HOM_ALT cell whose key
+    ``{CHROM}_{pos0}_{end}_{sample}_{SVTYPE or POINT}`` is a record gets the record's call."""
+    from .unfazed import summarize_record, uet_code
+    n = int(recs.shape[0])
+    dec = dec or HostDecoder()
+    regions = {(str(r["region"]["chrom"]), int(r["region"]["start"]), int(r["region"]["end"]))
+               for r in read_records.values()}
+    sidx = {s: i for i, s in enumerate(samples)}
+    kids = sorted({sidx[r["kid"]] for r in read_records.values() if r.get("kid") in sidx})
+    rows = []
+    if regions and kids and n:
+        pe = np.array(sorted({(p, e) for _c, p, e in regions}), dtype=np.int64)
+        key_l = recs["pos0"].astype(np.int64) * (1 << 32) + recs["rend"].astype(np.int64)
+        cand = np.flatnonzero(np.isin(key_l, pe[:, 0] * (1 << 32) + pe[:, 1]))
+        chrom = {}
+        keep = []
+        for i in cand.tolist():
+            o = int(recs["line_off"][i])
+            c = buf[o: o + int(recs["chrom_len"][i])].tobytes().decode()
+            if (c, int(recs["pos0"][i]), int(recs["rend"][i])) in regions:
+                chrom[i] = c
+                keep.append(i)
+        if keep:
+            sel = np.array(keep, dtype=np.int64)
+            slot_of = np.full(len(samples), -1, dtype=np.int32)
+            slot_of[kids] = np.arange(len(kids), dtype=np.int32)
+            gt = dec.samples(sel, slot_of, len(kids), True)["gt"]
+            for li, i in enumerate(keep):
+                carriers = np.flatnonzero((gt[li] == HET) | (gt[li] == HOM_ALT))
+                if not carriers.shape[0]:
+                    continue
+                head = "%s_%d_%d_" % (chrom[i], int(recs["pos0"][i]), int(recs["rend"][i]))
+                tail = "_" + _svtype(buf, recs[i])
+                for m in carriers.tolist():
+                    key = head + samples[kids[m]] + tail
+                    rec = read_records.get(key)
+                    if rec is None:
+                        continue
+                    s = summarize_record(rec, include_ambiguous, verbose, evidence_min_ratio)
+                    if s is None:
+                        continue
+                    phase = 1 if s["origin_parent"] == rec["dad"] else 2 if s["origin_parent"] == rec["mom"] else 0
+                    rows.append((i, kids[m], phase, int(s["evidence_count"]), uet_code(s["evidence_types"])))
+    rows.sort()
+    edits = np.zeros(len(rows), dtype=L.VCF_EDIT_DTYPE)
+    line = np.array([r[0] for r in rows], dtype=np.int64)
+    for k, name in enumerate(("sample", "phase", "uops", "uet")):
+        edits[name] = [r[k + 1] for r in rows]
+    edit_off = np.searchsorted(line, np.arange(n + 1), side="left").astype(np.int64)
+    return edit_off, edits
+
+
+def write_phased_vcf(in_path: str, read_records, include_ambiguous, verbose, outfile: str, evidence_min_ratio,
+                     engine=None) -> None:
+    """The phased VCF of ``unfazed.write_vcf_output`` without cyvcf2: every line of the plain or gzipped DNM VCF
+    ``in_path`` with GT 1|0 (paternal) / 0|1 (maternal) and UOPS / UET for the phased carriers, UOPS = UET = -1 in
+    every other cell.  The edit list is built on the host (``phase_edits``); the sample columns are rewritten in
+    native code (csrc/vcfout.cu), on ``engine``'s GPU when given.  Bytes the contract does not touch are copied
+    verbatim (DESIGN §5).  ``outfile``: ``/dev/stdout`` or a plain file, BGZF when it ends in ``.gz``."""
+    from . import __version__
+    opener = gzip.open if in_path.endswith((".gz", ".bgz")) else open
+    with opener(in_path, "rb") as f:
+        data = bytearray().join(iter(lambda: f.read(1 << 24), b""))      # writable: the device upload wraps it
+    if data and not data.endswith(b"\n"):
+        data += b"\n"
+    got = _parse_header(data, in_path)
+    if got is None:
+        raise ValueError("%s: no #CHROM header line" % in_path)
+    samples, _types, _chrom, body, _ = got
+    buf = np.frombuffer(data, dtype=np.uint8)[body:]
+    head_lines = data[:body].count(b"\n")
+    where = lambda off: "%s, line %d" % (in_path, head_lines + 1 + int(np.searchsorted(ends, off, side="left")))
+    dec = engine.vcf_decoder() if engine is not None else HostDecoder()
+    recs = _lines(dec, buf, lambda off: "%s, line at byte %d" % (in_path, body + off))
+    ends = (recs["line_off"] + recs["line_len"]).astype(np.int64)
+    edit_off, edits = phase_edits(buf, recs, samples, read_records, include_ambiguous, verbose, evidence_min_ratio, dec)
+    out, line_bad = dec.rewrite(edit_off, edits, len(samples))
+    bad = np.flatnonzero(line_bad)
+    if bad.shape[0]:
+        i = int(bad[0])
+        off = int(recs["line_off"][i])
+        st = int(line_bad[i])
+        if st & L.VCFOUT_COLUMNS:
+            raise ValueError("%s: more sample columns than header samples" % where(off))
+        if st & L.VCFOUT_FIELDS:
+            raise ValueError("%s: a sample with more subfields than FORMAT keys" % where(off))
+        cols = buf[off: off + int(recs["line_len"][i])].tobytes().decode("ascii", "replace").split("\t")
+        gi = cols[8].split(":").index("GT")
+        e = edits[int(edit_off[i]): int(edit_off[i + 1])]
+        for s in e["sample"][e["phase"] != 0].tolist():
+            sub = (cols[9 + s] if 9 + s < len(cols) else ".").split(":")
+            gt = sub[gi] if gi < len(sub) else "."
+            if "/" not in gt and "|" not in gt:
+                raise ValueError("%s: the haploid GT %r of sample %s cannot be phased" % (where(off), gt, samples[s]))
+    head = phased_header(data[:body], __version__)
+    if outfile == "/dev/stdout":
+        import sys
+        sys.stdout.flush()
+        sys.stdout.buffer.write(head)
+        sys.stdout.buffer.write(memoryview(out))
+        sys.stdout.buffer.flush()
+    elif outfile.endswith(".gz"):
+        write_bgzf(outfile, head, memoryview(out))
+    else:
+        with open(outfile, "wb") as f:
+            f.write(head)
+            f.write(memoryview(out))
 
 
 # ------------------------------------------------------------------------------------------------
