@@ -614,6 +614,44 @@ int unfz_bcf_samples(UnfzCtx*, const uint8_t* buf, const UnfzBcfRec* recs, const
                      const int32_t* member_sample, int32_t n_members, uint8_t* gt, float* gq, int32_t* rd, int32_t* ad,
                      uint8_t* status, void* stream);
 
+/* ---- phased VCF output from BCF (csrc/bcfout.cu) ----------------------------------------------------------
+ * Input: the inflated records and their UnfzBcfRec (unfz_bcf_parse_host / unfz_bcf_parse, no record with UNFZ_BCF_BAD);
+ * the string and contig dictionaries as names (names + off[id] .. off[id + 1], empty for an unused id); keys: 3 host
+ * int32, the string-dictionary ids of GT, UOPS and UET (-1: not in the header); and the sparse edit list of the phased
+ * cells, edit_off[n_recs + 1] (CSR by record), edits sorted by (record, sample).
+ *
+ * Output per record, the VCF line htslib's vcf_format prints: CHROM, POS, ID, REF, ALT, QUAL, FILTER, INFO, and with
+ * samples FORMAT (":UOPS" / ":UET" appended unless present; "." without FORMAT fields) and one cell per sample.  In a
+ * cell UOPS / UET are the edit's values (-1 without an edit); a phase edit writes GT "1|0" (dad) or "0|1" (mom)
+ * followed by every allele past the second behind '|'.  Floats are printed as "%g".  Every record ends in '\n'. */
+#define UNFZ_BCFOUT_HAPLOID 0x01     /* record status: a phase edit on a GT of fewer than two alleles */
+#define UNFZ_BCFOUT_FLOAT_HOST 0x02  /* record status: a float the device does not print (the host entry points do) */
+#define UNFZ_BCFOUT_BAD 0x04         /* record status: an id outside a dictionary, or a value of a type it cannot have */
+
+/* Host only: the output length of every record (int64, '\n' included) and its status (UNFZ_BCFOUT_*).  Returns the
+ * sum.  Floats off the exact path are printed with snprintf("%g"). */
+int64_t unfz_bcf_format_size_host(const uint8_t* buf, const UnfzBcfRec* recs, int64_t n_recs, const uint8_t* str_names,
+                                  const int64_t* str_off, int32_t n_str, const uint8_t* ctg_names, const int64_t* ctg_off,
+                                  int32_t n_ctg, const int32_t* keys, const int64_t* edit_off, const UnfzVcfEdit* edits,
+                                  int32_t n_samples, int64_t* out_len, uint8_t* status);
+/* Host only: the output of every record at out_off[i] (the exclusive scan of out_len). */
+int unfz_bcf_format_write_host(const uint8_t* buf, const UnfzBcfRec* recs, int64_t n_recs, const uint8_t* str_names,
+                               const int64_t* str_off, int32_t n_str, const uint8_t* ctg_names, const int64_t* ctg_off,
+                               int32_t n_ctg, const int32_t* keys, const int64_t* edit_off, const UnfzVcfEdit* edits,
+                               int32_t n_samples, const int64_t* out_off, uint8_t* out);
+/* Device: unfz_bcf_format_size_host, one warp per record.  The length of a record with UNFZ_BCFOUT_FLOAT_HOST lacks its
+ * floats: the caller takes it from the host entry point. */
+int unfz_bcf_format_size(UnfzCtx*, const uint8_t* buf, const UnfzBcfRec* recs, int64_t n_recs, const uint8_t* str_names,
+                         const int64_t* str_off, int32_t n_str, const uint8_t* ctg_names, const int64_t* ctg_off,
+                         int32_t n_ctg, const int32_t* keys, const int64_t* edit_off, const UnfzVcfEdit* edits,
+                         int32_t n_samples, int64_t* out_len, uint8_t* status, void* stream);
+/* Device: unfz_bcf_format_write_host, one warp per record (out_off from unfz_exclusive_scan_i64 of out_len).  Records
+ * whose status (of the size step) has UNFZ_BCFOUT_FLOAT_HOST are skipped: the caller copies in the host's text. */
+int unfz_bcf_format_write(UnfzCtx*, const uint8_t* buf, const UnfzBcfRec* recs, int64_t n_recs, const uint8_t* str_names,
+                          const int64_t* str_off, int32_t n_str, const uint8_t* ctg_names, const int64_t* ctg_off,
+                          int32_t n_ctg, const int32_t* keys, const int64_t* edit_off, const UnfzVcfEdit* edits,
+                          int32_t n_samples, const uint8_t* status, const int64_t* out_off, uint8_t* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

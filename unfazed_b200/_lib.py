@@ -112,6 +112,8 @@ assert BCF_REC_DTYPE.itemsize == 80
 # UnfzVcfEdit: one phased cell of the VCF writer (csrc/vcfout.cu)
 VCF_EDIT_DTYPE = np.dtype([("sample", "<i4"), ("phase", "<i4"), ("uops", "<i4"), ("uet", "<i4")])
 VCFOUT_COLUMNS, VCFOUT_HAPLOID, VCFOUT_FIELDS = 0x01, 0x02, 0x04
+# record status of the BCF -> VCF formatter (csrc/bcfout.cu)
+BCFOUT_HAPLOID, BCFOUT_FLOAT_HOST, BCFOUT_BAD = 0x01, 0x02, 0x04
 assert VCF_EDIT_DTYPE.itemsize == 16
 assert SEG_DTYPE.itemsize == 32 and DNM_DTYPE.itemsize == 48 and RSUM_DTYPE.itemsize == 32
 
@@ -186,6 +188,12 @@ SYMBOLS = {
     "unfz_bcf_samples_host": (C.c_int, [_P, _P, _P, c_int64, _P, c_int32, _P, _P, _P, _P, _P]),
     "unfz_bcf_parse": (C.c_int, [_P, _P, _P, c_int64, _P, c_int32, _P, _P]),
     "unfz_bcf_samples": (C.c_int, [_P, _P, _P, _P, c_int64, _P, c_int32, _P, _P, _P, _P, _P, _P]),
+    "unfz_bcf_format_size_host": (c_int64, [_P, _P, c_int64, _P, _P, c_int32, _P, _P, c_int32, _P, _P, _P, c_int32, _P, _P]),
+    "unfz_bcf_format_write_host": (C.c_int, [_P, _P, c_int64, _P, _P, c_int32, _P, _P, c_int32, _P, _P, _P, c_int32, _P, _P]),
+    "unfz_bcf_format_size": (C.c_int, [_P, _P, _P, c_int64, _P, _P, c_int32, _P, _P, c_int32, _P, _P, _P, c_int32, _P, _P,
+                                       _P]),
+    "unfz_bcf_format_write": (C.c_int, [_P, _P, _P, c_int64, _P, _P, c_int32, _P, _P, c_int32, _P, _P, _P, c_int32, _P, _P,
+                                        _P, _P]),
 }
 
 _lib = None

@@ -13,6 +13,8 @@ decoding in native code (csrc/bcf.cu), on the GPU with an engine.
   ``.bcf`` read whole.
 * ``write_bcf`` -- a sorted ``.bcf`` + ``.csi`` from a ``SiteTable`` with ``vcfio.write_vcf``'s options (tests and tools
   generate their inputs with it).
+* ``write_phased_vcf`` -- the phased VCF ``unfazed.write_vcf_output`` writes, from a BCF DNM list: the edit list on the
+  host (the core of the text writer, ``vcfio.match_edits``), every record printed as VCF text natively (csrc/bcfout.cu).
 
 The format rules this module assumes (BCF 2.2, VCF specification §6) are listed in DESIGN §5.
 """
@@ -31,7 +33,7 @@ from . import _lib as L
 from .bamio import BgzfReader, CsiIndex, write_bgzf, write_csi
 from .packers import build_site_table
 from .schema import GT_UNKNOWN, HET, HOM_ALT, HOM_REF, SiteTable
-from .vcfio import _records, member_columns, query_plan, select_records
+from .vcfio import _records, match_edits, member_columns, phased_header, query_plan, select_records, write_output
 
 MAGIC = b"BCF\x02\x02"
 FORMAT_KEYS = ("GT", "GQ", "AD", "RO", "AO")       # the order of UnfzBcfRec.fmt_off
@@ -89,6 +91,36 @@ class HostDecoder:
             L.load().unfz_bcf_samples_host(_ptr(self.buf), _ptr(self.recs), _ptr(sel), n, _ptr(ms), m,
                                            *(_ptr(out[k]) for k in ("gt", "gq", "rd", "ad", "status")))
         return out
+
+    def format(self, edit_off: np.ndarray, edits: np.ndarray, n_samples: int, names, fkeys: np.ndarray):
+        """Every record of ``records()`` printed as the phased VCF body (csrc/bcfout.cu): (the output bytes, the status
+        of every record, ``_lib.BCFOUT_*``).  With a haploid phase edit or a malformed record the output is empty."""
+        return format_host(self.buf, self.recs, edit_off, edits, n_samples, names, fkeys)[:2]
+
+
+def format_host(buf, recs, edit_off, edits, n_samples: int, names, fkeys):
+    """The host entry points of csrc/bcfout.cu over ``recs``: (output bytes, status of every record, output length of
+    every record).  ``names``: (string names, offsets, contig names, offsets) of ``dictionaries``; ``fkeys``: the
+    string-dictionary ids of GT, UOPS and UET."""
+    lib = L.load()
+    n = int(recs.shape[0])
+    recs = np.ascontiguousarray(recs, dtype=L.BCF_REC_DTYPE)
+    edit_off = np.ascontiguousarray(edit_off, dtype=np.int64)
+    edits = np.ascontiguousarray(edits, dtype=L.VCF_EDIT_DTYPE)
+    fkeys = np.ascontiguousarray(fkeys, dtype=np.int32)
+    sn, so, cn, co = names
+    args = (_ptr(buf), _ptr(recs), n, _ptr(sn), _ptr(so), int(so.shape[0]) - 1, _ptr(cn), _ptr(co), int(co.shape[0]) - 1,
+            _ptr(fkeys), _ptr(edit_off), _ptr(edits), int(n_samples))
+    out_len = np.zeros(max(n, 1), dtype=np.int64)
+    status = np.zeros(max(n, 1), dtype=np.uint8)
+    total = int(lib.unfz_bcf_format_size_host(*args, _ptr(out_len), _ptr(status)))
+    if (status[:n] & (L.BCFOUT_HAPLOID | L.BCFOUT_BAD)).any():
+        return np.zeros(0, dtype=np.uint8), status[:n], out_len[:n]
+    out_off = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(out_len[:n], out=out_off[1:])
+    out = np.empty(total, dtype=np.uint8)
+    lib.unfz_bcf_format_write_host(*args, _ptr(out_off), _ptr(out))
+    return out, status[:n], out_len[:n]
 
 
 def _checked_records(dec, buf, offs, keys, n_samples, where) -> np.ndarray:
@@ -354,17 +386,15 @@ def _info_string(buf: np.ndarray, rec, key: int) -> Optional[str]:
     return None
 
 
-def read_dnms(path: str):
-    """The DNMs of a BGZF-compressed or uncompressed BCF, read whole without an index: for every record and every
-    sample whose genotype is HET or HOM_ALT, in header order, {chrom, start, end, kid, vartype, bam: ""} with start
-    pos0, end pos0 + rlen and vartype INFO SVTYPE or "POINT" -- what ``vcfio.read_dnms`` yields for the same records as
-    text."""
-    from .utils import SNV_TYPES
+def _read_whole(path: str):
+    """A BGZF-compressed or uncompressed BCF read whole: (header text, samples, string dictionary, contig names, the
+    record bytes (writable), their offsets, and a function that names a byte of them for error messages)."""
     with open(path, "rb") as f:
-        data = f.read()
-    if data[:2] == b"\x1f\x8b":
+        bgzf = f.read(2) == b"\x1f\x8b"
+    if bgzf:
         BgzfReader(path)                             # the EOF block check
-        data = gzip.decompress(data)
+    with (gzip.open if bgzf else open)(path, "rb") as f:
+        data = bytearray().join(iter(lambda: f.read(1 << 24), b""))
     got = _read_head(data, path)
     if got is None:
         raise ValueError("%s: truncated BCF header" % path)
@@ -375,6 +405,29 @@ def read_dnms(path: str):
     offs, stop = record_offsets(buf)
     if stop < 0 or stop != buf.shape[0]:
         raise ValueError("%s: malformed or truncated BCF record" % where(stop if stop >= 0 else -1 - stop))
+    return text, samples, strs, contigs, buf, offs, where
+
+
+def is_bcf(path: str) -> bool:
+    """``path`` holds BCF 2.2, uncompressed or BGZF-compressed (by its magic)."""
+    with open(path, "rb") as f:
+        head = f.read(5)
+    if head[:2] == b"\x1f\x8b":
+        try:
+            with gzip.open(path, "rb") as g:
+                head = g.read(5)
+        except (OSError, EOFError):
+            return False
+    return head == MAGIC
+
+
+def read_dnms(path: str):
+    """The DNMs of a BGZF-compressed or uncompressed BCF, read whole without an index: for every record and every
+    sample whose genotype is HET or HOM_ALT, in header order, {chrom, start, end, kid, vartype, bam: ""} with start
+    pos0, end pos0 + rlen and vartype INFO SVTYPE or "POINT" -- what ``vcfio.read_dnms`` yields for the same records as
+    text."""
+    from .utils import SNV_TYPES
+    _text, samples, strs, contigs, buf, offs, where = _read_whole(path)
     dec = HostDecoder()
     keys = np.array([strs.get(k, -1) for k in FORMAT_KEYS], dtype=np.int32)
     recs = _checked_records(dec, buf, offs, keys, len(samples), where)
@@ -394,6 +447,89 @@ def read_dnms(path: str):
         for s in carriers:
             yield {"chrom": contigs[cid], "start": int(recs["pos0"][i]), "end": int(recs["rend"][i]),
                    "kid": samples[s], "vartype": vartype, "bam": ""}
+
+
+# ------------------------------------------------------------------------------------------------
+# phased VCF writer
+# ------------------------------------------------------------------------------------------------
+
+_IDX = re.compile(r",IDX=[0-9]+(?=[,>])")
+
+
+def vcf_header(text: str) -> str:
+    """The header text of a BCF as VCF: ``IDX=`` dropped from the dictionary lines (htslib writes it to BCF only)."""
+    return "\n".join(_IDX.sub("", x) if _HREC.match(x) else x for x in text.split("\n"))
+
+
+def dictionaries(strs: Dict[str, int], contigs: Sequence[str]):
+    """The string dictionary and the contig dictionary as names for csrc/bcfout.cu: (string names, int64 offsets,
+    contig names, int64 offsets); an unused index has an empty name."""
+    by_id = [""] * (max(strs.values()) + 1 if strs else 0)
+    for k, i in strs.items():
+        by_id[i] = k
+    out = []
+    for names in (by_id, list(contigs)):
+        b = [x.encode() for x in names]
+        off = np.zeros(len(b) + 1, dtype=np.int64)
+        np.cumsum([len(x) for x in b], out=off[1:])
+        out += [np.frombuffer(b"".join(b) + b"\0", dtype=np.uint8), off]
+    return tuple(out)
+
+
+def phase_edits(buf: np.ndarray, recs: np.ndarray, samples: Sequence[str], strs: Dict[str, int], contigs: Sequence[str],
+                read_records, include_ambiguous, verbose, evidence_min_ratio, dec=None):
+    """``vcfio.match_edits`` of the records of a BCF DNM list: CHROM from the contig dictionary, SVTYPE from INFO, the
+    kids' genotypes from the decoder's ``samples``."""
+    from .utils import SNV_TYPES
+    dec = dec or HostDecoder()
+    sv_key = strs.get("SVTYPE", -1)
+
+    def chrom_of(i):
+        cid = int(recs["contig"][i])
+        return contigs[cid] if 0 <= cid < len(contigs) else None
+
+    def svtype_of(i):
+        return (_info_string(buf, recs[i], sv_key) if sv_key >= 0 else None) or SNV_TYPES[0]
+    return match_edits(recs["pos0"], recs["rend"], chrom_of, svtype_of,
+                       lambda sel, kids: dec.samples(sel, np.asarray(kids, dtype=np.int32))["gt"], samples, read_records,
+                       include_ambiguous, verbose, evidence_min_ratio)
+
+
+def write_phased_vcf(in_path: str, read_records, include_ambiguous, verbose, outfile: str, evidence_min_ratio,
+                     engine=None) -> None:
+    """The phased VCF of ``unfazed.write_vcf_output`` from a BCF 2.2 DNM list (BGZF or uncompressed) without cyvcf2:
+    every record printed as htslib's vcf_format prints it, with GT 1|0 (paternal) / 0|1 (maternal) and UOPS / UET for
+    the phased carriers, UOPS = UET = -1 in every other cell.  The edit list is built on the host (``phase_edits``); the
+    records are printed in native code (csrc/bcfout.cu), on ``engine``'s GPU when given.  The header is the BCF's with
+    ``IDX=`` dropped, plus the lines ``vcfio.phased_header`` adds.  ``outfile``: ``/dev/stdout`` or a plain file, BGZF
+    when it ends in ``.gz``."""
+    from . import __version__
+    text, samples, strs, contigs, buf, offs, where = _read_whole(in_path)
+    dec = engine.bcf_decoder() if engine is not None else HostDecoder()
+    keys = np.array([strs.get(k, -1) for k in FORMAT_KEYS], dtype=np.int32)
+    recs = _checked_records(dec, buf, offs, keys, len(samples), where)
+    edit_off, edits = phase_edits(buf, recs, samples, strs, contigs, read_records, include_ambiguous, verbose,
+                                  evidence_min_ratio, dec)
+    names = dictionaries(strs, contigs)
+    fkeys = np.array([strs.get(k, -1) for k in ("GT", "UOPS", "UET")], dtype=np.int32)
+    out, status = dec.format(edit_off, edits, len(samples), names, fkeys)
+    bad = np.flatnonzero(status & (L.BCFOUT_HAPLOID | L.BCFOUT_BAD))
+    if bad.shape[0]:
+        i = int(bad[0])
+        off = int(recs["rec_off"][i])
+        if status[i] & L.BCFOUT_BAD:
+            raise ValueError("%s: malformed BCF record (an id outside the header's dictionaries, or a value of a type it "
+                             "cannot have)" % where(off))
+        # the record printed without edits names the GT
+        line, _, _ = format_host(buf, recs[i:i + 1], np.zeros(2, dtype=np.int64), edits[:0], len(samples), names, fkeys)
+        cols = line.tobytes().decode("utf-8", "replace").rstrip("\n").split("\t")
+        gi = cols[8].split(":").index("GT")
+        e = edits[int(edit_off[i]): int(edit_off[i + 1])]
+        for s in e["sample"][e["phase"] != 0].tolist():
+            gt = cols[9 + s].split(":")[gi]
+            if "/" not in gt and "|" not in gt:
+                raise ValueError("%s: the haploid GT %r of sample %s cannot be phased" % (where(off), gt, samples[s]))
+    write_output(outfile, phased_header(vcf_header(text).encode(), __version__), out)
 
 
 # ------------------------------------------------------------------------------------------------

@@ -16,6 +16,7 @@ import contextlib
 import ctypes as C
 import collections
 import os
+import time
 from dataclasses import dataclass, field
 from typing import Dict, List, Optional
 
@@ -488,6 +489,7 @@ class BcfDecoder:
             st = torch.cuda.current_stream(dev)
             e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
             e[0].record(st)
+            self.buf = buf
             self.dbuf = _to_device(np.ascontiguousarray(buf), dev, True) if buf.shape[0] else \
                 torch.zeros(16, dtype=torch.uint8, device=dev)
             doffs = _to_device(np.ascontiguousarray(offs, dtype=np.int64), dev, True) if n else \
@@ -506,6 +508,7 @@ class BcfDecoder:
         self._time("d2h_records", e[2], e[3])
         self.h2d_bytes += int(buf.nbytes + offs.nbytes)
         self.d2h_bytes += int(recs.nbytes)
+        self.recs = recs
         return recs
 
     def samples(self, sel: np.ndarray, member_sample: np.ndarray) -> Dict[str, np.ndarray]:
@@ -540,6 +543,98 @@ class BcfDecoder:
         self.h2d_bytes += int(sel.nbytes + member_sample.nbytes)
         self.d2h_bytes += cells * 14
         return {k: host[k][:cells].reshape(ns, m) for k in ("gt", "gq", "rd", "ad", "status")}
+
+    def format(self, edit_off: np.ndarray, edits: np.ndarray, n_samples: int, names, fkeys: np.ndarray):
+        """The records ``records()`` left on the device printed as the phased VCF body (csrc/bcfout.cu): (the output
+        bytes, the status of every record, UNFZ_BCFOUT_*), as ``bcfio.HostDecoder.format``.  Only the edits and the
+        dictionaries go up; the record lengths are sized (unfz_bcf_format_size), scanned (unfz_exclusive_scan_i64) and
+        written (unfz_bcf_format_write) on the engine's stream, the statuses and the total come down in one copy and
+        the output in another.  A record with a float off the device's exact path is printed by the host entry points
+        (``bcfio.format_host``): its length goes up before a second scan, and its text is copied into its slot.  With
+        a haploid phase edit or a malformed record nothing is written: the output is empty and the status says why."""
+        from .bcfio import format_host
+        eng = self.engine
+        lib, ctx, dev = eng.lib, eng.ctx, eng.device
+        n = int(self.recs.shape[0])
+        ne = int(edits.shape[0])
+        fkeys = np.ascontiguousarray(fkeys, dtype=np.int32)
+
+        def up(a, dtype):
+            return _to_device(np.ascontiguousarray(a, dtype=dtype), dev, True) if a.shape[0] else \
+                torch.zeros(16, dtype=torch.uint8, device=dev)
+        with eng.on_stream():
+            st = torch.cuda.current_stream(dev)
+            sp = C.c_void_p(st.cuda_stream)
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
+            e[0].record(st)
+            doff = up(edit_off, np.int64)
+            ded = up(edits, L.VCF_EDIT_DTYPE)
+            dnames = [up(a, a.dtype) for a in names]
+            e[1].record(st)
+            out_len = torch.empty((max(n, 1),), dtype=torch.int64, device=dev)
+            # the status of every record, then the total output length, in one download
+            nb = (n + 7) // 8 * 8
+            stat = torch.zeros((nb + 8,), dtype=torch.uint8, device=dev)
+            out_off = torch.zeros((n + 1,), dtype=torch.int64, device=dev)
+            work = torch.empty((int(lib.unfz_scan_work_bytes(max(n, 1))),), dtype=torch.uint8, device=dev)
+            args = (self.dbuf.data_ptr(), self.drecs.data_ptr(), n, dnames[0].data_ptr(), dnames[1].data_ptr(),
+                    int(names[1].shape[0]) - 1, dnames[2].data_ptr(), dnames[3].data_ptr(), int(names[3].shape[0]) - 1,
+                    fkeys.ctypes.data, doff.data_ptr(), ded.data_ptr(), int(n_samples))
+            eng._check(lib.unfz_bcf_format_size(ctx, *args, out_len.data_ptr(), stat.data_ptr(), sp), "bcf_format_size")
+            if n:
+                eng._check(lib.unfz_exclusive_scan_i64(ctx, out_len.data_ptr(), out_off.data_ptr(), n, work.data_ptr(), sp),
+                           "exclusive_scan_i64")
+            stat[nb:].view(torch.int64).copy_(out_off[n:])
+            host_stat = stat.cpu().numpy()
+            e[2].record(st)
+        status = host_stat[:n].copy()
+        total = int(host_stat[nb:].view(np.int64)[0])
+        self.h2d_bytes += int(edit_off.nbytes) + ne * L.VCF_EDIT_DTYPE.itemsize + sum(int(a.nbytes) for a in names)
+        self.d2h_bytes += nb + 8
+        if (status & (L.BCFOUT_HAPLOID | L.BCFOUT_BAD)).any():
+            self._time("h2d_edits", e[0], e[1])
+            return np.zeros(0, dtype=np.uint8), status
+        host = np.flatnonzero(status & L.BCFOUT_FLOAT_HOST)
+        if host.shape[0]:
+            # the host prints these records; their lengths replace the device's before the offsets are scanned again
+            t0 = time.perf_counter()
+            cnt = edit_off[host + 1] - edit_off[host]
+            sub_off = np.zeros(host.shape[0] + 1, dtype=np.int64)
+            np.cumsum(cnt, out=sub_off[1:])
+            sub_edits = edits[np.repeat(edit_off[host] - sub_off[:-1], cnt) + np.arange(int(sub_off[-1]))]
+            text, _st, lens = format_host(self.buf, self.recs[host], sub_off, sub_edits, n_samples, names, fkeys)
+            self.timings_ms["format_host"] = self.timings_ms.get("format_host", 0.0) + 1e3 * (time.perf_counter() - t0)
+            with eng.on_stream():
+                didx = _to_device(host.astype(np.int64), dev, True)
+                out_len[didx] = _to_device(np.ascontiguousarray(lens), dev, True)
+                eng._check(lib.unfz_exclusive_scan_i64(ctx, out_len.data_ptr(), out_off.data_ptr(), n, work.data_ptr(), sp),
+                           "exclusive_scan_i64")
+                total = int(out_off[n:].cpu()[0])
+                slot = out_off[didx].cpu().numpy()
+            self.h2d_bytes += 16 * int(host.shape[0])
+            self.d2h_bytes += 8 + 8 * int(host.shape[0])
+        with eng.on_stream():
+            out = torch.empty((max(total, 1),), dtype=torch.uint8, device=dev)
+            ew = torch.cuda.Event(enable_timing=True)
+            ew.record(st)
+            eng._check(lib.unfz_bcf_format_write(ctx, *args, stat.data_ptr(), out_off.data_ptr(), out.data_ptr(), sp),
+                       "bcf_format_write")
+            e[3].record(st)
+            res = out[:total].cpu()
+            e[4].record(st)
+        e[4].synchronize()
+        self._time("h2d_edits", e[0], e[1])
+        self._time("format_size", e[1], e[2])
+        self._time("format_write", ew, e[3])
+        self._time("d2h_output", e[3], e[4])
+        self.d2h_bytes += total
+        res = res.numpy()
+        if host.shape[0]:
+            src = np.zeros(host.shape[0] + 1, dtype=np.int64)
+            np.cumsum(lens, out=src[1:])
+            for k in range(host.shape[0]):
+                res[int(slot[k]): int(slot[k]) + int(lens[k])] = text[int(src[k]): int(src[k + 1])]
+        return res, status
 
 
 def _to_device(a: np.ndarray, device, pin: bool, pad: int = 0) -> torch.Tensor:

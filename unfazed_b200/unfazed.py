@@ -219,6 +219,13 @@ def write_vcf_output(in_vcf_name, read_records, include_ambiguous, verbose, outf
         from .vcfio import write_phased_vcf
         write_phased_vcf(in_vcf_name, read_records, include_ambiguous, verbose, outfile, evidence_min_ratio, engine)
         return
+    if os.path.isfile(in_vcf_name) and in_vcf_name.endswith(".bcf") and not outfile.endswith(".bcf"):
+        from . import bcfio
+        if bcfio.is_bcf(in_vcf_name):
+            # an existing BCF 2.2 written as text or BGZF: natively (bcfio), no cyvcf2 needed
+            bcfio.write_phased_vcf(in_vcf_name, read_records, include_ambiguous, verbose, outfile, evidence_min_ratio,
+                                   engine)
+            return
     import numpy as np
     from cyvcf2 import VCF, Writer
     vcf = VCF(in_vcf_name)

@@ -478,15 +478,17 @@ def _svtype(buf: np.ndarray, rec) -> str:
     return SNV_TYPES[0]
 
 
-def phase_edits(buf: np.ndarray, recs: np.ndarray, samples: Sequence[str], read_records, include_ambiguous, verbose,
-                evidence_min_ratio, dec=None):
-    """The edit list of the phased cells (``_lib.VCF_EDIT_DTYPE`` sorted by (line, sample), and its CSR offsets by
-    line), in O(#records): the candidate lines are those whose (CHROM, pos0, end) is some record's region; their
-    genotypes are decoded for the records' kids only, and every HET / HOM_ALT cell whose key
-    ``{CHROM}_{pos0}_{end}_{sample}_{SVTYPE or POINT}`` is a record gets the record's call."""
+def match_edits(pos0: np.ndarray, rend: np.ndarray, chrom_of, svtype_of, kid_gts, samples: Sequence[str], read_records,
+                include_ambiguous, verbose, evidence_min_ratio):
+    """The edit list of the phased cells of a DNM list's records (``_lib.VCF_EDIT_DTYPE`` sorted by (record, sample),
+    and its CSR offsets by record), in O(#records); the core of both phased writers (``phase_edits`` here, and
+    ``bcfio.phase_edits``).  The candidate records are those whose (CHROM, pos0, end) is some phasing record's region;
+    their genotypes are decoded for the kids only, and every HET / HOM_ALT cell whose key
+    ``{CHROM}_{pos0}_{end}_{sample}_{SVTYPE or POINT}`` is a phasing record gets that record's call.  ``chrom_of(i)`` /
+    ``svtype_of(i)``: CHROM and SVTYPE (or "POINT") of record i; ``kid_gts(sel, kids)``: the genotype codes
+    [len(sel), len(kids)] of the samples ``kids`` in the records ``sel``."""
     from .unfazed import summarize_record, uet_code
-    n = int(recs.shape[0])
-    dec = dec or HostDecoder()
+    n = int(pos0.shape[0])
     regions = {(str(r["region"]["chrom"]), int(r["region"]["start"]), int(r["region"]["end"]))
                for r in read_records.values()}
     sidx = {s: i for i, s in enumerate(samples)}
@@ -494,27 +496,23 @@ def phase_edits(buf: np.ndarray, recs: np.ndarray, samples: Sequence[str], read_
     rows = []
     if regions and kids and n:
         pe = np.array(sorted({(p, e) for _c, p, e in regions}), dtype=np.int64)
-        key_l = recs["pos0"].astype(np.int64) * (1 << 32) + recs["rend"].astype(np.int64)
+        key_l = pos0.astype(np.int64) * (1 << 32) + rend.astype(np.int64)
         cand = np.flatnonzero(np.isin(key_l, pe[:, 0] * (1 << 32) + pe[:, 1]))
         chrom = {}
         keep = []
         for i in cand.tolist():
-            o = int(recs["line_off"][i])
-            c = buf[o: o + int(recs["chrom_len"][i])].tobytes().decode()
-            if (c, int(recs["pos0"][i]), int(recs["rend"][i])) in regions:
+            c = chrom_of(i)
+            if (c, int(pos0[i]), int(rend[i])) in regions:
                 chrom[i] = c
                 keep.append(i)
         if keep:
-            sel = np.array(keep, dtype=np.int64)
-            slot_of = np.full(len(samples), -1, dtype=np.int32)
-            slot_of[kids] = np.arange(len(kids), dtype=np.int32)
-            gt = dec.samples(sel, slot_of, len(kids), True)["gt"]
+            gt = kid_gts(np.array(keep, dtype=np.int64), kids)
             for li, i in enumerate(keep):
                 carriers = np.flatnonzero((gt[li] == HET) | (gt[li] == HOM_ALT))
                 if not carriers.shape[0]:
                     continue
-                head = "%s_%d_%d_" % (chrom[i], int(recs["pos0"][i]), int(recs["rend"][i]))
-                tail = "_" + _svtype(buf, recs[i])
+                head = "%s_%d_%d_" % (chrom[i], int(pos0[i]), int(rend[i]))
+                tail = "_" + svtype_of(i)
                 for m in carriers.tolist():
                     key = head + samples[kids[m]] + tail
                     rec = read_records.get(key)
@@ -532,6 +530,41 @@ def phase_edits(buf: np.ndarray, recs: np.ndarray, samples: Sequence[str], read_
         edits[name] = [r[k + 1] for r in rows]
     edit_off = np.searchsorted(line, np.arange(n + 1), side="left").astype(np.int64)
     return edit_off, edits
+
+
+def phase_edits(buf: np.ndarray, recs: np.ndarray, samples: Sequence[str], read_records, include_ambiguous, verbose,
+                evidence_min_ratio, dec=None):
+    """``match_edits`` of the lines of a text DNM list: CHROM and SVTYPE from the text, the kids' genotypes from the
+    decoder's ``samples``."""
+    dec = dec or HostDecoder()
+
+    def chrom_of(i):
+        o = int(recs["line_off"][i])
+        return buf[o: o + int(recs["chrom_len"][i])].tobytes().decode()
+
+    def kid_gts(sel, kids):
+        slot_of = np.full(len(samples), -1, dtype=np.int32)
+        slot_of[kids] = np.arange(len(kids), dtype=np.int32)
+        return dec.samples(sel, slot_of, len(kids), True)["gt"]
+    return match_edits(recs["pos0"], recs["rend"], chrom_of, lambda i: _svtype(buf, recs[i]), kid_gts, samples,
+                       read_records, include_ambiguous, verbose, evidence_min_ratio)
+
+
+def write_output(outfile: str, head: bytes, body) -> None:
+    """The header and body of a phased VCF to ``/dev/stdout``, to BGZF with an EOF block when ``outfile`` ends in
+    ``.gz``, else to a plain file."""
+    if outfile == "/dev/stdout":
+        import sys
+        sys.stdout.flush()
+        sys.stdout.buffer.write(head)
+        sys.stdout.buffer.write(memoryview(body))
+        sys.stdout.buffer.flush()
+    elif outfile.endswith(".gz"):
+        write_bgzf(outfile, head, memoryview(body))
+    else:
+        with open(outfile, "wb") as f:
+            f.write(head)
+            f.write(memoryview(body))
 
 
 def write_phased_vcf(in_path: str, read_records, include_ambiguous, verbose, outfile: str, evidence_min_ratio,
@@ -576,19 +609,7 @@ def write_phased_vcf(in_path: str, read_records, include_ambiguous, verbose, out
             gt = sub[gi] if gi < len(sub) else "."
             if "/" not in gt and "|" not in gt:
                 raise ValueError("%s: the haploid GT %r of sample %s cannot be phased" % (where(off), gt, samples[s]))
-    head = phased_header(data[:body], __version__)
-    if outfile == "/dev/stdout":
-        import sys
-        sys.stdout.flush()
-        sys.stdout.buffer.write(head)
-        sys.stdout.buffer.write(memoryview(out))
-        sys.stdout.buffer.flush()
-    elif outfile.endswith(".gz"):
-        write_bgzf(outfile, head, memoryview(out))
-    else:
-        with open(outfile, "wb") as f:
-            f.write(head)
-            f.write(memoryview(out))
+    write_output(outfile, phased_header(data[:body], __version__), out)
 
 
 # ------------------------------------------------------------------------------------------------
