@@ -652,6 +652,72 @@ int unfz_bcf_format_write(UnfzCtx*, const uint8_t* buf, const UnfzBcfRec* recs, 
                           int32_t n_ctg, const int32_t* keys, const int64_t* edit_off, const UnfzVcfEdit* edits,
                           int32_t n_samples, const uint8_t* status, const int64_t* out_off, uint8_t* out, void* stream);
 
+/* ---- CRAM 3.0 slice decoding (csrc/cram.cu) ---------------------------------------------------------------------
+ * Input, built by the host (cramio.py) from the selected slices: `blocks`, the decompressed core and external blocks
+ * of every slice (plus one read-group table per file: int32 n_rg, int32 off[n_rg + 1] relative to the table, then the
+ * "RGZ<id>\0" aux bytes); `ext`, the external blocks of every slice in slice order; `prog`, one int32 program per slice:
+ * [0] the number of encodings, [1] the index of the tag dictionary, [2..3] 0, then 4 int32 per encoding (codec id, and
+ * EXTERNAL: block index in the slice; HUFFMAN: count, index of (code, length, symbol) triples sorted by length and code;
+ * BYTE_ARRAY_LEN: length and value encoding numbers; BYTE_ARRAY_STOP: stop byte, block index; BETA: offset, bits;
+ * SUBEXP: offset, k; GAMMA: offset) -- the 28 data series BF CF RI RL AP RG RN MF NS NP TS NF TL FN FC FP DL BB QQ BS IN
+ * RS PD HC SC MQ BA QS first -- and the tag dictionary: n_lines, line_off[n_lines + 1], then (key, encoding number)
+ * pairs, key = tag[0] << 16 | tag[1] << 8 | BAM type; `refs` / `rbytes`, the reference spans a slice may read.
+ *
+ * Output: BAM records (block_size ... aux) of every record of every slice, back to back in slice order. */
+#define UNFZ_CRAM_MAX_EXT 128        /* external blocks per slice */
+#define UNFZ_CRAM_AP_DELTA 0x1       /* slice flags: AP is a delta from the previous record (from ap_start) */
+#define UNFZ_CRAM_OVERRUN 1          /* slice status: a stream read past its block */
+#define UNFZ_CRAM_BAD_ENCODING 2     /* slice status: a data series without a usable encoding, or a missing block */
+#define UNFZ_CRAM_BAD_VALUE 3        /* slice status: a value out of range (length, feature position, code, mate line) */
+typedef struct {
+    int64_t core_off;     /* core block: bytes [core_off, core_off + core_len) of blocks */
+    int64_t core_len;
+    int64_t ext_off;      /* first UnfzCramExt of the slice */
+    int64_t prog_off;     /* first int32 of the slice's program */
+    int64_t refs_off;     /* first UnfzCramRef of the slice */
+    int64_t rec_first;    /* index of the slice's first record among all records */
+    int64_t rg_off;       /* byte offset of the read-group table in blocks, or -1 */
+    int32_t n_ext;
+    int32_t n_records;
+    int32_t n_refs;
+    int32_t ref_id;       /* -2: multi-reference slice (RI per record), -1: unmapped */
+    int32_t ap_start;     /* the slice's alignment start (1-based): the first AP delta is relative to it */
+    int32_t flags;        /* UNFZ_CRAM_AP_DELTA */
+    uint8_t sub[5];       /* substitution matrix of the preservation map (reference A C G T N) */
+    uint8_t _pad[3];
+} UnfzCramSlice;
+typedef struct { int64_t off; int64_t len; } UnfzCramExt;
+typedef struct {
+    int64_t off;          /* first byte in rbytes */
+    int64_t start;        /* 0-based reference position of that byte */
+    int64_t len;
+    int32_t ref_id;
+    int32_t _pad;
+} UnfzCramRef;
+
+/* Host only: rANS 4x8 (order 0 or 1) of in[0..in_len) into out (at most out_cap bytes).  Returns the decoded length, or
+ * -1 for a malformed stream. */
+int64_t unfz_rans4x8_decode_host(const uint8_t* in, int64_t in_len, uint8_t* out, int64_t out_cap);
+/* Host only: rec_len[r] (BAM bytes with block_size) and rec_cig[r] (n_cigar) of every record, status[s] of every slice
+ * (UNFZ_CRAM_*).  Returns the number of failed slices. */
+int64_t unfz_cram_decode_size_host(const UnfzCramSlice* slices, int64_t n, const uint8_t* blocks, const UnfzCramExt* ext,
+                                   const int32_t* prog, const UnfzCramRef* refs, const uint8_t* rbytes, int64_t* rec_len,
+                                   int32_t* rec_cig, int32_t* status);
+/* Host only: the records at out + rec_off[r] (rec_off: the exclusive scan of rec_len, n_records + 1 entries), then the
+ * in-slice fix-up of attached mates.  Returns the number of failed slices. */
+int64_t unfz_cram_decode_write_host(const UnfzCramSlice* slices, int64_t n, const uint8_t* blocks, const UnfzCramExt* ext,
+                                    const int32_t* prog, const UnfzCramRef* refs, const uint8_t* rbytes,
+                                    const int32_t* rec_cig, const int64_t* rec_off, uint8_t* out, int32_t* status);
+/* Device: unfz_cram_decode_size_host, one thread per slice (cram_slice_size_kernel). */
+int unfz_cram_decode_size(UnfzCtx*, const UnfzCramSlice* slices, int64_t n, const uint8_t* blocks, const UnfzCramExt* ext,
+                          const int32_t* prog, const UnfzCramRef* refs, const uint8_t* rbytes, int64_t* rec_len,
+                          int32_t* rec_cig, int32_t* status, void* stream);
+/* Device: unfz_cram_decode_write_host, one thread per slice (cram_slice_write_kernel); slices whose size-step status is
+ * not 0 are skipped. */
+int unfz_cram_decode_write(UnfzCtx*, const UnfzCramSlice* slices, int64_t n, const uint8_t* blocks, const UnfzCramExt* ext,
+                           const int32_t* prog, const UnfzCramRef* refs, const uint8_t* rbytes, const int32_t* rec_cig,
+                           const int64_t* rec_off, uint8_t* out, int32_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

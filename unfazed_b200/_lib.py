@@ -115,6 +115,7 @@ VCFOUT_COLUMNS, VCFOUT_HAPLOID, VCFOUT_FIELDS = 0x01, 0x02, 0x04
 # record status of the BCF -> VCF formatter (csrc/bcfout.cu)
 BCFOUT_HAPLOID, BCFOUT_FLOAT_HOST, BCFOUT_BAD = 0x01, 0x02, 0x04
 assert VCF_EDIT_DTYPE.itemsize == 16
+CRAM_MAX_EXT = 128                       # UNFZ_CRAM_MAX_EXT: external blocks per slice (csrc/cram.cu)
 assert SEG_DTYPE.itemsize == 32 and DNM_DTYPE.itemsize == 48 and RSUM_DTYPE.itemsize == 32
 
 # constants of include/unfazed_sm100.h
@@ -194,6 +195,11 @@ SYMBOLS = {
                                        _P]),
     "unfz_bcf_format_write": (C.c_int, [_P, _P, _P, c_int64, _P, _P, c_int32, _P, _P, c_int32, _P, _P, _P, c_int32, _P, _P,
                                         _P, _P]),
+    "unfz_rans4x8_decode_host": (c_int64, [_P, c_int64, _P, c_int64]),
+    "unfz_cram_decode_size_host": (c_int64, [_P, c_int64, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "unfz_cram_decode_write_host": (c_int64, [_P, c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "unfz_cram_decode_size": (C.c_int, [_P, _P, c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "unfz_cram_decode_write": (C.c_int, [_P, _P, c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None

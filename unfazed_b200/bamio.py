@@ -14,7 +14,8 @@
 * ``CsiIndex`` / ``write_csi`` -- the CSI index (any ``min_shift`` / ``depth``) with the ``chunks`` queries of
   ``BaiIndex``; a BAM may come with a ``.csi`` instead of a ``.bai``, and ``vcfio`` and ``bcfio`` use it too.
 
-CRAM is not read here; ``datasource.load_reads`` sends it to pysam.
+CRAM 3.0 is decoded to these same BAM records by ``cramio.CramFile``, which ``read_regions`` takes in place of a
+``BamFile``; other CRAM versions go to pysam (``datasource.load_reads``).
 """
 from __future__ import annotations
 
@@ -596,7 +597,7 @@ def read_regions(paths: Dict[str, str], regions: Dict[str, Dict[str, List[Tuple[
     dev = engine.bam_decoder() if engine is not None else None
     parse = (lambda buf, offs, part: parse_records(buf, offs)) if dev is None else dev.parse
     kids = list(paths)
-    files = {kid: (p if isinstance(p, BamFile) else BamFile(p)) for kid, p in paths.items()}
+    files = {kid: (BamFile(p) if isinstance(p, str) else p) for kid, p in paths.items()}     # BamFile or cramio.CramFile
     recs = _Records(parse)
     head_tlen: Dict[str, np.ndarray] = {}
     if head_reads:

@@ -4,10 +4,12 @@
 * indexed BAM files (``*.bam`` with a ``.bai``) through ``bamio.py``, natively -- no pysam needed, and with an
   engine the bulk of the records is decoded on the GPU, or
 * indexed BAM files (``*.bam`` with a ``.bai`` or ``.csi``) through ``bamio.py`` as above, or
+* CRAM 3.0 files with a ``.crai`` and a plain-text FASTA reference through ``cramio.py``, decoded to the BAM records
+  ``bamio.py`` reads, or
 * a bgzipped, indexed sites VCF (``*.vcf.gz`` / ``*.vcf.bgz`` with a ``.tbi`` or ``.csi``) through ``vcfio.py``, natively
   -- no cyvcf2 needed, and with an engine the genotype fields are decoded on the GPU, or
 * a CSI-indexed BCF 2.2 sites file (``*.bcf`` with a ``.csi``) through ``bcfio.py``, natively, likewise, or
-* other sites VCF/BCF files (unindexed, uncompressed BCF, other BCF versions) through ``cyvcf2`` and the kids' other alignment files (CRAM, unindexed BAM) through ``pysam``
+* other sites VCF/BCF files (unindexed, uncompressed BCF, other BCF versions) through ``cyvcf2`` and the kids' other alignment files (other CRAM versions, unindexed CRAM or BAM) through ``pysam``
   -- imported lazily, so the package works without them as long as tables are supplied -- decoded only around
   the DNMs and packed by ``packers.py``.
 
@@ -21,7 +23,7 @@ from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 
-from . import bamio, bcfio, packers, vcfio
+from . import bamio, bcfio, cramio, packers, vcfio
 from .plan import strip_chr
 from .schema import ReadTable, SiteTable
 from .tableio import load_tables
@@ -132,7 +134,8 @@ def load_reads(dnms: List[dict], search_dist: int, readlen: int, insert_size_max
                min_gt_qual=20) -> Optional[ReadTable]:
     """One ReadTable for all kids of the DNM list (their ``bam`` entries name the files).
 
-    When every file is an indexed BAM it is read by ``bamio`` (no pysam).  With ``engine`` the bases and qualities
+    When every file is an indexed BAM or a CRAM 3.0 with a ``.crai`` and a plain FASTA ``cram_ref`` it is read by
+    ``bamio`` / ``cramio`` (no pysam; with ``engine`` the CRAM slices are decoded on the GPU too).  With ``engine`` the bases and qualities
     are then decoded on that engine's GPU: the table has no ``qual`` / ``seq2`` and carries its ``DeviceReads`` for
     the base-quality threshold of ``min_gt_qual`` (``table.device_reads``).  Every other input goes through pysam."""
     bam_of: Dict[str, str] = {}
@@ -150,8 +153,10 @@ def load_reads(dnms: List[dict], search_dist: int, readlen: int, insert_size_max
     reg = [_registry[n][1] for n in names if n in _registry and _registry[n][1] is not None]
     if reg and all(r is reg[0] for r in reg) and len(reg) == len(names):
         return reg[0]
-    if all(is_indexed_bam(n) for n in names):
-        files = {kid: bamio.BamFile(name) for kid, name in bam_of.items()}
+    ref_of = {kid: next((d.get("cram_ref") for d in dnms if d["kid"] == kid), None) for kid in bam_of}
+    if all(is_indexed_bam(name) or cramio.is_native_cram(name, ref_of[kid]) for kid, name in bam_of.items()):
+        files = {kid: bamio.BamFile(name) if is_indexed_bam(name) else cramio.CramFile(name, ref_of[kid], engine=engine)
+                 for kid, name in bam_of.items()}
         heads = {kid: f.head_tlen(insert_size_max_sample + 1) for kid, f in files.items()}
         regions = _regions(dnms, heads, lambda kid, c: c in files[kid].tids, search_dist, readlen)
         table = bamio.read_regions(files, regions, engine=engine, min_gt_qual=min_gt_qual)

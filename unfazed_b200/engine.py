@@ -220,7 +220,10 @@ class BamDecoder:
             st = torch.cuda.current_stream(eng.device)
             e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
             e[0].record(st)
-            d = _to_device(np.ascontiguousarray(buf), eng.device, True, 16)
+            d = buf.resident if isinstance(buf, ResidentBytes) else None   # records decoded on this GPU stay there
+            if d is None:
+                d = _to_device(np.ascontiguousarray(buf), eng.device, True, 16)
+                self.h2d_bytes += int(buf.nbytes)
             doffs = _to_device(np.ascontiguousarray(offs, dtype=np.int64), eng.device, True)
             e[1].record(st)
             out = torch.empty((max(n, 1) * L.BAM_REC_DTYPE.itemsize,), dtype=torch.uint8, device=eng.device)
@@ -230,7 +233,7 @@ class BamDecoder:
             rec = out[: n * L.BAM_REC_DTYPE.itemsize].cpu().numpy().view(L.BAM_REC_DTYPE)
         self._time("h2d_records", e[0], e[1])
         self._time("parse", e[1], e[2])
-        self.h2d_bytes += int(buf.nbytes + offs.nbytes)
+        self.h2d_bytes += int(offs.nbytes)
         bad = int(np.count_nonzero(rec["aux"] & L.BAM_AUX_BAD))
         if bad:
             raise ValueError("%d malformed BAM record(s): fields or aux tags overrun block_size" % bad)
@@ -304,6 +307,75 @@ class BamDecoder:
             e1.synchronize()
             self._time("emit", e0, e1)
         return self._reads
+
+
+class ResidentBytes(np.ndarray):
+    """Host bytes with an identical copy on the device (``resident``, 16 bytes of tail padding): ``BamDecoder.parse``
+    takes that copy instead of uploading the host one."""
+    resident = None
+
+
+class CramDecoder:
+    """Device side of ``cramio.CramFile`` with an engine: the decompressed blocks of the selected slices, their
+    descriptors and the reference spans go up; cram_slice_size_kernel sizes every record, unfz_exclusive_scan_i64
+    places them, cram_slice_write_kernel writes the BAM records.  The records stay on the device for the BAM stages
+    (``ResidentBytes``); a host copy comes back because ``bamio.read_regions`` reads names, CIGARs and the lone mates'
+    bytes on the host."""
+
+    def __init__(self, engine: "Engine"):
+        self.engine = engine
+        self.h2d_bytes = 0
+        self.d2h_bytes = 0
+        self.timings_ms: Dict[str, float] = {}
+
+    def _time(self, name, e0, e1):
+        self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
+
+    def decode(self, cram, desc):
+        sl, blocks, ext, prog, ref, rbytes, n_rec, coffs = desc
+        eng = self.engine
+        lib, ctx, dev = eng.lib, eng.ctx, eng.device
+        n = int(sl.shape[0])
+        with eng.on_stream():
+            st = torch.cuda.current_stream(dev)
+            sp = C.c_void_p(st.cuda_stream)
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(6)]
+            e[0].record(st)
+            up = [_to_device(np.ascontiguousarray(a).view(np.uint8).reshape(-1), dev, True, 16)
+                  for a in (sl, blocks, ext, prog, ref, rbytes)]
+            args = (up[0].data_ptr(), n) + tuple(u.data_ptr() for u in up[1:])
+            e[1].record(st)
+            rec_len = torch.zeros((n_rec + 1,), dtype=torch.int64, device=dev)
+            rec_cig = eng._zeros(n_rec, torch.int32)
+            status = eng._zeros(n, torch.int32)
+            eng._check(lib.unfz_cram_decode_size(ctx, *args, rec_len.data_ptr(), rec_cig.data_ptr(), status.data_ptr(), sp),
+                       "cram_decode_size")
+            e[2].record(st)
+            offs = torch.empty((n_rec + 1,), dtype=torch.int64, device=dev)
+            work = torch.empty((int(lib.unfz_scan_work_bytes(n_rec + 1)),), dtype=torch.uint8, device=dev)
+            eng._check(lib.unfz_exclusive_scan_i64(ctx, rec_len.data_ptr(), offs.data_ptr(), n_rec + 1, work.data_ptr(), sp),
+                       "exclusive_scan_i64")
+            e[3].record(st)
+            total = int(offs[n_rec].item())
+            cram.check_status(status.cpu().numpy(), coffs)
+            out = torch.zeros((total + 16,), dtype=torch.uint8, device=dev)
+            e[4].record(st)
+            eng._check(lib.unfz_cram_decode_write(ctx, *args, rec_cig.data_ptr(), offs.data_ptr(), out.data_ptr(),
+                                                  status.data_ptr(), sp), "cram_decode_write")
+            e[5].record(st)
+            stat = status.cpu().numpy()
+            host = out[:total].cpu().numpy()
+            hoffs = offs[:n_rec].cpu().numpy()
+        cram.check_status(stat, coffs)
+        self._time("h2d", e[0], e[1])
+        self._time("size", e[1], e[2])
+        self._time("scan", e[2], e[3])
+        self._time("write", e[4], e[5])
+        self.h2d_bytes += sum(int(u.numel()) for u in up)
+        self.d2h_bytes += total + 8 * n_rec + 8 * n + 8
+        buf = host.view(ResidentBytes)
+        buf.resident = out
+        return buf, hoffs
 
 
 class VcfDecoder:
@@ -863,6 +935,12 @@ class Engine:
     def bcf_decoder(self) -> BcfDecoder:
         """A device decoder for one ``bcfio.read_sites`` load."""
         return BcfDecoder(self)
+
+    def cram_decoder(self) -> CramDecoder:
+        """The device slice decoder of this engine's ``cramio.CramFile`` loads (timings and bytes accumulate)."""
+        if getattr(self, "_cram", None) is None:
+            self._cram = CramDecoder(self)
+        return self._cram
 
     def decode_bam(self, paths, regions, head_reads: int = 0, min_gt_qual=20) -> DeviceReads:
         """Indexed BAM files -> DeviceReads, the bulk of the records decoded on this GPU (``bamio.read_regions``).
