@@ -222,7 +222,9 @@ int unfz_ctx_set_guard(UnfzCtx*, const int32_t* flag);
 int unfz_check_caps(UnfzCtx*, int32_t k, const int64_t* const* h_totals, const int64_t* h_caps, int32_t* flag,
                     int64_t* actual, void* stream);
 
-/* Exclusive prefix sums (device-wide).  `work` needs unfz_scan_work_bytes(n) bytes. */
+/* Exclusive prefix sums (device-wide).  `work` needs unfz_scan_work_bytes(n) bytes.  unfz_exclusive_scan_i64 writes
+ * n + 1 values: out[0..n) the exclusive sums of in[0..n), and out[n] the total (0 when n = 0), so `out` needs n + 1
+ * entries. */
 int64_t unfz_scan_work_bytes(int64_t n);
 int unfz_exclusive_scan_i64(UnfzCtx*, const int64_t* in, int64_t* out, int64_t n, void* work, void* stream);
 int unfz_exclusive_scan_u8_i32(UnfzCtx*, const uint8_t* in, int32_t* out, int64_t n, void* work, void* stream);

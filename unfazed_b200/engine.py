@@ -194,7 +194,99 @@ class DeviceReads:
         return self.h2d_bytes
 
 
-class BamDecoder:
+class _Decoder:
+    """What the device decoders share: the bytes that crossed PCIe each way, the device time of every stage by name
+    (``timings_ms``, accumulated over calls), and the upload, launch and two-pass output they all use."""
+
+    def __init__(self, engine: "Engine"):
+        self.engine = engine
+        self.h2d_bytes = self.d2h_bytes = 0
+        self.timings_ms: Dict[str, float] = {}
+
+    @contextlib.contextmanager
+    def _stages(self):
+        """Context on the engine's stream that yields ``mark``: ``mark(name)`` records an event that closes the
+        interval ``name``, begun at the previous mark (or on entry); ``mark(None)`` begins an interval without timing
+        the gap before it.  On a normal exit every interval is added to ``timings_ms``, read once the last event has
+        completed."""
+        marks = []
+
+        def mark(name):
+            ev = torch.cuda.Event(enable_timing=True)
+            ev.record(self.engine.stream)
+            marks.append((name, ev))
+        with self.engine.on_stream():
+            mark(None)
+            yield mark
+        marks[-1][1].synchronize()
+        for (_, e0), (name, e1) in zip(marks, marks[1:]):
+            if name is not None:
+                self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
+
+    def _up(self, a: np.ndarray, dtype=None, pad: int = 0, fill: int = 0) -> torch.Tensor:
+        """Host array -> device through pinned staging (+ ``pad`` zero elements), its bytes counted in ``h2d_bytes``.
+        An empty array becomes one 16-byte buffer with ``fill`` in every element, so a kernel that is told there are no
+        items still gets a valid address (``fill=-1`` for a ``slot_of``: no column)."""
+        a = np.ascontiguousarray(a, dtype=dtype)
+        self.h2d_bytes += int(a.nbytes)
+        if a.shape[0]:
+            return _to_device(a, self.engine.device, True, pad)
+        t = torch.from_numpy(a.view(np.uint8) if a.dtype.fields is not None else a)
+        return torch.full((16 // t.element_size(),), fill, dtype=t.dtype, device=self.engine.device)
+
+    def _launch(self, fn: str, *args) -> None:
+        """``lib.<fn>(ctx, *args, stream)`` on the engine's stream, a tensor passed by its device address; raises
+        with the library's message when it fails."""
+        eng = self.engine
+        args = [a.data_ptr() if isinstance(a, torch.Tensor) else a for a in args]
+        eng._check(getattr(eng.lib, fn)(eng.ctx, *args, C.c_void_p(eng.stream.cuda_stream)), fn)
+
+    def _scan(self, lens: torch.Tensor, off: torch.Tensor, n: int) -> None:
+        """``off[0..n]``: the exclusive scan of ``lens[:n]``, ``off[n]`` the total."""
+        self._launch("unfz_exclusive_scan_i64", lens, off, n, self.engine._scan_work(n))
+
+    def _size_scan(self, mark, names, n: int, n_status: int, status_dtype, size):
+        """First pass of an output of ``n`` items of variable length: ``size(out_len, status)`` launches the kernel
+        that writes the length of every item to ``out_len[:n]`` and the statuses (``n_status`` zeroed elements of
+        ``status_dtype``); ``_scan`` places the items; the statuses and the total come down in one copy, for the
+        caller to check before ``_write``.  ``names``: the timed intervals (``mark``) that end after the size kernel,
+        the scan and the download.  Returns (out_len, offsets, device status, host status, total)."""
+        eng = self.engine
+        out_len = eng._empty(n, torch.int64)
+        off = torch.empty((n + 1,), dtype=torch.int64, device=eng.device)
+        # the statuses, then the total at the next multiple of 8 bytes: one download
+        sb = n_status * torch.iinfo(status_dtype).bits // 8
+        nb = (sb + 7) // 8 * 8
+        stat = torch.zeros((nb + 8,), dtype=torch.uint8, device=eng.device)
+        status = stat[:sb].view(status_dtype)
+        size(out_len, status)
+        mark(names[0])
+        self._scan(out_len, off, n)
+        mark(names[1])
+        stat[nb:].view(torch.int64).copy_(off[n:])
+        host = stat.cpu()
+        mark(names[2])
+        self.d2h_bytes += nb + 8
+        return out_len, off, status, host[:sb].view(status_dtype).numpy(), int(host[nb:].view(torch.int64)[0])
+
+    def _write(self, mark, names, total: int, write, out: Optional[torch.Tensor] = None) -> np.ndarray:
+        """Second pass: ``write(out)`` launches the kernel that writes the items into ``out`` (``total`` bytes unless
+        the caller passes one), and the output comes down in one copy.  ``names``: the timed intervals (``mark``)
+        that end after the kernel and after the download; the gap before the kernel is not timed."""
+        if out is None:
+            out = self.engine._empty(total, torch.uint8)
+        mark(None)
+        write(out)
+        mark(names[0])
+        # one copy into pageable memory (the driver stages it): page-locking a fresh block of the output's size costs
+        # more than the copy itself
+        host = out[:total].cpu()
+        mark(names[1])
+        self.d2h_bytes += total
+        return host.numpy()
+
+
+class BamDecoder(_Decoder):
     """Device side of ``bamio.read_regions(engine=...)``: the inflated record bytes go up once (pinned), the fixed
     fields are parsed there (unfz_bam_parse) and come back for the host's selection, and the bulk columns are emitted
     on the device.  The record bytes stay resident, so the planes of another base-quality threshold are decoded again
@@ -203,37 +295,25 @@ class BamDecoder:
     with several files the parts are concatenated once on the device, which briefly holds both copies."""
 
     def __init__(self, engine: "Engine"):
-        self.engine = engine
+        super().__init__(engine)
         self.parts: List[torch.Tensor] = []
         self.dbuf = self.dsrc = self.table = None
         self._reads: Optional[DeviceReads] = None
-        self.h2d_bytes = 0
-        self.timings_ms: Dict[str, float] = {}
-
-    def _time(self, name, e0, e1):
-        self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
 
     def parse(self, buf: np.ndarray, offs: np.ndarray, part: int) -> np.ndarray:
-        eng = self.engine
         n = int(offs.shape[0])
-        with eng.on_stream():
-            st = torch.cuda.current_stream(eng.device)
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
-            e[0].record(st)
+        rsz = L.BAM_REC_DTYPE.itemsize
+        with self._stages() as mark:
             d = buf.resident if isinstance(buf, ResidentBytes) else None   # records decoded on this GPU stay there
             if d is None:
-                d = _to_device(np.ascontiguousarray(buf), eng.device, True, 16)
-                self.h2d_bytes += int(buf.nbytes)
-            doffs = _to_device(np.ascontiguousarray(offs, dtype=np.int64), eng.device, True)
-            e[1].record(st)
-            out = torch.empty((max(n, 1) * L.BAM_REC_DTYPE.itemsize,), dtype=torch.uint8, device=eng.device)
-            eng._check(eng.lib.unfz_bam_parse(eng.ctx, d.data_ptr(), int(buf.shape[0]), doffs.data_ptr(), n, out.data_ptr(),
-                                              C.c_void_p(st.cuda_stream)), "bam_parse")
-            e[2].record(st)
-            rec = out[: n * L.BAM_REC_DTYPE.itemsize].cpu().numpy().view(L.BAM_REC_DTYPE)
-        self._time("h2d_records", e[0], e[1])
-        self._time("parse", e[1], e[2])
-        self.h2d_bytes += int(offs.nbytes)
+                d = self._up(buf, pad=16)
+            doffs = self._up(offs, np.int64)
+            mark("h2d_records")
+            out = self.engine._empty(n * rsz, torch.uint8)
+            self._launch("unfz_bam_parse", d, int(buf.shape[0]), doffs, n, out)
+            mark("parse")
+            rec = out[: n * rsz].cpu().numpy().view(L.BAM_REC_DTYPE)
+        self.d2h_bytes += int(rec.nbytes)
         bad = int(np.count_nonzero(rec["aux"] & L.BAM_AUX_BAD))
         if bad:
             raise ValueError("%d malformed BAM record(s): fields or aux tags overrun block_size" % bad)
@@ -243,48 +323,33 @@ class BamDecoder:
     def prepare(self, src: np.ndarray) -> None:
         """The parts as one device buffer and the record offset of every output read (``src``: byte offsets in the parts
         back to back)."""
-        eng = self.engine
-        with eng.on_stream():
-            st = torch.cuda.current_stream(eng.device)
-            e0 = torch.cuda.Event(enable_timing=True)
-            e0.record(st)
+        with self._stages() as mark:
             self.dbuf = torch.cat(self.parts) if len(self.parts) != 1 else self.parts[0]
             if self.dbuf.numel() == 0:
-                self.dbuf = torch.zeros((16,), dtype=torch.uint8, device=eng.device)
+                self.dbuf = torch.zeros((16,), dtype=torch.uint8, device=self.engine.device)
             self.parts = [self.dbuf]
-            self.dsrc = _to_device(np.ascontiguousarray(src, dtype=np.int64), eng.device, True)
-            self.h2d_bytes += int(src.nbytes)
-            e1 = torch.cuda.Event(enable_timing=True)
-            e1.record(st)
-        e1.synchronize()
-        self._time("concat_src", e0, e1)
+            self.dsrc = self._up(src, np.int64)
+            mark("concat_src")
 
     def mate_join(self, name_hash: np.ndarray, blk: np.ndarray, flag: np.ndarray) -> np.ndarray:
         """Mate index of every output read (after ``prepare``), as packers._mate_join defines it inside each block:
         the reads are ordered by (block, name hash) with torch's stable sort, unfz_bam_mate_join picks the first primary
         read of the other segment in each group and compares the name bytes of every joined pair; -2 marks the reads
         left to the host (a hash collision, or a read that is its own candidate)."""
-        eng = self.engine
         n = int(name_hash.shape[0])
         if n == 0:
             return np.zeros(0, dtype=np.int64)
-        with eng.on_stream():
-            st = torch.cuda.current_stream(eng.device)
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(st)
-            dh = _to_device(np.ascontiguousarray(name_hash).view(np.int64), eng.device, True)
-            db = _to_device(np.ascontiguousarray(blk, dtype=np.int32), eng.device, True)
-            df = _to_device(np.ascontiguousarray(flag, dtype=np.int32), eng.device, True)
+        with self._stages() as mark:
+            dh = self._up(np.ascontiguousarray(name_hash).view(np.int64))
+            db = self._up(blk, np.int32)
+            df = self._up(flag, np.int32)
             o1 = torch.sort(dh, stable=True).indices
             order = o1[torch.sort(db[o1], stable=True).indices].contiguous()
-            mate = torch.empty((n,), dtype=torch.int32, device=eng.device)
-            eng._check(eng.lib.unfz_bam_mate_join(eng.ctx, order.data_ptr(), dh.data_ptr(), db.data_ptr(), df.data_ptr(), n,
-                                                  self.dbuf.data_ptr(), self.dsrc.data_ptr(), mate.data_ptr(),
-                                                  C.c_void_p(st.cuda_stream)), "bam_mate_join")
-            e1.record(st)
+            mate = torch.empty((n,), dtype=torch.int32, device=self.engine.device)
+            self._launch("unfz_bam_mate_join", order, dh, db, df, n, self.dbuf, self.dsrc, mate)
+            mark("mate_join")
             out = mate.cpu().numpy().astype(np.int64)
-        self._time("mate_join", e0, e1)
-        self.h2d_bytes += 16 * n
+        self.d2h_bytes += 4 * n
         return out
 
     def emit(self, table: ReadTable, min_gt_qual) -> DeviceReads:
@@ -298,14 +363,9 @@ class BamDecoder:
         if self._reads is None or self._reads.min_bq != mb:
             self._reads = None
             eng = self.engine
-            with eng.on_stream():
-                st = torch.cuda.current_stream(eng.device)
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record(st)
+            with self._stages() as mark:
                 self._reads = DeviceReads.from_bam(self.table, eng.device, mb, eng, self.dbuf, self.dsrc)
-                e1.record(st)
-            e1.synchronize()
-            self._time("emit", e0, e1)
+                mark("emit")
         return self._reads
 
 
@@ -315,70 +375,44 @@ class ResidentBytes(np.ndarray):
     resident = None
 
 
-class CramDecoder:
+class CramDecoder(_Decoder):
     """Device side of ``cramio.CramFile`` with an engine: the decompressed blocks of the selected slices, their
     descriptors and the reference spans go up; cram_slice_size_kernel sizes every record, unfz_exclusive_scan_i64
     places them, cram_slice_write_kernel writes the BAM records.  The records stay on the device for the BAM stages
     (``ResidentBytes``); a host copy comes back because ``bamio.read_regions`` reads names, CIGARs and the lone mates'
     bytes on the host."""
 
-    def __init__(self, engine: "Engine"):
-        self.engine = engine
-        self.h2d_bytes = 0
-        self.d2h_bytes = 0
-        self.timings_ms: Dict[str, float] = {}
-
-    def _time(self, name, e0, e1):
-        self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
-
     def decode(self, cram, desc):
         sl, blocks, ext, prog, ref, rbytes, n_rec, coffs = desc
         eng = self.engine
-        lib, ctx, dev = eng.lib, eng.ctx, eng.device
         n = int(sl.shape[0])
-        with eng.on_stream():
-            st = torch.cuda.current_stream(dev)
-            sp = C.c_void_p(st.cuda_stream)
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(6)]
-            e[0].record(st)
-            up = [_to_device(np.ascontiguousarray(a).view(np.uint8).reshape(-1), dev, True, 16)
-                  for a in (sl, blocks, ext, prog, ref, rbytes)]
-            args = (up[0].data_ptr(), n) + tuple(u.data_ptr() for u in up[1:])
-            e[1].record(st)
-            rec_len = torch.zeros((n_rec + 1,), dtype=torch.int64, device=dev)
+        with self._stages() as mark:
+            args = [self._up(np.ascontiguousarray(a).view(np.uint8).reshape(-1), pad=16)
+                    for a in (sl, blocks, ext, prog, ref, rbytes)]
+            args.insert(1, n)
+            mark("h2d")
             rec_cig = eng._zeros(n_rec, torch.int32)
-            status = eng._zeros(n, torch.int32)
-            eng._check(lib.unfz_cram_decode_size(ctx, *args, rec_len.data_ptr(), rec_cig.data_ptr(), status.data_ptr(), sp),
-                       "cram_decode_size")
-            e[2].record(st)
-            offs = torch.empty((n_rec + 1,), dtype=torch.int64, device=dev)
-            work = torch.empty((int(lib.unfz_scan_work_bytes(n_rec + 1)),), dtype=torch.uint8, device=dev)
-            eng._check(lib.unfz_exclusive_scan_i64(ctx, rec_len.data_ptr(), offs.data_ptr(), n_rec + 1, work.data_ptr(), sp),
-                       "exclusive_scan_i64")
-            e[3].record(st)
-            total = int(offs[n_rec].item())
-            cram.check_status(status.cpu().numpy(), coffs)
-            out = torch.zeros((total + 16,), dtype=torch.uint8, device=dev)
-            e[4].record(st)
-            eng._check(lib.unfz_cram_decode_write(ctx, *args, rec_cig.data_ptr(), offs.data_ptr(), out.data_ptr(),
-                                                  status.data_ptr(), sp), "cram_decode_write")
-            e[5].record(st)
+            _, offs, status, stat, total = self._size_scan(
+                mark, ("size", "scan", None), n_rec, n, torch.int32,
+                lambda rec_len, st: self._launch("unfz_cram_decode_size", *args, rec_len, rec_cig, st))
+            cram.check_status(stat, coffs)
+            # zeroed: the write step ORs the bases into place, two to a byte, and the 16-byte tail stays zero
+            out = torch.zeros((total + 16,), dtype=torch.uint8, device=eng.device)
+            host = self._write(mark, ("write", None), total,
+                               lambda out: self._launch("unfz_cram_decode_write", *args, rec_cig, offs, out, status), out)
             stat = status.cpu().numpy()
-            host = out[:total].cpu().numpy()
             hoffs = offs[:n_rec].cpu().numpy()
+        self.d2h_bytes += int(stat.nbytes + hoffs.nbytes)
         cram.check_status(stat, coffs)
-        self._time("h2d", e[0], e[1])
-        self._time("size", e[1], e[2])
-        self._time("scan", e[2], e[3])
-        self._time("write", e[4], e[5])
-        self.h2d_bytes += sum(int(u.numel()) for u in up)
-        self.d2h_bytes += total + 8 * n_rec + 8 * n + 8
         buf = host.view(ResidentBytes)
         buf.resident = out
         return buf, hoffs
 
 
-class VcfDecoder:
+_CELLS = (("gt", torch.uint8), ("gq", torch.float32), ("rd", torch.int32), ("ad", torch.int32), ("status", torch.uint8))
+
+
+class VcfDecoder(_Decoder):
     """Device side of ``vcfio.read_sites(engine=...)``, with the calls of ``vcfio.HostDecoder``: the inflated text goes
     up once (pinned staging), the newline pass (unfz_vcf_line_count, a scan, unfz_vcf_line_write) and the fixed-field
     parse (unfz_vcf_parse) run on the engine's stream and the 64-byte records come back for the host's selection; then
@@ -386,92 +420,50 @@ class VcfDecoder:
     The floats it leaves to the host are decoded by ``vcfio.finish_cells``.  ``rewrite`` writes the phased VCF body from
     the same resident text and records (``vcfio.write_phased_vcf``)."""
 
-    def __init__(self, engine: "Engine"):
-        self.engine = engine
-        self.h2d_bytes = self.d2h_bytes = 0
-        self.timings_ms: Dict[str, float] = {}
-
-    def _time(self, name, e0, e1):
-        self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
-
     def lines(self, buf: np.ndarray) -> np.ndarray:
         eng = self.engine
-        lib, ctx, dev = eng.lib, eng.ctx, eng.device
         n = int(buf.shape[0])
-        chunks = int(lib.unfz_vcf_chunks(n))
-        with eng.on_stream():
-            st = torch.cuda.current_stream(dev)
-            sp = C.c_void_p(st.cuda_stream)
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
-            e[0].record(st)
+        chunks = int(eng.lib.unfz_vcf_chunks(n))
+        rsz = L.VCF_REC_DTYPE.itemsize
+        with self._stages() as mark:
             # 16 bytes of padding: the sample pass reads whole 16-byte words
-            self.dbuf = _to_device(np.ascontiguousarray(buf), dev, True, 16) if n else torch.zeros(16, dtype=torch.uint8,
-                                                                                                 device=dev)
-            e[1].record(st)
-            cnt = torch.empty((max(chunks, 1),), dtype=torch.int32, device=dev)
-            at = torch.empty((chunks + 1,), dtype=torch.int32, device=dev)
-            total = torch.zeros((1,), dtype=torch.int64, device=dev)
-            work = torch.empty((int(lib.unfz_scan_work_bytes(chunks)),), dtype=torch.uint8, device=dev)
-            eng._check(lib.unfz_vcf_line_count(ctx, self.dbuf.data_ptr(), n, cnt.data_ptr(), sp), "vcf_line_count")
-            eng._check(lib.unfz_exclusive_scan_u32(ctx, cnt.data_ptr(), at.data_ptr(), chunks, total.data_ptr(),
-                                                   work.data_ptr(), sp), "exclusive_scan_u32")
+            self.dbuf = self._up(buf, pad=16)
+            mark("h2d_text")
+            cnt = eng._empty(chunks, torch.int32)
+            at = torch.empty((chunks + 1,), dtype=torch.int32, device=eng.device)
+            total = torch.zeros((1,), dtype=torch.int64, device=eng.device)
+            self._launch("unfz_vcf_line_count", self.dbuf, n, cnt)
+            self._launch("unfz_exclusive_scan_u32", cnt, at, chunks, total, eng._scan_work(chunks))
             n_lines = self.n_lines = int(total.item())
-            self.ends = torch.empty((max(n_lines, 1),), dtype=torch.int64, device=dev)
-            eng._check(lib.unfz_vcf_line_write(ctx, self.dbuf.data_ptr(), n, at.data_ptr(), self.ends.data_ptr(), sp),
-                       "vcf_line_write")
-            e[2].record(st)
-            rsz = L.VCF_REC_DTYPE.itemsize
-            self.drecs = torch.empty((max(n_lines, 1) * rsz,), dtype=torch.uint8, device=dev)
-            eng._check(lib.unfz_vcf_parse(ctx, self.dbuf.data_ptr(), self.ends.data_ptr(), n_lines, self.drecs.data_ptr(),
-                                          sp), "vcf_parse")
-            e[3].record(st)
+            self.ends = eng._empty(n_lines, torch.int64)
+            self._launch("unfz_vcf_line_write", self.dbuf, n, at, self.ends)
+            mark("line_bounds")
+            self.drecs = eng._empty(n_lines * rsz, torch.uint8)
+            self._launch("unfz_vcf_parse", self.dbuf, self.ends, n_lines, self.drecs)
+            mark("parse")
             recs = self.drecs[: n_lines * rsz].cpu().numpy().view(L.VCF_REC_DTYPE)
-            e[4].record(st)
-        e[4].synchronize()
-        self._time("h2d_text", e[0], e[1])
-        self._time("line_bounds", e[1], e[2])
-        self._time("parse", e[2], e[3])
-        self._time("d2h_records", e[3], e[4])
-        self.h2d_bytes += n
+            mark("d2h_records")
         self.d2h_bytes += int(recs.nbytes) + 8
         return recs
 
     def samples(self, sel: np.ndarray, slot_of: np.ndarray, n_members: int, gq_float: bool,
                 max_digits: int = 15) -> Dict[str, np.ndarray]:
         eng = self.engine
-        lib, ctx, dev = eng.lib, eng.ctx, eng.device
-        ns = int(sel.shape[0])
-        m = int(n_members)
+        ns, m = int(sel.shape[0]), int(n_members)
         cells = ns * m
-        with eng.on_stream():
-            st = torch.cuda.current_stream(dev)
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
-            e[0].record(st)
-            dsel = _to_device(np.ascontiguousarray(sel, dtype=np.int64), dev, True) if ns else \
-                torch.zeros(1, dtype=torch.int64, device=dev)
-            dslot = _to_device(np.ascontiguousarray(slot_of, dtype=np.int32), dev, True) if slot_of.shape[0] else \
-                torch.full((1,), -1, dtype=torch.int32, device=dev)
-            e[1].record(st)
-            out = {"gt": torch.empty((max(cells, 1),), dtype=torch.uint8, device=dev),
-                   "gq": torch.empty((max(cells, 1),), dtype=torch.float32, device=dev),
-                   "rd": torch.empty((max(cells, 1),), dtype=torch.int32, device=dev),
-                   "ad": torch.empty((max(cells, 1),), dtype=torch.int32, device=dev),
-                   "status": torch.empty((max(cells, 1),), dtype=torch.uint8, device=dev),
-                   "line_bad": torch.empty((max(ns, 1),), dtype=torch.uint8, device=dev)}
-            eng._check(lib.unfz_vcf_samples(ctx, self.dbuf.data_ptr(), self.drecs.data_ptr(), dsel.data_ptr(), ns,
-                                            dslot.data_ptr(), int(slot_of.shape[0]), m, int(bool(gq_float)), int(max_digits),
-                                            *(out[k].data_ptr() for k in ("gt", "gq", "rd", "ad", "status", "line_bad")),
-                                            C.c_void_p(st.cuda_stream)), "vcf_samples")
-            e[2].record(st)
+        with self._stages() as mark:
+            dsel = self._up(sel, np.int64)
+            dslot = self._up(slot_of, np.int32, fill=-1)
+            mark("h2d_select")
+            out = {k: eng._empty(cells, dt) for k, dt in _CELLS}
+            out["line_bad"] = eng._empty(ns, torch.uint8)
+            self._launch("unfz_vcf_samples", self.dbuf, self.drecs, dsel, ns, dslot, int(slot_of.shape[0]), m,
+                         int(bool(gq_float)), int(max_digits), *(out[k] for k, _ in _CELLS), out["line_bad"])
+            mark("samples")
             host = {k: v.cpu().numpy() for k, v in out.items()}
-            e[3].record(st)
-        e[3].synchronize()
-        self._time("h2d_select", e[0], e[1])
-        self._time("samples", e[1], e[2])
-        self._time("d2h_cells", e[2], e[3])
-        self.h2d_bytes += int(sel.nbytes + slot_of.nbytes)
+            mark("d2h_cells")
         self.d2h_bytes += cells * 14 + ns
-        res = {k: host[k][:cells].reshape(ns, m) for k in ("gt", "gq", "rd", "ad", "status")}
+        res = {k: host[k][:cells].reshape(ns, m) for k, _ in _CELLS}
         res["line_bad"] = host["line_bad"][:ns]
         return res
 
@@ -481,140 +473,61 @@ class VcfDecoder:
         (unfz_vcf_rewrite_size), scanned (unfz_exclusive_scan_i64) and written (unfz_vcf_rewrite_write) on the engine's
         stream, and the output comes down in one copy.  With a bad line nothing is written: the output
         is empty and the status says why."""
-        eng = self.engine
-        lib, ctx, dev = eng.lib, eng.ctx, eng.device
         n = self.n_lines
-        ne = int(edits.shape[0])
-        with eng.on_stream():
-            st = torch.cuda.current_stream(dev)
-            sp = C.c_void_p(st.cuda_stream)
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
-            e[0].record(st)
-            doff = _to_device(np.ascontiguousarray(edit_off, dtype=np.int64), dev, True)
-            ded = _to_device(np.ascontiguousarray(edits, dtype=L.VCF_EDIT_DTYPE), dev, True) if ne else \
-                torch.zeros(16, dtype=torch.uint8, device=dev)
-            e[1].record(st)
-            out_len = torch.empty((max(n, 1),), dtype=torch.int64, device=dev)
-            # the status of every line, then the total output length, in one download
-            nb = (n + 7) // 8 * 8
-            stat = torch.zeros((nb + 8,), dtype=torch.uint8, device=dev)
-            out_off = torch.empty((n + 1,), dtype=torch.int64, device=dev)
-            work = torch.empty((int(lib.unfz_scan_work_bytes(max(n, 1))),), dtype=torch.uint8, device=dev)
-            eng._check(lib.unfz_vcf_rewrite_size(ctx, self.dbuf.data_ptr(), self.drecs.data_ptr(), n, doff.data_ptr(),
-                                                 ded.data_ptr(), int(n_samples), out_len.data_ptr(), stat.data_ptr(), sp),
-                       "vcf_rewrite_size")
-            if n:
-                eng._check(lib.unfz_exclusive_scan_i64(ctx, out_len.data_ptr(), out_off.data_ptr(), n, work.data_ptr(), sp),
-                           "exclusive_scan_i64")
-            else:
-                out_off.zero_()
-            stat[nb:].view(torch.int64).copy_(out_off[n:])
-            host_stat = stat.cpu().numpy()
-            e[2].record(st)
-        line_bad = host_stat[:n].copy()
-        total = int(host_stat[nb:].view(np.int64)[0])
-        self.h2d_bytes += int(edit_off.nbytes) + ne * L.VCF_EDIT_DTYPE.itemsize
-        self.d2h_bytes += nb + 8
-        if line_bad.any():
-            self._time("h2d_edits", e[0], e[1])
-            return np.zeros(0, dtype=np.uint8), line_bad
-        with eng.on_stream():
-            out = torch.empty((max(total, 1),), dtype=torch.uint8, device=dev)
-            eng._check(lib.unfz_vcf_rewrite_write(ctx, self.dbuf.data_ptr(), self.drecs.data_ptr(), n, doff.data_ptr(),
-                                                  ded.data_ptr(), int(n_samples), out_off.data_ptr(), out.data_ptr(), sp),
-                       "vcf_rewrite_write")
-            e[3].record(st)
-            # one copy into pageable memory (the driver stages it): page-locking a fresh block of the output's size costs
-            # more than the copy itself
-            host = out[:total].cpu()
-            e[4].record(st)
-        e[4].synchronize()
-        self._time("h2d_edits", e[0], e[1])
-        self._time("rewrite_size", e[1], e[2])
-        self._time("rewrite_write", e[2], e[3])
-        self._time("d2h_output", e[3], e[4])
-        self.d2h_bytes += total
-        return host.numpy(), line_bad
+        with self._stages() as mark:
+            doff = self._up(edit_off, np.int64)
+            ded = self._up(edits, L.VCF_EDIT_DTYPE)
+            mark("h2d_edits")
+            args = (self.dbuf, self.drecs, n, doff, ded, int(n_samples))
+            _, off, _, line_bad, total = self._size_scan(
+                mark, ("rewrite_size",) * 3, n, n, torch.uint8,
+                lambda out_len, stat: self._launch("unfz_vcf_rewrite_size", *args, out_len, stat))
+            if line_bad.any():
+                return np.zeros(0, dtype=np.uint8), line_bad
+            out = self._write(mark, ("rewrite_write", "d2h_output"), total,
+                              lambda out: self._launch("unfz_vcf_rewrite_write", *args, off, out))
+        return out, line_bad
 
 
-class BcfDecoder:
+class BcfDecoder(_Decoder):
     """Device side of ``bcfio.read_sites(engine=...)``, with the calls of ``bcfio.HostDecoder``: the inflated record
     bytes go up once (pinned staging) with the record offsets the host walked, unfz_bcf_parse runs on the engine's stream
     and the 80-byte records come back for the host's selection; then unfz_bcf_samples decodes the member cells of the
     selected records -- one thread per cell, a direct load at the field's sample stride -- which come back as the
     table's genotype arrays."""
 
-    def __init__(self, engine: "Engine"):
-        self.engine = engine
-        self.h2d_bytes = self.d2h_bytes = 0
-        self.timings_ms: Dict[str, float] = {}
-
-    def _time(self, name, e0, e1):
-        self.timings_ms[name] = self.timings_ms.get(name, 0.0) + e0.elapsed_time(e1)
-
     def records(self, buf: np.ndarray, offs: np.ndarray, keys: np.ndarray, n_samples: int) -> np.ndarray:
-        eng = self.engine
-        lib, ctx, dev = eng.lib, eng.ctx, eng.device
         n = int(offs.shape[0])
+        rsz = L.BCF_REC_DTYPE.itemsize
         keys = np.ascontiguousarray(keys, dtype=np.int32)
-        with eng.on_stream():
-            st = torch.cuda.current_stream(dev)
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
-            e[0].record(st)
+        with self._stages() as mark:
             self.buf = buf
-            self.dbuf = _to_device(np.ascontiguousarray(buf), dev, True) if buf.shape[0] else \
-                torch.zeros(16, dtype=torch.uint8, device=dev)
-            doffs = _to_device(np.ascontiguousarray(offs, dtype=np.int64), dev, True) if n else \
-                torch.zeros(1, dtype=torch.int64, device=dev)
-            e[1].record(st)
-            rsz = L.BCF_REC_DTYPE.itemsize
-            self.drecs = torch.empty((max(n, 1) * rsz,), dtype=torch.uint8, device=dev)
-            eng._check(lib.unfz_bcf_parse(ctx, self.dbuf.data_ptr(), doffs.data_ptr(), n, keys.ctypes.data, int(n_samples),
-                                          self.drecs.data_ptr(), C.c_void_p(st.cuda_stream)), "bcf_parse")
-            e[2].record(st)
+            self.dbuf = self._up(buf)
+            doffs = self._up(offs, np.int64)
+            mark("h2d_records")
+            self.drecs = self.engine._empty(n * rsz, torch.uint8)
+            self._launch("unfz_bcf_parse", self.dbuf, doffs, n, keys.ctypes.data, int(n_samples), self.drecs)
+            mark("parse")
             recs = self.drecs[: n * rsz].cpu().numpy().view(L.BCF_REC_DTYPE)
-            e[3].record(st)
-        e[3].synchronize()
-        self._time("h2d_records", e[0], e[1])
-        self._time("parse", e[1], e[2])
-        self._time("d2h_records", e[2], e[3])
-        self.h2d_bytes += int(buf.nbytes + offs.nbytes)
+            mark("d2h_records")
         self.d2h_bytes += int(recs.nbytes)
         self.recs = recs
         return recs
 
     def samples(self, sel: np.ndarray, member_sample: np.ndarray) -> Dict[str, np.ndarray]:
-        eng = self.engine
-        lib, ctx, dev = eng.lib, eng.ctx, eng.device
         ns, m = int(sel.shape[0]), int(member_sample.shape[0])
         cells = ns * m
-        with eng.on_stream():
-            st = torch.cuda.current_stream(dev)
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
-            e[0].record(st)
-            dsel = _to_device(np.ascontiguousarray(sel, dtype=np.int64), dev, True) if ns else \
-                torch.zeros(1, dtype=torch.int64, device=dev)
-            dms = _to_device(np.ascontiguousarray(member_sample, dtype=np.int32), dev, True) if m else \
-                torch.zeros(1, dtype=torch.int32, device=dev)
-            e[1].record(st)
-            out = {"gt": torch.empty((max(cells, 1),), dtype=torch.uint8, device=dev),
-                   "gq": torch.empty((max(cells, 1),), dtype=torch.float32, device=dev),
-                   "rd": torch.empty((max(cells, 1),), dtype=torch.int32, device=dev),
-                   "ad": torch.empty((max(cells, 1),), dtype=torch.int32, device=dev),
-                   "status": torch.empty((max(cells, 1),), dtype=torch.uint8, device=dev)}
-            eng._check(lib.unfz_bcf_samples(ctx, self.dbuf.data_ptr(), self.drecs.data_ptr(), dsel.data_ptr(), ns,
-                                            dms.data_ptr(), m, *(out[k].data_ptr() for k in ("gt", "gq", "rd", "ad", "status")),
-                                            C.c_void_p(st.cuda_stream)), "bcf_samples")
-            e[2].record(st)
+        with self._stages() as mark:
+            dsel = self._up(sel, np.int64)
+            dms = self._up(member_sample, np.int32)
+            mark("h2d_select")
+            out = {k: self.engine._empty(cells, dt) for k, dt in _CELLS}
+            self._launch("unfz_bcf_samples", self.dbuf, self.drecs, dsel, ns, dms, m, *(out[k] for k, _ in _CELLS))
+            mark("samples")
             host = {k: v.cpu().numpy() for k, v in out.items()}
-            e[3].record(st)
-        e[3].synchronize()
-        self._time("h2d_select", e[0], e[1])
-        self._time("samples", e[1], e[2])
-        self._time("d2h_cells", e[2], e[3])
-        self.h2d_bytes += int(sel.nbytes + member_sample.nbytes)
+            mark("d2h_cells")
         self.d2h_bytes += cells * 14
-        return {k: host[k][:cells].reshape(ns, m) for k in ("gt", "gq", "rd", "ad", "status")}
+        return {k: host[k][:cells].reshape(ns, m) for k, _ in _CELLS}
 
     def format(self, edit_off: np.ndarray, edits: np.ndarray, n_samples: int, names, fkeys: np.ndarray):
         """The records ``records()`` left on the device printed as the phased VCF body (csrc/bcfout.cu): (the output
@@ -625,82 +538,38 @@ class BcfDecoder:
         (``bcfio.format_host``): its length goes up before a second scan, and its text is copied into its slot.  With
         a haploid phase edit or a malformed record nothing is written: the output is empty and the status says why."""
         from .bcfio import format_host
-        eng = self.engine
-        lib, ctx, dev = eng.lib, eng.ctx, eng.device
         n = int(self.recs.shape[0])
-        ne = int(edits.shape[0])
         fkeys = np.ascontiguousarray(fkeys, dtype=np.int32)
-
-        def up(a, dtype):
-            return _to_device(np.ascontiguousarray(a, dtype=dtype), dev, True) if a.shape[0] else \
-                torch.zeros(16, dtype=torch.uint8, device=dev)
-        with eng.on_stream():
-            st = torch.cuda.current_stream(dev)
-            sp = C.c_void_p(st.cuda_stream)
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
-            e[0].record(st)
-            doff = up(edit_off, np.int64)
-            ded = up(edits, L.VCF_EDIT_DTYPE)
-            dnames = [up(a, a.dtype) for a in names]
-            e[1].record(st)
-            out_len = torch.empty((max(n, 1),), dtype=torch.int64, device=dev)
-            # the status of every record, then the total output length, in one download
-            nb = (n + 7) // 8 * 8
-            stat = torch.zeros((nb + 8,), dtype=torch.uint8, device=dev)
-            out_off = torch.zeros((n + 1,), dtype=torch.int64, device=dev)
-            work = torch.empty((int(lib.unfz_scan_work_bytes(max(n, 1))),), dtype=torch.uint8, device=dev)
-            args = (self.dbuf.data_ptr(), self.drecs.data_ptr(), n, dnames[0].data_ptr(), dnames[1].data_ptr(),
-                    int(names[1].shape[0]) - 1, dnames[2].data_ptr(), dnames[3].data_ptr(), int(names[3].shape[0]) - 1,
-                    fkeys.ctypes.data, doff.data_ptr(), ded.data_ptr(), int(n_samples))
-            eng._check(lib.unfz_bcf_format_size(ctx, *args, out_len.data_ptr(), stat.data_ptr(), sp), "bcf_format_size")
-            if n:
-                eng._check(lib.unfz_exclusive_scan_i64(ctx, out_len.data_ptr(), out_off.data_ptr(), n, work.data_ptr(), sp),
-                           "exclusive_scan_i64")
-            stat[nb:].view(torch.int64).copy_(out_off[n:])
-            host_stat = stat.cpu().numpy()
-            e[2].record(st)
-        status = host_stat[:n].copy()
-        total = int(host_stat[nb:].view(np.int64)[0])
-        self.h2d_bytes += int(edit_off.nbytes) + ne * L.VCF_EDIT_DTYPE.itemsize + sum(int(a.nbytes) for a in names)
-        self.d2h_bytes += nb + 8
-        if (status & (L.BCFOUT_HAPLOID | L.BCFOUT_BAD)).any():
-            self._time("h2d_edits", e[0], e[1])
-            return np.zeros(0, dtype=np.uint8), status
-        host = np.flatnonzero(status & L.BCFOUT_FLOAT_HOST)
-        if host.shape[0]:
-            # the host prints these records; their lengths replace the device's before the offsets are scanned again
-            t0 = time.perf_counter()
-            cnt = edit_off[host + 1] - edit_off[host]
-            sub_off = np.zeros(host.shape[0] + 1, dtype=np.int64)
-            np.cumsum(cnt, out=sub_off[1:])
-            sub_edits = edits[np.repeat(edit_off[host] - sub_off[:-1], cnt) + np.arange(int(sub_off[-1]))]
-            text, _st, lens = format_host(self.buf, self.recs[host], sub_off, sub_edits, n_samples, names, fkeys)
-            self.timings_ms["format_host"] = self.timings_ms.get("format_host", 0.0) + 1e3 * (time.perf_counter() - t0)
-            with eng.on_stream():
-                didx = _to_device(host.astype(np.int64), dev, True)
-                out_len[didx] = _to_device(np.ascontiguousarray(lens), dev, True)
-                eng._check(lib.unfz_exclusive_scan_i64(ctx, out_len.data_ptr(), out_off.data_ptr(), n, work.data_ptr(), sp),
-                           "exclusive_scan_i64")
-                total = int(out_off[n:].cpu()[0])
-                slot = out_off[didx].cpu().numpy()
-            self.h2d_bytes += 16 * int(host.shape[0])
-            self.d2h_bytes += 8 + 8 * int(host.shape[0])
-        with eng.on_stream():
-            out = torch.empty((max(total, 1),), dtype=torch.uint8, device=dev)
-            ew = torch.cuda.Event(enable_timing=True)
-            ew.record(st)
-            eng._check(lib.unfz_bcf_format_write(ctx, *args, stat.data_ptr(), out_off.data_ptr(), out.data_ptr(), sp),
-                       "bcf_format_write")
-            e[3].record(st)
-            res = out[:total].cpu()
-            e[4].record(st)
-        e[4].synchronize()
-        self._time("h2d_edits", e[0], e[1])
-        self._time("format_size", e[1], e[2])
-        self._time("format_write", ew, e[3])
-        self._time("d2h_output", e[3], e[4])
-        self.d2h_bytes += total
-        res = res.numpy()
+        with self._stages() as mark:
+            doff = self._up(edit_off, np.int64)
+            ded = self._up(edits, L.VCF_EDIT_DTYPE)
+            dnames = [self._up(a) for a in names]
+            mark("h2d_edits")
+            args = (self.dbuf, self.drecs, n, dnames[0], dnames[1], int(names[1].shape[0]) - 1, dnames[2], dnames[3],
+                    int(names[3].shape[0]) - 1, fkeys.ctypes.data, doff, ded, int(n_samples))
+            out_len, off, dstat, status, total = self._size_scan(
+                mark, ("format_size",) * 3, n, n, torch.uint8,
+                lambda out_len, stat: self._launch("unfz_bcf_format_size", *args, out_len, stat))
+            if (status & (L.BCFOUT_HAPLOID | L.BCFOUT_BAD)).any():
+                return np.zeros(0, dtype=np.uint8), status
+            host = np.flatnonzero(status & L.BCFOUT_FLOAT_HOST)
+            if host.shape[0]:
+                # the host prints these records; their lengths replace the device's before the offsets are scanned again
+                t0 = time.perf_counter()
+                cnt = edit_off[host + 1] - edit_off[host]
+                sub_off = np.zeros(host.shape[0] + 1, dtype=np.int64)
+                np.cumsum(cnt, out=sub_off[1:])
+                sub_edits = edits[np.repeat(edit_off[host] - sub_off[:-1], cnt) + np.arange(int(sub_off[-1]))]
+                text, _st, lens = format_host(self.buf, self.recs[host], sub_off, sub_edits, n_samples, names, fkeys)
+                self.timings_ms["format_host"] = self.timings_ms.get("format_host", 0.0) + 1e3 * (time.perf_counter() - t0)
+                didx = self._up(host, np.int64)
+                out_len[didx] = self._up(lens)
+                self._scan(out_len, off, n)
+                total = int(off[n:].cpu()[0])
+                slot = off[didx].cpu().numpy()
+                self.d2h_bytes += 8 + 8 * int(host.shape[0])
+            res = self._write(mark, ("format_write", "d2h_output"), total,
+                              lambda out: self._launch("unfz_bcf_format_write", *args, dstat, off, out))
         if host.shape[0]:
             src = np.zeros(host.shape[0] + 1, dtype=np.int64)
             np.cumsum(lens, out=src[1:])
